@@ -1,15 +1,20 @@
 #!/usr/bin/env python
 """bench.py - STE-GAN hot-path benchmark (BASELINE.json: GAN train samples/s, configs[1]).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--torch-compile] [--no-cpu-baseline] [--quick]
+    python bench.py --gpus N --steps K --warmup W [--repeats R] [--impl reference] [--torch-compile] [--no-cpu-baseline]
+                    [--quick] [--dump-outputs DIR]
     (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 One "step" = one full GAN train step (train.py:165-268 without the encoder losses) on a synthetic batch of 16 samples
 per GPU, 100 unit frames -> 1600x8 EMG samples, bf16 tensor-core mode, weak scaling (per-GPU batch fixed).  Prints ONE
-JSON line (rank 0).
+JSON line (rank 0).  Inputs and initial weights come from fixed seeds: the same arguments give the same inputs.
 
-  value     whole-job samples/s with inputs resident in HBM, CUDA-graph replay, device-timed; the K-step timed region is
-            repeated `repeats` times (each bracketed by barrier + synchronize) and the MEDIAN is reported
+  value     whole-job samples/s with inputs resident in HBM, CUDA-graph replay, device-timed; K timed steps in all, split
+            into R timed regions (default 1, each bracketed by barrier + synchronize); the MEDIAN of their ms per step is
+            reported
+  --dump-outputs DIR  after those K steps: the loss slots, the generated batch and a fixed sample of the updated weights
+            of the last step, as DIR/<name>.npy (float32), for comparing the outputs of two builds (two runs of one build
+            differ by rounding noise that grows with the number of steps: DESIGN.md section 8)
   e2e       the same through GanTrainer.step_graph() with pinned HOST inputs (H2D inside the timed region) and a host
             read of the loss slots every step
   parity_gate  BEFORE any timing: the first graph step's losses against the CPU reference arm on the same batch and
@@ -209,21 +214,43 @@ def cupti_by_kernel(fn, n_rep: int):
 
 
 def timed_region(fn_step, fn_tail, steps: int, repeats: int, barrier, max_over_ranks):
-    """`repeats` timed regions of exactly `steps` steps each, every one bracketed by barrier + synchronize on both
-    sides and timed with CUDA events on the launching stream; returns (median ms per step, all ms per step)."""
+    """Exactly `steps` steps in all, split into `repeats` consecutive timed regions of (nearly) equal length, every one
+    bracketed by barrier + synchronize on both sides and timed with CUDA events on the launching stream; returns
+    (median ms per step, ms per step of every region)."""
     import torch
     per = []
-    for _ in range(repeats):
+    n_regions = min(repeats, steps)
+    done = 0
+    for r in range(n_regions):
+        n = steps // n_regions + (r < steps % n_regions)
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for i in range(steps):
+        for i in range(done, done + n):
             fn_step(i)
         fn_tail()
         e1.record()
         barrier()
-        per.append(max_over_ranks(e0.elapsed_time(e1)) / steps)
+        per.append(max_over_ranks(e0.elapsed_time(e1)) / n)
+        done += n
     return statistics.median(per), per
+
+
+def dump_outputs(out_dir: str, tr, net_g, net_d, sample: int = 1 << 20) -> None:
+    """What the timed train step has handed its caller after its last step, as float32 .npy files: the loss slots
+    (losses.npy, in the order of trainer.LOSS_NAMES), the generated EMG batch (x_pred.npy, [B, T, C]) and the updated
+    weights of both networks (g_params.npy, d_params.npy: `sample` elements of all parameters concatenated in
+    registration order, at indices drawn with seed 0, the same in every run) - 9 MB in all."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"losses": tr.slots, "x_pred": tr.x_pred}
+    for name, net in (("g_params", net_g), ("d_params", net_d)):
+        flat = torch.cat([p.detach().reshape(-1) for p in net.parameters()])
+        idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:sample].sort().values
+        arrays[name] = flat[idx.to(flat.device)]
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------ GPU arm
@@ -309,6 +336,8 @@ def run_ours(args):
     clocks = sampler.stop()
     value = BATCH_PER_GPU * world / (ms_step / 1e3)
     final_losses = tr.losses()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tr, g, d)
 
     # ---- timed region 2: end to end (pinned host inputs, loss read back every step)
     for i in range(2):
@@ -497,7 +526,7 @@ def run_ours(args):
         ph = torch.randint(0, 48, (BATCH_PER_GPU, FRAMES), generator=torch.Generator().manual_seed(3)).to(dev)
         for i in range(3):
             tr2.step_graph(*devb[i % nb], phoneme_targets=ph)
-        ms_enc, _ = timed_region(lambda i: tr2.step_graph(*devb[i % nb], phoneme_targets=ph), tr2.flush, 10, 3, barrier, max_over_ranks)
+        ms_enc, _ = timed_region(lambda i: tr2.step_graph(*devb[i % nb], phoneme_targets=ph), tr2.flush, 30, 3, barrier, max_over_ranks)
         L2 = tr2.losses()
         gf = STEP_GFLOP_PER_SAMPLE + 35.0
         encoder_step = {"workload": "configs[1] + speech-unit and phoneme losses through the frozen EMG encoder (768-d, 4 ResBlocks, 6 rel-pos "
@@ -519,7 +548,7 @@ def run_ours(args):
         line = {"metric": "GAN train samples/s", "value": value, "unit": "samples/s", "n_gpus": world, "steps": args.steps,
                 "warmup": max(3, args.warmup), "ms_per_step": ms_step, "higher_is_better": True, "scaling": "weak",
                 "vs_baseline": None, "dtype": "bf16", "data": "synthetic", "config": config_dict(world), "clocks": clocks,
-                "timed_repeats": repeats, "ms_per_step_all_repeats": [round(x, 4) for x in ms_all],
+                "timed_repeats": len(ms_all), "ms_per_step_all_repeats": [round(x, 4) for x in ms_all],
                 "e2e": e2e, "gpu_launches": int(launches_per_step * args.steps), "launches_per_step": int(launches_per_step),
                 "parity_gate": gate, "roofline": roofline, "cpu_baseline": cpu, "inference": inference, "disc_losses": disc_losses,
                 "encoder_step": encoder_step,
@@ -570,7 +599,7 @@ def disc_losses_sweep(torch, tr_unused, dev, peaks, with_cpu, DiscriminatorSmall
                 dx = tr.disc_losses_step(x_pred, x_real)
             for _ in range(3):
                 graph.replay()
-            ms, _ = timed_region(lambda i: graph.replay(), lambda: None, 10, 3, barrier, lambda x: x)
+            ms, _ = timed_region(lambda i: graph.replay(), lambda: None, 30, 3, barrier, lambda x: x)
             tf = DISC_GFLOP_PER_SAMPLE[family] * B / ms
             finite = bool(torch.isfinite(dx).all()) and bool(torch.isfinite(tr.slots).all())
             out["points"].append({"discriminator": family, "batch": B, "ms_per_step": round(ms, 4), "value": round(B / (ms / 1e3), 1),
@@ -612,12 +641,19 @@ def main():
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
-    ap.add_argument("--repeats", type=int, default=5, help="timed regions of --steps steps each; the median is reported")
+    ap.add_argument("--repeats", type=int, default=1,
+                    help="timed regions the --steps steps are split into; the median of their ms per step is reported")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--torch-compile", action="store_true", help="also time the reference step under torch.compile on the GPU")
-    ap.add_argument("--quick", action="store_true", help="train + inference lines only, one timed repeat")
+    ap.add_argument("--quick", action="store_true", help="train + inference lines only, one timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed train step computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.repeats < 1:
+        ap.error("--steps and --repeats must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU train step; --impl reference does not run it")
     if args.impl == "reference":
         run_reference(args)
     else:

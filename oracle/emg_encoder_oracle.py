@@ -29,6 +29,33 @@ StateDict = Dict[str, Tensor]
 BN_EPS, LN_EPS = 1e-5, 1e-5
 MAX_REL = 100          # relative_positional_distance (emg_encoder.py:64)
 
+# tests/golden/emg_encoder_tiny.pt holds the reference's outputs only: the weights and inputs they were computed from are
+# drawn from seeds by the two functions below, for the reference module (oracle/make_golden.py) and for the tests alike
+TINY_ENCODER = dict(model_size=32, num_extra_res_blocks=3, num_transformer_layers=2)
+TINY_CASE_SHAPES = ((2, 400, 8), (1, 1776, 8))          # 25 frames; 111 frames (> 100: out-of-range relative positions)
+
+
+def tiny_encoder_state(encoder_cls) -> StateDict:
+    """Weights of the fixture encoder, as halves: the seed-0 initialisation of encoder_cls(8, 256, 48, **TINY_ENCODER) (the
+    reference's EMGEncoderTransformer, or the drop-in, which initialises bit-identically), then non-trivial BatchNorm
+    statistics (a trained checkpoint has them), everything rounded to the fp16 grid."""
+    torch.manual_seed(0)
+    enc = encoder_cls(8, 256, 48, **TINY_ENCODER)
+    with torch.no_grad():
+        for mod in enc.modules():
+            if isinstance(mod, torch.nn.BatchNorm1d):
+                mod.running_mean.normal_(0, 0.3); mod.running_var.uniform_(0.5, 1.5)
+                mod.weight.uniform_(0.5, 1.5); mod.bias.normal_(0, 0.2)
+    return {k: (v.half() if v.is_floating_point() else v.clone()) for k, v in enc.state_dict().items()}
+
+
+def tiny_case_inputs(i: int) -> Tuple[Tensor, Tensor, Tensor]:
+    """Fixture case i: EMG input [B, T, 8] in (-1, 1), speech-unit targets [B, T/16, 256], phoneme labels [B, T/16]."""
+    B, T, C = TINY_CASE_SHAPES[i]
+    g = torch.Generator().manual_seed(20 + i)
+    x = torch.tanh(torch.randn(B, T, C, generator=g))
+    return x, torch.randn(B, T // 16, 256, generator=g), torch.randint(0, 48, (B, T // 16), generator=g)
+
 
 def _bn_eval(sd: StateDict, p: str, x: Tensor) -> Tensor:
     """BatchNorm1d in eval mode on [B,C,T] (conv.py:112,114,118)."""

@@ -1,7 +1,7 @@
 """Generate tests/golden/*.pt by running the UNMODIFIED reference modules.
 
-Run in the authoring container only (needs /root/reference):
-    python oracle/make_golden.py
+Needs a checkout of the original STE-GAN (the directory that holds its `ste_gan` package):
+    STE_GAN_REFERENCE=<checkout> python oracle/make_golden.py
 The reference imports `omegaconf` (absent here) for type annotations only, so a
 3-line in-memory stub is installed first (SURVEY.md 8c).  Nothing from the
 reference is copied; only its *outputs* on seeded inputs are stored.
@@ -19,8 +19,10 @@ Fixtures (all fp32, seed 0):
                       losses, G output, per-parameter gradient norms and samples.
   emg_encoder_init.pt per-key checksums of the seed-0 initialisation of that encoder (pins the drop-in module's init).
   emg_encoder_tiny.pt (SURVEY.md 8f rank 1) a model_size=32, 2-layer EMG encoder in eval
-                      mode: state_dict, two inputs (25 and 111 frames), both outputs, the speech-unit and
-                      phoneme losses and the gradient of their sum w.r.t. the EMG input.
+                      mode on two inputs (25 and 111 frames): both outputs, the speech-unit and
+                      phoneme losses and the gradient of their sum w.r.t. the EMG input.  Its
+                      weights and inputs are drawn from seeds (oracle/emg_encoder_oracle.py,
+                      tiny_encoder_state / tiny_case_inputs), not stored.
 """
 import os
 import sys
@@ -34,7 +36,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 m = types.ModuleType("omegaconf"); m.OmegaConf = object; m.DictConfig = dict
 sys.modules["omegaconf"] = m
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.environ["STE_GAN_REFERENCE"])
 
 import torch.nn.functional as F  # noqa: E402
 from ste_gan.losses.time_domain_loss import MultiTimeDomainFeatureLoss  # noqa: E402
@@ -179,17 +181,12 @@ def emg_encoder_fixture():
     .forward rejects the reference's custom layer (it reads self_attn.batch_first; the reference pins torch 2.0.1), so
     the encoder's own layers are applied one after the other - exactly what 2.0.1 does for a mask-free stack."""
     from ste_gan.models.emg_encoder import EMGEncoderTransformer
+    from oracle import emg_encoder_oracle as E
     torch.manual_seed(0)
-    enc = EMGEncoderTransformer(8, 256, 48, model_size=32, num_extra_res_blocks=3, num_transformer_layers=2).eval()
+    enc = EMGEncoderTransformer(8, 256, 48, **E.TINY_ENCODER).eval()
     # seed-0 initialisation checksums (key order included): pins that the drop-in module consumes the RNG identically
     torch.save({k: tensor_summary(v.float()) for k, v in enc.state_dict().items()}, os.path.join(OUT, "emg_encoder_init.pt"))
-    for mod in enc.modules():           # non-trivial BatchNorm statistics (a trained checkpoint has them)
-        if isinstance(mod, torch.nn.BatchNorm1d):
-            mod.running_mean.normal_(0, 0.3); mod.running_var.uniform_(0.5, 1.5)
-            mod.weight.data.uniform_(0.5, 1.5); mod.bias.data.normal_(0, 0.2)
-    with torch.no_grad():               # weights on the fp16 grid: the fixture stores them as halves (0.9 MB instead of 2.4)
-        for t in list(enc.parameters()) + [b for b in enc.buffers() if b.is_floating_point()]:
-            t.copy_(t.half().float())
+    enc.load_state_dict(E.tiny_encoder_state(EMGEncoderTransformer))     # fp16-grid weights, non-trivial BatchNorm statistics
 
     def fwd(x):
         h = enc.conv_blocks(x.transpose(1, 2)).transpose(1, 2)
@@ -200,20 +197,16 @@ def emg_encoder_fixture():
         return enc.w_out(h), enc.w_aux(h)
 
     cases = []
-    for i, shape in enumerate(((2, 400, 8), (1, 1776, 8))):       # 25 frames; 111 frames (> 100: out-of-range positions)
-        g = torch.Generator().manual_seed(20 + i)
-        x = torch.tanh(torch.randn(*shape, generator=g)).requires_grad_(True)
+    for i in range(len(E.TINY_CASE_SHAPES)):
+        x, tgt, ph = E.tiny_case_inputs(i)
+        x.requires_grad_(True)
         units, phon = fwd(x)
-        tgt = torch.randn(units.shape, generator=g)
-        ph = torch.randint(0, 48, phon.shape[:2], generator=g)
         unit_loss = F.pairwise_distance(tgt.reshape(-1, 256), units.reshape(-1, 256)).mean()     # emg_encoder_loss.py:63-67
         ce = F.cross_entropy(phon.transpose(1, 2), ph)                                           # :80-83
         (dx,) = torch.autograd.grad(unit_loss + ce, x)
-        cases.append(dict(x=x.detach(), unit_target=tgt, phoneme_target=ph, units=units.detach(), phonemes=phon.detach(),
-                          unit_loss=unit_loss.detach(), phoneme_loss=ce.detach(), dx=dx))
-    torch.save(dict(state_dict={k: (v.half() if v.is_floating_point() else v.clone()) for k, v in enc.state_dict().items()}, cases=cases),
-               os.path.join(OUT, "emg_encoder_tiny.pt"))
-    print("emg_encoder_tiny.pt", sum(v.numel() for v in enc.state_dict().values()), "weights")
+        cases.append(dict(units=units.detach(), phonemes=phon.detach(), unit_loss=unit_loss.detach(), phoneme_loss=ce.detach(),
+                          dx=dx))
+    torch.save(dict(cases=cases), os.path.join(OUT, "emg_encoder_tiny.pt"))
 
 
 if __name__ == "__main__":

@@ -21,8 +21,10 @@ DT = {"fp32": torch.float32, "bf16": torch.bfloat16}
 def _tiny_encoder():
     from ste_gan_b200.models.emg_encoder import EMGEncoderTransformer
     fx = torch.load(os.path.join(GOLD, "emg_encoder_tiny.pt"))
-    enc = EMGEncoderTransformer(8, 256, 48, model_size=32, num_extra_res_blocks=3, num_transformer_layers=2)
-    sd = {k: (v.float() if v.is_floating_point() else v) for k, v in fx["state_dict"].items()}
+    for i, case in enumerate(fx["cases"]):
+        case["x"], case["unit_target"], case["phoneme_target"] = E.tiny_case_inputs(i)
+    enc = EMGEncoderTransformer(8, 256, 48, **E.TINY_ENCODER)
+    sd = {k: (v.float() if v.is_floating_point() else v) for k, v in E.tiny_encoder_state(EMGEncoderTransformer).items()}
     enc.load_state_dict(sd)
     return enc.eval(), sd, fx
 

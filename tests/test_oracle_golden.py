@@ -1,6 +1,7 @@
 """CPU: the oracle (oracle/ste_gan_oracle.py) against the committed golden fixtures produced from the
-UNMODIFIED reference modules (oracle/make_golden.py), and against the live reference when
-/root/reference is present (authoring container only)."""
+UNMODIFIED reference modules (oracle/make_golden.py), and against the live reference when the
+environment variable STE_GAN_REFERENCE names a checkout of the original STE-GAN (the directory that
+holds its `ste_gan` package)."""
 import os
 import sys
 import types
@@ -11,7 +12,8 @@ import torch
 from oracle import ste_gan_oracle as O
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
-HAVE_REF = os.path.isdir("/root/reference/ste_gan")
+REF = os.environ.get("STE_GAN_REFERENCE", "")
+HAVE_REF = bool(REF) and os.path.isdir(os.path.join(REF, "ste_gan"))
 
 
 def _seed0_state_dicts():
@@ -79,12 +81,12 @@ def test_train_step_b1_golden():
             assert abs(t.norm().item() - ref["l2"]) <= 2e-4 * max(ref["l2"], 1e-9), (name, k)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference not present (GPU box)")
+@pytest.mark.skipif(not HAVE_REF, reason="STE_GAN_REFERENCE does not name a checkout of the original STE-GAN")
 def test_oracle_vs_live_reference():
     m = types.ModuleType("omegaconf"); m.OmegaConf = object; m.DictConfig = dict
     sys.modules.setdefault("omegaconf", m)
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
+    if REF not in sys.path:
+        sys.path.insert(0, REF)
     import warnings
     warnings.filterwarnings("ignore")
     from ste_gan.models.discriminator import DiscriminatorSmall
@@ -110,9 +112,12 @@ def test_emg_encoder_oracle_matches_reference_fixture():
     speech-unit / phoneme losses taken through it and the gradient of their sum w.r.t. the EMG input, against the
     reference modules' outputs (25 frames, and 111 frames > the 100-frame relative-position range)."""
     from oracle import emg_encoder_oracle as E
+    from ste_gan_b200.models.emg_encoder import EMGEncoderTransformer
     fx = torch.load(os.path.join(GOLD, "emg_encoder_tiny.pt"))
-    sd = {k: v.double() for k, v in fx["state_dict"].items()}      # stored as halves (the reference ran on exactly these values)
-    for case in fx["cases"]:
+    # the halves the reference ran on, drawn from their seeds (bit-identical: the drop-in initialises as the reference does)
+    sd = {k: v.double() for k, v in E.tiny_encoder_state(EMGEncoderTransformer).items()}
+    for i, case in enumerate(fx["cases"]):
+        case["x"], case["unit_target"], case["phoneme_target"] = E.tiny_case_inputs(i)
         x = case["x"].double().requires_grad_(True)
         units, phon = E.emg_encoder_forward(sd, x)
         assert list(units.shape) == list(case["units"].shape) and list(phon.shape) == list(case["phonemes"].shape)
