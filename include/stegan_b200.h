@@ -92,6 +92,19 @@ typedef struct StgConv {
 int stg_conv(const StgConv* d, stg_stream_t stream);
 
 /*
+ * stg_conv with per-sample length masks in the epilogue, for batches of utterances zero-padded to a common length:
+ * accumulator row r of sample b is kept iff r < valid_units[b] * rows_per_unit; every other row is written as 0 to
+ * y_raw and y_act (both 2r and 2r+1 when dup_rows).  The zero is a select, so whatever the padded rows of add_post or
+ * src hold - NaN included - a masked output row is exactly 0.  When every layer of a stack masks its outputs, each
+ * convolution reads zeros past a sample's end, which is the zero padding of that sample run on its own.
+ * valid_units: DEVICE array of n_samples ints, read at execution time (a captured graph serves any length mix);
+ * negative values count as 0, values past t_dst mask nothing.  Forward only: STG_EINVAL when valid_units is NULL,
+ * rows_per_unit < 1, or the call is transposed, pair_sum or phases != 1.  Same engines and launch plan as stg_conv
+ * (tcgen05 when stg_conv_tc_supported, otherwise the CUDA-core engine; never the 1-channel matvec kernels).
+ */
+int stg_conv_masked(const StgConv* d, const int32_t* valid_units, int32_t rows_per_unit, stg_stream_t stream);
+
+/*
  * Weight gradient: dw[c][j][q] += sum_{n,r} dy[n][r][c] * x[n][r*stride + j*dilation - pad][g(c)*cin_g + q]
  * dw is float32 [c_out][k][c_in/groups] and is ACCUMULATED into (caller zeroes it).
  * Replaces the autograd conv backward-weight of the call sites listed for StgConv.

@@ -50,6 +50,7 @@ MAX_LOSS_ITEMS = 32
 _P, _I, _L, _F = C.c_void_p, C.c_int, C.c_int64, C.c_float
 _SIGS = {
     "stg_conv": [C.POINTER(StgConv), _P],
+    "stg_conv_masked": [C.POINTER(StgConv), _P, C.c_int32, _P],
     "stg_conv_wgrad": [C.POINTER(StgWgrad), _P],
     "stg_conv_tc_supported": [C.POINTER(StgConv)],
     "stg_conv_route": [C.POINTER(StgConv)],

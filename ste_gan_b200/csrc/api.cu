@@ -51,6 +51,21 @@ extern "C" int stg_conv(const StgConv* d, stg_stream_t stream) {
   }
 }
 
+/* stg_conv with per-sample length masks (forward only; the matvec engine is never chosen) */
+extern "C" int stg_conv_masked(const StgConv* d, const int32_t* valid_units, int32_t rows_per_unit, stg_stream_t stream) {
+  int r = validate_conv(d);
+  if (r) return r;
+  if (!valid_units || rows_per_unit < 1 || d->transposed || d->pair_sum || d->phases != 1) return STG_EINVAL;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  switch (d->engine) {
+    case STG_ENGINE_SIMT: return conv_simt(d, s, valid_units, rows_per_unit);
+    case STG_ENGINE_TCGEN05: return conv_tc(d, s, valid_units, rows_per_unit);
+    case STG_ENGINE_AUTO:
+      return conv_tc_supported(d) ? conv_tc(d, s, valid_units, rows_per_unit) : conv_simt(d, s, valid_units, rows_per_unit);
+    default: return STG_EINVAL;
+  }
+}
+
 /* which engine a call will run on: STG_ENGINE_SIMT, STG_ENGINE_TCGEN05 or STG_ENGINE_MATVEC */
 extern "C" int stg_conv_route(const StgConv* d) {
   if (!d || validate_conv(d) != STG_OK) return STG_EINVAL;

@@ -97,9 +97,9 @@ __device__ __forceinline__ float block_sum(float v, float* red) {
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 
-// engines
-int conv_simt(const StgConv* d, cudaStream_t s);
-int conv_tc(const StgConv* d, cudaStream_t s);
+// engines.  valid_units / rows_per_unit: the per-sample length mask of stg_conv_masked (nullptr: none)
+int conv_simt(const StgConv* d, cudaStream_t s, const int32_t* valid_units = nullptr, int rows_per_unit = 1);
+int conv_tc(const StgConv* d, cudaStream_t s, const int32_t* valid_units = nullptr, int rows_per_unit = 1);
 int conv_tc_plan(const StgConv* d, int* out);   // host-only: the plan conv_tc would launch (16 ints, see stg_debug_conv_plan)
 bool conv_tc_supported(const StgConv* d);
 int wgrad_simt(const StgWgrad* d, cudaStream_t s);

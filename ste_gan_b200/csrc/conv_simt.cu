@@ -15,10 +15,12 @@ struct EpiP {
   const float* bias;
   const void *add_pre, *mask, *add_post;
   void *y_raw, *y_act;
+  const int32_t* valid_units;   // stg_conv_masked: rows >= valid_units[b] * rows_per_unit are written as 0 (nullptr: no mask)
+  int rows_per_unit;
 };
 
 // Writes up to 4 consecutive channels of one output row.
-template <typename T>
+template <typename T, bool kMask>
 __device__ __forceinline__ void epilogue_row(const EpiP& e, int b, int ph, int row, int col, int ncols, float (&v)[4]) {
   const int64_t pitch = (int64_t)e.phases * e.c_dst;
   const int64_t off = ((int64_t)b * e.t_out + row) * pitch + (int64_t)ph * e.c_dst + col;
@@ -43,6 +45,11 @@ __device__ __forceinline__ void epilogue_row(const EpiP& e, int b, int ph, int r
     float x = v[i] + pre[i];
     if (e.mask) x *= act_grad_from_output(e.mask_mode, mk[i]);
     v[i] = x + post[i];
+  }
+  if constexpr (kMask) {   // a select, not a product: NaN in the padded rows of add_post cannot leak into a masked row
+    const bool keep = (int64_t)row < (int64_t)max(e.valid_units[b], 0) * e.rows_per_unit;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) v[i] = keep ? v[i] : 0.f;
   }
   if (e.y_raw) {
     if (e.out_f32) {
@@ -77,7 +84,8 @@ struct ConvP {
   EpiP e;
 };
 
-template <typename T>
+// kMask: stg_conv_masked (per-sample length masks in the epilogue); the unmasked instances compile without them
+template <typename T, bool kMask>
 __global__ void __launch_bounds__(256) conv_simt_kernel(const ConvP p) {
   __shared__ __align__(16) float As[BK][LDS];
   __shared__ __align__(16) float Bs[BK][LDS];
@@ -174,7 +182,7 @@ __global__ void __launch_bounds__(256) conv_simt_kernel(const ConvP p) {
         float v[4];
 #pragma unroll
         for (int j = 0; j < 4; ++j) v[j] = acc[i][j] + acc[i + 1][j] + 2.f * bias[j];
-        epilogue_row<T>(p.e, b, ph, row >> 1, col, ncols, v);
+        epilogue_row<T, kMask>(p.e, b, ph, row >> 1, col, ncols, v);
       }
     }
   } else {
@@ -185,7 +193,7 @@ __global__ void __launch_bounds__(256) conv_simt_kernel(const ConvP p) {
         float v[4];
 #pragma unroll
         for (int j = 0; j < 4; ++j) v[j] = acc[i][j] + bias[j];
-        epilogue_row<T>(p.e, b, ph, row, col, ncols, v);
+        epilogue_row<T, kMask>(p.e, b, ph, row, col, ncols, v);
       }
     }
   }
@@ -341,7 +349,7 @@ __global__ void __launch_bounds__(256) colsum_vec_kernel(const T* __restrict__ d
 
 }  // namespace
 
-int conv_simt(const StgConv* d, cudaStream_t s) {
+int conv_simt(const StgConv* d, cudaStream_t s, const int32_t* valid_units, int rows_per_unit) {
   ConvP p;
   p.n_vs = d->n_samples * d->phases; p.phases = d->phases; p.t_src = d->t_src; p.t_dst = d->t_dst;
   p.c_src = d->c_src; p.c_dst = d->c_dst; p.groups = d->groups; p.k = d->k; p.dilation = d->dilation;
@@ -355,10 +363,12 @@ int conv_simt(const StgConv* d, cudaStream_t s) {
   e.post_shift = d->post_shift; e.mask_mode = d->mask_mode; e.act = d->act; e.dup_rows = d->dup_rows;
   e.out_f32 = d->out_f32; e.pair_sum = d->pair_sum; e.bias = d->bias; e.add_pre = d->add_pre; e.mask = d->mask;
   e.add_post = d->add_post; e.y_raw = d->y_raw; e.y_act = d->y_act;
+  e.valid_units = valid_units; e.rows_per_unit = rows_per_unit;
   dim3 grid(ceil_div(d->t_dst, BM), d->groups * p.tiles_per_group, p.n_vs);
   if (grid.z > 65535 || grid.y > 65535) return STG_EINVAL;
-  if (d->dtype == STG_F32) conv_simt_kernel<float><<<grid, 256, 0, s>>>(p);
-  else conv_simt_kernel<bf16><<<grid, 256, 0, s>>>(p);
+  const bool masked = valid_units != nullptr;
+  if (d->dtype == STG_F32) (masked ? conv_simt_kernel<float, true> : conv_simt_kernel<float, false>)<<<grid, 256, 0, s>>>(p);
+  else (masked ? conv_simt_kernel<bf16, true> : conv_simt_kernel<bf16, false>)<<<grid, 256, 0, s>>>(p);
   STG_LAUNCH_CHECK();
   return STG_OK;
 }

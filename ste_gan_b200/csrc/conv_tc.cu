@@ -57,6 +57,8 @@ struct TcEpi {
   const bf16 *add_pre, *mask, *add_post;
   void* y_raw;
   void* y_act;
+  const int32_t* valid_units;   // stg_conv_masked: accumulator rows >= valid_units[b] * rows_per_unit are written as 0 (nullptr: no mask)
+  int rows_per_unit;
 };
 
 // Per-group / per-tap tables, read with warp-uniform indices (uniform constant loads) by the producer / MMA warps.
@@ -240,6 +242,12 @@ __device__ __forceinline__ int out_row(const TcP& p, const Tile& x, int m) {
   return h < p.t_dst ? h * p.phases + ph : -1;
 }
 
+// stg_conv_masked: does output row `row` of sample b (before dup_rows) lie inside the sample's valid length?  Called after
+// pdl_wait (valid_units may be written by the previous kernel of the stream).
+__device__ __forceinline__ bool row_kept(const TcEpi& e, int b, int row) {
+  return (int64_t)row < (int64_t)max(e.valid_units[b], 0) * e.rows_per_unit;
+}
+
 // ---------------------------------------------------------------------------------------------- direct epilogue
 struct EpiIn {
   float pre[16], mk[16], post[16];
@@ -261,7 +269,8 @@ __device__ __forceinline__ void epi_load(const TcEpi& e, int b, int row, int col
   }
 }
 // v: accumulator (+bias, pair-summed) of one output row, 16 channels
-__device__ __forceinline__ void epi_store(const TcEpi& e, int b, int row, int col, float (&v)[16], const EpiIn& in) {
+// keep == false (length mask): the row is written as 0 - a select, so NaN in the padded rows of add_post never reaches it
+__device__ __forceinline__ void epi_store(const TcEpi& e, int b, int row, int col, float (&v)[16], const EpiIn& in, bool keep) {
   const int64_t off = ((int64_t)b * e.rows + row) * e.c_dst + col;
   const int ncols = min(16, e.c_dst - col);
   const bool vec = (ncols == 16) && ((e.c_dst & 7) == 0);
@@ -276,6 +285,10 @@ __device__ __forceinline__ void epi_store(const TcEpi& e, int b, int row, int co
   if (e.add_post) {
 #pragma unroll
     for (int i = 0; i < 16; ++i) v[i] += in.post[i];
+  }
+  if (!keep) {
+#pragma unroll
+    for (int i = 0; i < 16; ++i) v[i] = 0.f;
   }
   if (e.y_raw) {
     if (e.out_f32) {
@@ -304,7 +317,8 @@ __device__ __forceinline__ void epi_store(const TcEpi& e, int b, int row, int co
 }
 
 // ---------------------------------------------------------------------------------------------- kernel
-template <bool kStaged, bool kPair>
+// kMask: stg_conv_masked (per-sample length masks in both epilogues); the unmasked instances compile without them
+template <bool kStaged, bool kPair, bool kMask>
 __global__ void __launch_bounds__(kStaged ? 384 : 352, (kStaged && !kPair) ? 2 : 1)
 conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtensorMap tmW,
                const __grid_constant__ EpiMaps em, const TcP p) {
@@ -694,6 +708,17 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
         const Tile x = decode_tile<kPair>(p, t, rank);
         const int as = acc_i & 1, aph = (acc_i >> 1) & 1;
         trc.ev(10, t);
+        // length mask: my row is (x.b, x.h0 + m), or in a row-class tail tile, which stacks seg-row slices of 128 / seg
+        // samples, (x.b + m / seg, x.h0 + m % seg).  Rows past the sample or the batch are clipped by the TMA stores.
+        // The select runs only in warps that hold a masked row (warp-uniform branch): the epilogue is issue-bound, and
+        // most tiles of a padded batch lie wholly inside their samples.
+        bool keep = true, warp_masked = false;
+        if constexpr (kMask) {
+          int mb = x.b, mh = x.h0 + m;
+          if (p.n_cls > 1 && p.cls_tps[x.cls] == 0) { const int seg = p.cls_seg[x.cls]; mb += m / seg; mh = x.h0 + m % seg; }
+          keep = mb < p.n_samples && row_kept(e, mb, mh);
+          warp_masked = __any_sync(0xffffffffu, !keep);
+        }
         // bias of this column tile -> smem (nobody reads the previous tile's bias any more: every thread has
         // passed its FULL arrive of the last sub-tile, which comes after its bias reads ... of ITS OWN rows only,
         // hence the 128-thread barrier below also orders the overwrite against slower warps)
@@ -788,6 +813,10 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
           const int obuf = ring(q);
           if (q >= p.out_ring) asm volatile("bar.sync %0, 160;" ::"r"(bar_free(obuf)) : "memory");  // stores of sub-tile q - out_ring drained
           trc.ev(23, s);
+          if (warp_masked) {
+#pragma unroll
+            for (int i = 0; i < 32; ++i) v[i] = keep ? v[i] : 0.f;
+          }
           if (writer) {
             int o = 0;
             if (e.has_raw) {
@@ -826,6 +855,7 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
       const int arow = out_row(p, x, sub * 32 + lane);  // output row of this thread (before pair_sum)
       const bool row_ok = arow >= 0 && (!e.pair_sum || (lane & 1) == 0);
       const int orow = e.pair_sum ? (arow >> 1) : arow;
+      const bool keep = !kMask || (row_ok && row_kept(e, x.b, orow));
       EpiIn inA, inB;
       if (c_lo < c_hi) epi_load(e, x.b, orow, x.col0 + c_lo * 16, row_ok, inA);
       if (x.n_iters > 0) {
@@ -851,7 +881,7 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
 #pragma unroll
           for (int i = 0; i < 16; ++i) v[i] += __shfl_xor_sync(0xffffffffu, v[i], 1);
         }
-        if (row_ok) epi_store(e, x.b, orow, col, v, in);
+        if (row_ok) epi_store(e, x.b, orow, col, v, in, keep);
       };
 #pragma unroll 1
       for (int c = c_lo; c < c_hi; c += 2) {
@@ -1113,7 +1143,7 @@ int conv_tc_plan(const StgConv* d, int* out) {
   return r;
 }
 
-int conv_tc(const StgConv* d, cudaStream_t s) {
+int conv_tc(const StgConv* d, cudaStream_t s, const int32_t* valid_units, int rows_per_unit) {
   if (!conv_tc_supported(d)) return STG_EUNSUPPORTED;
   TcP p;
   p.trace = g_trace;
@@ -1163,6 +1193,7 @@ int conv_tc(const StgConv* d, cudaStream_t s) {
   e.add_post = static_cast<const bf16*>(d->add_post); e.y_raw = d->y_raw; e.y_act = d->y_act;
   e.has_pre = d->add_pre != nullptr; e.has_mask = d->mask != nullptr; e.has_post = d->add_post != nullptr;
   e.has_raw = d->y_raw != nullptr; e.has_act = d->y_act != nullptr;
+  e.valid_units = valid_units; e.rows_per_unit = rows_per_unit;
   e.n_in = e.has_pre + e.has_mask + e.has_post; e.n_out = e.has_raw + e.has_act;
   e.act_slope = d->act == STG_ACT_RELU ? 0.f : (d->act == STG_ACT_LEAKY ? 0.1f : 1.f);
   e.mask_slope = d->mask_mode == STG_ACT_RELU ? 0.f : (d->mask_mode == STG_ACT_LEAKY ? 0.1f : 1.f);
@@ -1423,15 +1454,24 @@ int conv_tc(const StgConv* d, cudaStream_t s) {
     }
     if (r) return STG_ECUDA;
   }
+  using Kernel = decltype(&conv_tc_kernel<true, false, false>);
+  // [kPair][kStaged][kMask]
+  static const Kernel kernels[2][2][2] = {
+      {{conv_tc_kernel<false, false, false>, conv_tc_kernel<false, false, true>},
+       {conv_tc_kernel<true, false, false>, conv_tc_kernel<true, false, true>}},
+      {{conv_tc_kernel<false, true, false>, conv_tc_kernel<false, true, true>},
+       {conv_tc_kernel<true, true, false>, conv_tc_kernel<true, true, true>}}};
   static bool attr_set = false;
   if (!attr_set) {
-    STG_CUDA_CHECK(cudaFuncSetAttribute(conv_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    STG_CUDA_CHECK(cudaFuncSetAttribute(conv_tc_kernel<true, false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    STG_CUDA_CHECK(cudaFuncSetAttribute(conv_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    STG_CUDA_CHECK(cudaFuncSetAttribute(conv_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    STG_CUDA_CHECK(cudaFuncSetAttribute(conv_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    for (int i = 0; i < 8; ++i) {
+      const Kernel k = kernels[i >> 2][(i >> 1) & 1][i & 1];
+      STG_CUDA_CHECK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      if ((i >> 1) == 1)   // staged single-CTA kernels: two may share an SM
+        STG_CUDA_CHECK(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    }
     attr_set = true;
   }
+  const bool masked = valid_units != nullptr;
   p.tiles_n = ceil_div(d->c_dst, p.bn);
   if (pair) {
     const int64_t n_tiles = (int64_t)p.n_res * p.pairs_per_res * p.tiles_n;
@@ -1443,8 +1483,7 @@ int conv_tc(const StgConv* d, cudaStream_t s) {
     cfg.gridDim = dim3(2 * n_pairs); cfg.blockDim = dim3(staged ? 384 : 352); cfg.dynamicSmemBytes = smem; cfg.stream = s;
     cudaLaunchAttribute at[2];
     cfg.attrs = at; cfg.numAttrs = tc_launch_attrs(at, true);
-    if (staged) STG_CUDA_CHECK(cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, true>, tmA, tmW, em, p));
-    else STG_CUDA_CHECK(cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, true>, tmA, tmW, em, p));
+    STG_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernels[1][staged][masked], tmA, tmW, em, p));
     STG_LAUNCH_CHECK();
     return STG_OK;
   }
@@ -1460,8 +1499,7 @@ int conv_tc(const StgConv* d, cudaStream_t s) {
   cfg.gridDim = dim3(grid); cfg.blockDim = dim3(staged ? 384 : 352); cfg.dynamicSmemBytes = smem; cfg.stream = s;
   cudaLaunchAttribute at[2];
   cfg.attrs = at; cfg.numAttrs = tc_launch_attrs(at, false);
-  if (staged) STG_CUDA_CHECK(cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false>, tmA, tmW, em, p));
-  else STG_CUDA_CHECK(cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false>, tmA, tmW, em, p));
+  STG_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernels[0][staged][masked], tmA, tmW, em, p));
   STG_LAUNCH_CHECK();
   return STG_OK;
 }

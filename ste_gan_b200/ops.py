@@ -61,11 +61,14 @@ def conv(src: Tensor, w: Tensor, *, n_samples: int, t_src: int, t_dst: int, c_sr
          pair_sum: bool = False, post_shift: int = 0, mask: Optional[Tensor] = None, mask_mode: int = ACT_NONE,
          act: int = ACT_NONE, dup_rows: bool = False, bias: Optional[Tensor] = None, add_pre: Optional[Tensor] = None,
          add_post: Optional[Tensor] = None, y_raw: Optional[Tensor] = None, y_act: Optional[Tensor] = None,
-         engine: int = ENGINE_AUTO, w_fwd_pack: bool = False, acct_groups: Optional[int] = None) -> None:
+         engine: int = ENGINE_AUTO, w_fwd_pack: bool = False, acct_groups: Optional[int] = None,
+         valid_units: Optional[Tensor] = None, rows_per_unit: int = 1) -> None:
     """One StgConv launch (see include/stegan_b200.h for the exact contraction + epilogue).
     w_fwd_pack (transposed only): `w` is the forward pack wf - what the tcgen05 engine wants for data-gradients.
     acct_groups: the MODULE's group count when `groups` is a (merged) pack-group count - only used to account the
-    algorithmic FLOPs of the launch (block-diagonal packs run redundant MMAs that are not work)."""
+    algorithmic FLOPs of the launch (block-diagonal packs run redundant MMAs that are not work).
+    valid_units (int32 [n_samples] on the device): stg_conv_masked - output rows >= valid_units[b] * rows_per_unit of
+    sample b are written as 0 (forward only)."""
     dt = src.dtype
     nv = n_samples * phases
     t_out = t_dst // 2 if pair_sum else t_dst
@@ -80,6 +83,7 @@ def conv(src: Tensor, w: Tensor, *, n_samples: int, t_src: int, t_dst: int, c_sr
     odt = torch.float32 if out_f32 else dt
     _need(y_raw, nv * t_out * c_dst, odt, "y_raw")
     _need(y_act, nv * t_out * c_dst * (2 if dup_rows else 1), odt, "y_act")
+    _need(valid_units, n_samples, torch.int32, "valid_units")
     d = StgConv(dtype=code_of(dt), engine=_engine_override if _engine_override is not None else engine,
                 n_samples=n_samples, phases=phases, t_src=t_src, t_dst=t_dst, c_src=c_src, c_dst=c_dst, groups=groups,
                 k=k, dilation=dilation, stride=stride, pad=pad, transposed=int(transposed), pair_sum=int(pair_sum),
@@ -87,10 +91,21 @@ def conv(src: Tensor, w: Tensor, *, n_samples: int, t_src: int, t_dst: int, c_sr
                 w_fwd_pack=int(w_fwd_pack), src=_ptr(src), w=_ptr(w), bias=_ptr(bias), add_pre=_ptr(add_pre), mask=_ptr(mask),
                 add_post=_ptr(add_post), y_raw=_ptr(y_raw), y_act=_ptr(y_act))
     lib = _lib.load()
+
+    def launch():
+        if valid_units is None:
+            check(lib.stg_conv(C.byref(d), _stream()), "stg_conv")
+        else:
+            check(lib.stg_conv_masked(C.byref(d), _ptr(valid_units), rows_per_unit, _stream()), "stg_conv_masked")
+
     if profile is None and flop_log is None:
-        check(lib.stg_conv(C.byref(d), _stream()), "stg_conv")
+        launch()
         return
-    route = {1: "simt", 2: "tcgen05", 3: "matvec"}[lib.stg_conv_route(C.byref(d))]
+    if valid_units is None:
+        route = {1: "simt", 2: "tcgen05", 3: "matvec"}[lib.stg_conv_route(C.byref(d))]
+    else:   # stg_conv_masked never takes the matvec engine
+        eng = d.engine if d.engine != ENGINE_AUTO else (ENGINE_TCGEN05 if lib.stg_conv_tc_supported(C.byref(d)) else ENGINE_SIMT)
+        route = "tcgen05" if eng == ENGINE_TCGEN05 else "simt"
     ag = acct_groups if acct_groups is not None else groups
     flops = 2.0 * nv * t_src * c_src * k * (c_dst // ag) if transposed else 2.0 * nv * t_dst * c_dst * k * (c_src // ag)
     esz = 2 if dt == torch.bfloat16 else 4
@@ -101,14 +116,17 @@ def conv(src: Tensor, w: Tensor, *, n_samples: int, t_src: int, t_dst: int, c_sr
     if flop_log is not None:
         flop_log.append(rec)
     if profile is None:
-        check(lib.stg_conv(C.byref(d), _stream()), "stg_conv")
+        launch()
         return
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    check(lib.stg_conv(C.byref(d), _stream()), "stg_conv")
+    launch()
     e1.record()
     rec["ingest"] = _ingest(lib)
-    profile.append(dict(rec, events=(e0, e1), desc=d, fn="stg_conv", keep=(src, w, bias, add_pre, mask, add_post, y_raw, y_act)))
+    # a record replays as fn(desc, *args, stream)
+    fn, args = ("stg_conv", ()) if valid_units is None else ("stg_conv_masked", (_ptr(valid_units), rows_per_unit))
+    profile.append(dict(rec, events=(e0, e1), desc=d, fn=fn, args=args,
+                        keep=(src, w, bias, add_pre, mask, add_post, y_raw, y_act, valid_units)))
 
 
 def _ingest(lib) -> float:

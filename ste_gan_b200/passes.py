@@ -286,8 +286,9 @@ def unfold_input(f: Folded, src: Tensor, B: int, t_src: int, phases: int = 1) ->
 
 def _fwd(f: Folded, src: Tensor, B: int, t_src: int, *, phases: int = 1, act: int = ACT_NONE, want_raw: bool = False,
          want_act: bool = False, dup: bool = False, add_post: Optional[Tensor] = None, post_shift: int = 0,
-         out_f32: bool = False) -> Tuple[Optional[Tensor], Optional[Tensor], int]:
-    """One conv forward.  For an `unfold` layer `src` is the im2col tensor from unfold_input()."""
+         out_f32: bool = False, lengths: Optional[Tensor] = None, rate: int = 1) -> Tuple[Optional[Tensor], Optional[Tensor], int]:
+    """One conv forward.  For an `unfold` layer `src` is the im2col tensor from unfold_input().
+    lengths (int32 [B] frames, optional): output rows >= rate * lengths[b] of sample b are written as 0."""
     m = f.mod
     t_dst = m.t_out(t_src)
     odt = torch.float32 if out_f32 else f.dtype
@@ -295,11 +296,13 @@ def _fwd(f: Folded, src: Tensor, B: int, t_src: int, *, phases: int = 1, act: in
     y_act = torch.empty((B, t_dst * phases * (2 if dup else 1), m.out_channels), device=src.device, dtype=odt) if want_act else None
     if f.unfold:
         ops.conv(src, f.wf, n_samples=B, phases=phases, t_src=t_dst, t_dst=t_dst, c_src=f.kp, c_dst=m.out_channels, k=1,
-                 bias=m.bias.data, act=act, dup_rows=dup, add_post=add_post, post_shift=post_shift, y_raw=y_raw, y_act=y_act)
+                 bias=m.bias.data, act=act, dup_rows=dup, add_post=add_post, post_shift=post_shift, y_raw=y_raw, y_act=y_act,
+                 valid_units=lengths, rows_per_unit=rate)
     else:
         ops.conv(src, f.wf, n_samples=B, phases=phases, t_src=t_src, t_dst=t_dst, c_src=m.in_channels, c_dst=m.out_channels,
                  groups=f.pg, k=m.kernel, dilation=m.dilation, stride=m.stride, pad=m.pad, bias=m.bias.data, act=act,
-                 dup_rows=dup, add_post=add_post, post_shift=post_shift, y_raw=y_raw, y_act=y_act, acct_groups=m.groups)
+                 dup_rows=dup, add_post=add_post, post_shift=post_shift, y_raw=y_raw, y_act=y_act, acct_groups=m.groups,
+                 valid_units=lengths, rows_per_unit=rate)
     return y_raw, y_act, t_dst
 
 
@@ -371,24 +374,28 @@ def generator_convs(model) -> List:
 
 
 def gblock_fwd(blk, folds: Dict[int, Folded], x_raw: Tensor, x_act: Tensor, B: int, t: int, *, want_raw: bool,
-               want_act: bool, dup_next: bool, side=None):
+               want_act: bool, dup_next: bool, side=None, lengths: Optional[Tensor] = None, rate: int = 1):
     """GBlock.forward (layers/conv.py:82-84) on channels-last tensors.
     x_raw [B,t,C_in]: block input; x_act [B,t*up,C_in]: relu(x) with rows duplicated when the block upsamples.
+    lengths (optional): frames per sample, the input having `rate` rows per frame; every output row past a sample's
+    end is written as 0.
     Returns (y_raw|None, relu(y) (rows duplicated if dup_next)|None, saved)."""
     c = blk.convs()
     up = blk.upsample
     t_hi = t * up
+    lo = dict(lengths=lengths, rate=rate)
+    hi = dict(lengths=lengths, rate=rate * up)
     # conv1: ReLU -> [Up] -> conv(d1) -> ReLU -> conv(d3);  res1: [Up] -> conv(k1) on the raw input   (conv.py:38-56,83)
     # the residual 1x1 conv is independent of conv1's first conv: optionally on a side stream
     (r, _, _), (_, a1, _) = fork_join(
-        side, lambda: _fwd(folds[id(c["res"])], x_raw, B, t, want_raw=True),     # 1x1 commutes with nearest upsampling
-        lambda: _fwd(folds[id(c["c1"])], x_act, B, t_hi, act=ACT_RELU, want_act=True))
+        side, lambda: _fwd(folds[id(c["res"])], x_raw, B, t, want_raw=True, **lo),     # 1x1 commutes with nearest upsampling
+        lambda: _fwd(folds[id(c["c1"])], x_act, B, t_hi, act=ACT_RELU, want_act=True, **hi))
     h_raw, h_act, _ = _fwd(folds[id(c["c2"])], a1, B, t_hi, act=ACT_RELU, want_raw=True, want_act=True,
-                           add_post=r, post_shift=1 if up > 1 else 0)
+                           add_post=r, post_shift=1 if up > 1 else 0, **hi)
     # conv2: ReLU -> conv(d9) -> ReLU -> conv(d27);  y = h + conv2(h)                                (conv.py:61-75,84)
-    _, a3, _ = _fwd(folds[id(c["c3"])], h_act, B, t_hi, act=ACT_RELU, want_act=True)
+    _, a3, _ = _fwd(folds[id(c["c3"])], h_act, B, t_hi, act=ACT_RELU, want_act=True, **hi)
     y_raw, y_act, _ = _fwd(folds[id(c["c4"])], a3, B, t_hi, act=ACT_RELU, want_raw=want_raw, want_act=want_act,
-                           add_post=h_raw, dup=dup_next)
+                           add_post=h_raw, dup=dup_next, **hi)
     saved = dict(x_raw=x_raw, x_act=x_act, a1=a1, h_act=h_act, a3=a3, t_lo=t, t_hi=t_hi, up=up)
     return y_raw, y_act, saved
 
@@ -439,8 +446,14 @@ class GenCtx:
 
 
 def generator_forward(model, speech_units: Tensor, session_ids: Optional[Tensor], speaking_mode_ids: Optional[Tensor],
-                      dtype: torch.dtype, need_ctx: bool, folds: Optional[Dict[int, Folded]] = None, side=None):
-    """EMGGeneratorGanTTS.forward (generator.py:140-162).  Returns (x_pred fp32 [B,16T,C], ctx|None)."""
+                      dtype: torch.dtype, need_ctx: bool, folds: Optional[Dict[int, Folded]] = None, side=None,
+                      lengths: Optional[Tensor] = None):
+    """EMGGeneratorGanTTS.forward (generator.py:140-162).  Returns (x_pred fp32 [B,16T,C], ctx|None).
+    lengths (int32 [B] on the device, frames; forward only): sample b is an utterance of lengths[b] frames zero-padded
+    to T.  Every convolution writes 0 past its sample's end, so rows [0, r*lengths[b]) of x_pred[b] are what the
+    utterance gives on its own (r = output rows per frame) and the rows after it are 0, whatever the padded units hold."""
+    if need_ctx and lengths is not None:
+        raise ValueError("generator_forward: length masks are forward-only (need_ctx=True with lengths)")
     su = speech_units.contiguous().float()
     B, T, du = su.shape
     if folds is None:
@@ -467,18 +480,21 @@ def generator_forward(model, speech_units: Tensor, session_ids: Optional[Tensor]
     f0 = folds[id(model.gblocks[0])]
     if f0.unfold:                 # input channels not a multiple of 8 (MFCC variant): zero-padded rows for the tensor engine
         x0 = unfold_input(f0, x0, B, T)
-    x_raw, x_act, t = _fwd(f0, x0, B, T, act=ACT_RELU, want_raw=True, want_act=True, dup=ups[0] > 1)
+    x_raw, x_act, t = _fwd(f0, x0, B, T, act=ACT_RELU, want_raw=True, want_act=True, dup=ups[0] > 1, lengths=lengths)
     saved = []
+    rate = 1                      # rows per unit frame of the current activations
     for i, blk in enumerate(blocks):
         last = i + 1 == len(blocks)
         nxt_dup = (not last) and ups[i + 1] > 1
         y_raw, y_act, s = gblock_fwd(blk, folds, x_raw, x_act, B, t, want_raw=not last, want_act=True, dup_next=nxt_dup,
-                                     side=side)
+                                     side=side, lengths=lengths, rate=rate)
         if need_ctx:
             saved.append(s)
         x_raw, x_act, t = y_raw, y_act, s["t_hi"]
+        rate *= s["up"]
     # last_conv: ReLU -> conv(k3) ; tanh after the channel-last transpose (generator.py:133-137,157-160)
-    _, x_pred, _ = _fwd(folds[id(model.last_conv[1])], x_act, B, t, act=ACT_TANH, want_act=True, out_f32=True)
+    _, x_pred, _ = _fwd(folds[id(model.last_conv[1])], x_act, B, t, act=ACT_TANH, want_act=True, out_f32=True,
+                        lengths=lengths, rate=rate)
     if not need_ctx:
         return x_pred, None
     ctx = GenCtx(B=B, T=T, dtype=dtype, folds=folds, x0=x0, ids=ids, emb_dims=[tb.shape[1] for tb in tables],
