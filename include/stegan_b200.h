@@ -313,13 +313,27 @@ int stg_layernorm_bwd(const void* dy, const void* x, int dtype, const float* sta
  * embeddings added to the keys): qkv [B][L][3*H*d] = (q | k | v), each [H][d] per row, in `dtype`; emb [H][2*max_rel-1][d]
  * float32; logit(i,j) = scale * q_i.k_j + (|j-i| < max_rel ? q_i.emb[h][j-i+max_rel-1] : -1e8); probs [B][H][L][L] float32
  * (softmax, kept for the backward); o [B][L][H*d] = probs * v.  The backward returns dqkv from dout = d/do.
- * One CTA per (sample, head) with its operands in shared memory: L up to ~140 frames at d = 96 (STG_EUNSUPPORTED beyond;
- * the train step has 100-128 frames: chunk_size 1600-2048 EMG samples / 16).
+ * One CTA per (sample, head) with its operands in shared memory, so L is bounded (STG_EUNSUPPORTED beyond):
+ * stg_relattn_dense_supported tells which (L, d) these two calls take; stg_relattn_band_fwd/bwd take any L.
  */
 int stg_relattn_fwd(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel, float scale, void* o,
                     float* probs, stg_stream_t stream);
 int stg_relattn_bwd(const void* qkv, int dtype, const float* emb, const float* probs, const void* dout, int B, int L, int H,
                     int d, int max_rel, float scale, void* dqkv, stg_stream_t stream);
+/* Host-only, no GPU: 1 if stg_relattn_fwd (and, when need_bwd, stg_relattn_bwd) takes (L, d) - the smem rule those calls use
+ * (d = 96: forward up to L = 206, backward up to 133). */
+int stg_relattn_dense_supported(int L, int d, int need_bwd);
+/*
+ * The same attention at any sequence length, tiled over the band |j - i| < max_rel (out-of-band probabilities are exactly 0 in
+ * fp32, so this is the same softmax), in the same fp32 arithmetic.  probs_band [B][H][L][2*max_rel-1] float32: entry (i, w) =
+ * P(i, j = i + w - (max_rel - 1)), exactly 0 where that j lies outside [0, L).  The backward runs in two launches without atomics
+ * (deterministic); scratch [B][H][L] float32 is caller-owned.  STG_EINVAL: a NULL pointer, d % 4 != 0, L < 1, max_rel < 1, an
+ * unknown dtype.  STG_EUNSUPPORTED: d > 128, max_rel > 256, B or H > 65535.  L is not bounded.
+ */
+int stg_relattn_band_fwd(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel, float scale,
+                         void* o, float* probs_band, stg_stream_t stream);
+int stg_relattn_band_bwd(const void* qkv, int dtype, const float* emb, const float* probs_band, const void* dout, int B, int L,
+                         int H, int d, int max_rel, float scale, void* dqkv, float* scratch, stg_stream_t stream);
 /*
  * EMGEncoderLoss (losses/emg_encoder_loss.py:63-84) over N = B*T rows: slots[0] += mean_r ||target_r - pred_r + 1e-6||_2
  * (F.pairwise_distance), slots[1] += mean_r cross_entropy(logits_r, phoneme_r); d_units / d_logits (`grad_dtype`, may be

@@ -2,8 +2,9 @@
 // ste_gan/layers/transformer.py:63-306, ste_gan/losses/emg_encoder_loss.py:56-84) that are not convolutions / GEMMs:
 //   * LayerNorm forward / input-gradient (post-norm transformer layers, transformer.py:54-60)
 //   * multi-head self-attention with per-head learned relative positional logits, forward and input-gradient
-//     (transformer.py:87-113 + LearnedRelativePositionalEmbedding, unmasked, :163-306) - sequence length T/16 = 100-128
-//     frames, head dim 96: one CTA per (sample, head), operands in shared memory, fp32 arithmetic
+//     (transformer.py:87-113 + LearnedRelativePositionalEmbedding, unmasked, :163-306), fp32 arithmetic: one CTA per
+//     (sample, head) with the operands in shared memory where they fit (the train step's T/16 = 100-128 frames at head dim
+//     96), and band-tiled kernels for any sequence length
 //   * speech-unit (mean pairwise L2 distance, eps 1e-6) and phoneme (cross-entropy) losses with their gradients
 // The projections (q/k/v, output, feed-forward, w_raw_in / w_out / w_aux) and the strided ResBlocks with their eval-mode
 // BatchNorm folded into weights and bias run on the tcgen05 convolution engine as k = 1 / k = 3 convs (passes_encoder.py).
@@ -303,6 +304,290 @@ __global__ void __launch_bounds__(512, 1) relattn_bwd_kernel(const T* __restrict
   }
 }
 
+// ---------------------------------------------------------------------------------------------- band-tiled attention (any L)
+// Out-of-band logits are -1e8, so exp(-1e8 - max) is exactly 0 in fp32 and the softmax over the band j in [i-M+1, i+M-1] n [0, L)
+// IS the softmax over the row.  Probabilities are kept in band layout probs_band [B][H][L][W], W = 2M - 1: entry (i, w) is
+// P(i, j = i + w - (M - 1)), exactly 0 where that j lies outside [0, L).
+// One CTA per (query or key tile of BQT rows, head, sample); every warp owns one block of AR rows r0 .. r0 + AR - 1 and meets the
+// partner rows r0 - M + 1 + s, slot s in [0, U), U = W + AR - 1.  Row r of a query block meets slot s at band entry w = s - r, row r
+// of a key block at w = W - 1 - (s - r); either is in the band when 0 <= s - r < W.  The partner rows of the whole tile pass through
+// shared memory in chunks of BKC rows, so shared memory depends on d and M only.  The arithmetic is the dense kernels', term for term.
+constexpr int BNW = 8, BQT = BNW * AR, BKC = 64, BAND_D_MAX = 128, BAND_M_MAX = 256;
+struct BandP { int L, H, d, M, W, U, Up; float scale; };
+
+struct BandTile {               // the indices one warp of a band kernel works with
+  int b, h, r0, nr, s0, lo, hi;
+  int64_t bh;
+  __device__ BandTile(const BandP& p) {
+    b = blockIdx.z; h = blockIdx.y; bh = (int64_t)b * p.H + h;
+    const int t0 = blockIdx.x * BQT;
+    r0 = t0 + (threadIdx.x >> 5) * AR;
+    nr = max(0, min(AR, p.L - r0));                      // rows of this warp's block inside [0, L) (0: the warp only syncs)
+    s0 = r0 - p.M + 1;                                   // partner row of slot 0
+    lo = max(0, t0 - p.M + 1); hi = min(p.L, t0 + BQT + p.M - 1);   // partner rows of the whole tile
+  }
+};
+
+// this warp's AR rows (zero past row L - 1) of a [L][stride] operand -> dst [AR][d]
+template <typename T>
+__device__ __forceinline__ void load_block(const T* __restrict__ base, int64_t stride, int r0, int nr, int d, float* __restrict__ dst) {
+  for (int x = threadIdx.x & 31; x < AR * d; x += 32) {
+    const int r = x / d, c = x - r * d;
+    dst[x] = r < nr ? to_f(base[(int64_t)(r0 + r) * stride + c]) : 0.f;
+  }
+  __syncwarp();
+}
+
+// shared memory (floats): partner chunk [BKC][ds] | per warp: q [AR][d] + logits/probs [AR][Up]      (embedding rows through L1)
+template <typename T>
+__global__ void __launch_bounds__(BNW * 32) relattn_band_fwd_kernel(const T* __restrict__ qkv, const float* __restrict__ emb,
+                                                                    BandP p, T* __restrict__ o, float* __restrict__ probs) {
+  extern __shared__ __align__(16) float sm[];
+  const BandTile t(p);
+  const int L = p.L, d = p.d, ds = d + 4, d4 = d >> 2, M = p.M, W = p.W, U = p.U, Up = p.Up, HD = p.H * d;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nr = t.nr, s0 = t.s0;
+  float* Cs = sm;
+  float* qs = Cs + BKC * ds + warp * (AR * d + AR * Up); float* lg = qs + AR * d;
+  const float* Eh = emb + (int64_t)t.h * W * d;
+  const T* base = qkv + (int64_t)t.b * L * 3 * HD + t.h * d;
+  load_block(base, 3 * HD, t.r0, nr, d, qs);
+  for (int x = lane; x < AR * Up; x += 32) lg[x] = 0.f;                 // every slot defined before the += below
+  __syncwarp();
+  const float4* q4 = reinterpret_cast<const float4*>(qs);
+  for (int w = lane; w < W && nr > 0; w += 32) {                  // positional logits lg[r][w + r] = q_r . emb[w]
+    const float4* e4 = reinterpret_cast<const float4*>(Eh + (int64_t)w * d);
+    float acc[AR] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll 2
+    for (int c = 0; c < d4; ++c) {
+      const float4 e = e4[c];
+#pragma unroll
+      for (int r = 0; r < AR; ++r) acc[r] = dot4(q4[r * d4 + c], e, acc[r]);
+    }
+#pragma unroll
+    for (int r = 0; r < AR; ++r) lg[r * Up + w + r] = acc[r];
+  }
+  for (int c0 = t.lo; c0 < t.hi; c0 += BKC) {                     // + scale * q . k, key chunk by key chunk
+    const int n = min(BKC, t.hi - c0);
+    __syncthreads();
+    load_rows(base + HD + (int64_t)c0 * 3 * HD, 3 * HD, n, d, ds, Cs);
+    __syncthreads();
+    if (nr == 0) continue;
+    for (int j = max(c0, s0) + lane; j < min(c0 + n, s0 + U); j += 32) {
+      const float4* k4 = reinterpret_cast<const float4*>(Cs + (j - c0) * ds);
+      float acc[AR] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll 2
+      for (int c = 0; c < d4; ++c) {
+        const float4 k = k4[c];
+#pragma unroll
+        for (int r = 0; r < AR; ++r) acc[r] = dot4(q4[r * d4 + c], k, acc[r]);
+      }
+#pragma unroll
+      for (int r = 0; r < AR; ++r) lg[r * Up + j - s0] = __fmul_rn(acc[r], p.scale) + lg[r * Up + j - s0];   // slots off row r's
+    }                                                                                                    // band: dropped below
+  }
+  __syncwarp();
+  for (int r = 0; r < nr; ++r) {                                  // softmax of row i over its band
+    float* row = lg + r * Up + r;                                 // row[w] = logit of band entry w
+    const int i = t.r0 + r;
+    float mx = -INFINITY;
+    for (int w = lane; w < W; w += 32) {
+      const int j = i + w - (M - 1);
+      if (j >= 0 && j < L) mx = fmaxf(mx, row[w]);
+    }
+    mx = warp_max_f(mx);
+    float sum = 0.f;
+    for (int w = lane; w < W; w += 32) {
+      const int j = i + w - (M - 1);
+      const float e = j >= 0 && j < L ? __expf(row[w] - mx) : 0.f;
+      row[w] = e; sum += e;
+    }
+    sum = warp_sum_f(sum);
+    const float inv = 1.f / sum;
+    float* pr = probs + (t.bh * L + i) * W;
+    for (int w = lane; w < W; w += 32) { const float pv = row[w] * inv; row[w] = pv; pr[w] = pv; }
+    for (int s = lane; s < U; s += 32)
+      if (s < r || s >= r + W) lg[r * Up + s] = 0.f;
+  }
+  __syncwarp();
+  float4 acc[AR];                                                 // probs . v, 4 output channels per lane (d <= 128)
+#pragma unroll
+  for (int r = 0; r < AR; ++r) acc[r] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int c0 = t.lo; c0 < t.hi; c0 += BKC) {
+    const int n = min(BKC, t.hi - c0);
+    __syncthreads();
+    load_rows(base + 2 * HD + (int64_t)c0 * 3 * HD, 3 * HD, n, d, ds, Cs);
+    __syncthreads();
+    if (nr == 0 || lane >= d4) continue;
+#pragma unroll 2
+    for (int j = max(c0, s0); j < min(c0 + n, s0 + U); ++j) {
+      const float4 v = *reinterpret_cast<const float4*>(Cs + (j - c0) * ds + 4 * lane);
+#pragma unroll
+      for (int r = 0; r < AR; ++r) axpy4(lg[r * Up + j - s0], v, acc[r]);
+    }
+  }
+  if (lane < d4)
+    for (int r = 0; r < nr; ++r) store4(o + ((int64_t)t.b * L + t.r0 + r) * HD + t.h * d + 4 * lane, acc[r], 1.f);
+}
+
+// Backward, query side: dP_ij = dO_i . v_j ; D_i = sum_j dP_ij P_ij (-> Dsc [B][H][L]) ; dS_ij = P_ij (dP_ij - D_i) ;
+// dq_i = sum_j dS_ij (scale k_j + emb[w]).   shared memory (floats): chunk [BKC][ds] | per warp: dO [AR][d] + dP / dS [AR][Up]
+template <typename T>
+__global__ void __launch_bounds__(BNW * 32) relattn_band_bwd_q_kernel(const T* __restrict__ qkv, const float* __restrict__ emb,
+                                                                      const float* __restrict__ probs, const T* __restrict__ dout,
+                                                                      BandP p, T* __restrict__ dqkv, float* __restrict__ Dsc) {
+  extern __shared__ __align__(16) float sm[];
+  const BandTile t(p);
+  const int L = p.L, d = p.d, ds = d + 4, d4 = d >> 2, M = p.M, W = p.W, U = p.U, Up = p.Up, HD = p.H * d;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nr = t.nr, s0 = t.s0;
+  float* Cs = sm;
+  float* gs = Cs + BKC * ds + warp * (AR * d + AR * Up); float* dS = gs + AR * d;
+  const float* Eh = emb + (int64_t)t.h * W * d;
+  const T* base = qkv + (int64_t)t.b * L * 3 * HD + t.h * d;
+  load_block(dout + (int64_t)t.b * L * HD + t.h * d, HD, t.r0, nr, d, gs);
+  for (int x = lane; x < AR * Up; x += 32) dS[x] = 0.f;                 // slots outside the window stay defined
+  __syncwarp();
+  const float4* g4 = reinterpret_cast<const float4*>(gs);
+  for (int c0 = t.lo; c0 < t.hi; c0 += BKC) {                     // dP, value chunk by value chunk
+    const int n = min(BKC, t.hi - c0);
+    __syncthreads();
+    load_rows(base + 2 * HD + (int64_t)c0 * 3 * HD, 3 * HD, n, d, ds, Cs);
+    __syncthreads();
+    if (nr == 0) continue;
+    for (int j = max(c0, s0) + lane; j < min(c0 + n, s0 + U); j += 32) {
+      const float4* v4 = reinterpret_cast<const float4*>(Cs + (j - c0) * ds);
+      float acc[AR] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll 2
+      for (int c = 0; c < d4; ++c) {
+        const float4 v = v4[c];
+#pragma unroll
+        for (int r = 0; r < AR; ++r) acc[r] = dot4(g4[r * d4 + c], v, acc[r]);
+      }
+#pragma unroll
+      for (int r = 0; r < AR; ++r) dS[r * Up + j - s0] = acc[r];
+    }
+  }
+  __syncwarp();
+  for (int r = 0; r < nr; ++r) {
+    const int i = t.r0 + r;
+    const float* pr = probs + (t.bh * L + i) * W;
+    float dsum = 0.f;
+    for (int w = lane; w < W; w += 32) {
+      const int j = i + w - (M - 1);
+      if (j >= 0 && j < L) dsum = fmaf(dS[r * Up + w + r], pr[w], dsum);
+    }
+    dsum = warp_sum_f(dsum);
+    if (lane == 0) Dsc[t.bh * L + i] = dsum;
+    for (int s = lane; s < U; s += 32) {
+      const int w = s - r, j = s0 + s;
+      dS[r * Up + s] = w >= 0 && w < W && j >= 0 && j < L ? pr[w] * (dS[r * Up + s] - dsum) : 0.f;
+    }
+  }
+  __syncwarp();
+  float4 ak[AR], ae[AR];
+#pragma unroll
+  for (int r = 0; r < AR; ++r) { ak[r] = make_float4(0.f, 0.f, 0.f, 0.f); ae[r] = ak[r]; }
+  if (nr > 0 && lane < d4)
+    for (int w = 0; w < W; ++w) {                                 // band entry w of row r is slot w + r
+      const float4 e = *reinterpret_cast<const float4*>(Eh + (int64_t)w * d + 4 * lane);
+#pragma unroll
+      for (int r = 0; r < AR; ++r) axpy4(dS[r * Up + w + r], e, ae[r]);
+    }
+  for (int c0 = t.lo; c0 < t.hi; c0 += BKC) {                     // + sum_j dS_ij k_j, key chunk by key chunk
+    const int n = min(BKC, t.hi - c0);
+    __syncthreads();
+    load_rows(base + HD + (int64_t)c0 * 3 * HD, 3 * HD, n, d, ds, Cs);
+    __syncthreads();
+    if (nr == 0 || lane >= d4) continue;
+#pragma unroll 2
+    for (int j = max(c0, s0); j < min(c0 + n, s0 + U); ++j) {
+      const float4 k = *reinterpret_cast<const float4*>(Cs + (j - c0) * ds + 4 * lane);
+#pragma unroll
+      for (int r = 0; r < AR; ++r) axpy4(dS[r * Up + j - s0], k, ak[r]);
+    }
+  }
+  if (lane < d4)
+    for (int r = 0; r < nr; ++r) {
+      float4 q = ak[r];
+      q.x = q.x * p.scale + ae[r].x; q.y = q.y * p.scale + ae[r].y; q.z = q.z * p.scale + ae[r].z; q.w = q.w * p.scale + ae[r].w;
+      store4(dqkv + ((int64_t)t.b * L + t.r0 + r) * 3 * HD + t.h * d + 4 * lane, q, 1.f);
+    }
+}
+
+// Backward, key side (after the query side has written D): dS_ij = P_ij (dO_i . v_j - D_i) ; dk_j = scale sum_i dS_ij q_i ;
+// dv_j = sum_i P_ij dO_i.   shared memory (floats): chunk [BKC][ds] | per warp: v [AR][d] + dS [AR][Up] + P [AR][Up]
+template <typename T>
+__global__ void __launch_bounds__(BNW * 32) relattn_band_bwd_kv_kernel(const T* __restrict__ qkv, const float* __restrict__ probs,
+                                                                       const T* __restrict__ dout, const float* __restrict__ Dsc,
+                                                                       BandP p, T* __restrict__ dqkv) {
+  extern __shared__ __align__(16) float sm[];
+  const BandTile t(p);
+  const int L = p.L, d = p.d, ds = d + 4, d4 = d >> 2, W = p.W, U = p.U, Up = p.Up, HD = p.H * d;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nr = t.nr, s0 = t.s0;
+  float* Cs = sm;
+  float* vs = Cs + BKC * ds + warp * (AR * d + 2 * AR * Up); float* dS = vs + AR * d; float* Pk = dS + AR * Up;
+  const T* base = qkv + (int64_t)t.b * L * 3 * HD + t.h * d;
+  load_block(base + 2 * HD, 3 * HD, t.r0, nr, d, vs);
+  const float4* v4 = reinterpret_cast<const float4*>(vs);
+  float4 dk[AR], dv[AR];
+#pragma unroll
+  for (int r = 0; r < AR; ++r) { dk[r] = make_float4(0.f, 0.f, 0.f, 0.f); dv[r] = dk[r]; }
+  for (int c0 = t.lo; c0 < t.hi; c0 += BKC) {                     // dS and P of this chunk of queries, then dv
+    const int n = min(BKC, t.hi - c0);
+    __syncthreads();
+    load_rows(dout + (int64_t)t.b * L * HD + t.h * d + (int64_t)c0 * HD, HD, n, d, ds, Cs);
+    __syncthreads();
+    if (nr == 0) continue;
+    const int i_lo = max(c0, s0), i_hi = min(c0 + n, s0 + U);
+    for (int i = i_lo + lane; i < i_hi; i += 32) {
+      const float4* g4 = reinterpret_cast<const float4*>(Cs + (i - c0) * ds);
+      float acc[AR] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll 2
+      for (int c = 0; c < d4; ++c) {
+        const float4 g = g4[c];
+#pragma unroll
+        for (int r = 0; r < AR; ++r) acc[r] = dot4(g, v4[r * d4 + c], acc[r]);
+      }
+      const float* pr = probs + (t.bh * L + i) * W;
+      const float di = Dsc[t.bh * L + i];
+      const int s = i - s0;
+#pragma unroll
+      for (int r = 0; r < AR; ++r) {
+        const int w = W - 1 - (s - r);
+        const float pv = r < nr && w >= 0 && w < W ? pr[w] : 0.f;
+        Pk[r * Up + s] = pv;
+        dS[r * Up + s] = pv * (acc[r] - di);
+      }
+    }
+    __syncwarp();
+    if (lane < d4) {
+#pragma unroll 2
+      for (int i = i_lo; i < i_hi; ++i) {
+        const float4 g = *reinterpret_cast<const float4*>(Cs + (i - c0) * ds + 4 * lane);
+#pragma unroll
+        for (int r = 0; r < AR; ++r) axpy4(Pk[r * Up + i - s0], g, dv[r]);
+      }
+    }
+  }
+  for (int c0 = t.lo; c0 < t.hi; c0 += BKC) {                     // dk, query chunk by query chunk
+    const int n = min(BKC, t.hi - c0);
+    __syncthreads();
+    load_rows(base + (int64_t)c0 * 3 * HD, 3 * HD, n, d, ds, Cs);
+    __syncthreads();
+    if (nr == 0 || lane >= d4) continue;
+#pragma unroll 2
+    for (int i = max(c0, s0); i < min(c0 + n, s0 + U); ++i) {
+      const float4 q = *reinterpret_cast<const float4*>(Cs + (i - c0) * ds + 4 * lane);
+#pragma unroll
+      for (int r = 0; r < AR; ++r) axpy4(dS[r * Up + i - s0], q, dk[r]);
+    }
+  }
+  if (lane < d4)
+    for (int r = 0; r < nr; ++r) {
+      store4(dqkv + ((int64_t)t.b * L + t.r0 + r) * 3 * HD + HD + t.h * d + 4 * lane, dk[r], p.scale);
+      store4(dqkv + ((int64_t)t.b * L + t.r0 + r) * 3 * HD + 2 * HD + t.h * d + 4 * lane, dv[r], 1.f);
+    }
+}
+
 // ---------------------------------------------------------------------------------------------- losses
 // one warp per (b, t) row.  slots[0] += mean_r || tgt_r - pred_r + 1e-6 ||_2          (F.pairwise_distance, eps 1e-6)
 //                           slots[1] += mean_r -log softmax(logits_r)[target_r]       (F.cross_entropy)
@@ -376,15 +661,39 @@ static size_t attn_smem(int L, int d, int n_tiles, int per_warp, int extra, int 
 }
 constexpr size_t ATTN_SMEM_MAX = 226 * 1024;
 
+// Shared memory of the dense (one CTA per head) kernels at (L, d), with the warps they then run: 16 when the per-warp scratch
+// fits beside the operand tiles, else 8.  0: the sequence is too long for them.  (Far past the limits of L and d: no int
+// overflow below.)
+static size_t dense_fwd_smem(int L, int d, int* nw) {
+  if (L > (1 << 16) || d > 4096) return 0;
+  const int Lp = (L + 3) & ~3;
+  const int Lt = (L + 4 + 3) & ~3, pw = 4 * d + 4 * Lp + 4 * Lt;      // per-warp scratch (AR = 4 rows)
+  *nw = 16;
+  size_t smem = attn_smem(L, d, 2, pw, 0, *nw);
+  if (smem > ATTN_SMEM_MAX) { *nw = 8; smem = attn_smem(L, d, 2, pw, 0, *nw); }
+  return smem > ATTN_SMEM_MAX ? 0 : smem;
+}
+static size_t dense_bwd_smem(int L, int d, int* nw) {
+  if (L > (1 << 16) || d > 4096) return 0;
+  const int Lp = (L + 3) & ~3;
+  *nw = 16;
+  size_t smem = attn_smem(L, d, 4, 4 * Lp, Lp, *nw);
+  if (smem > ATTN_SMEM_MAX) { *nw = 8; smem = attn_smem(L, d, 4, 4 * Lp, Lp, *nw); }
+  return smem > ATTN_SMEM_MAX ? 0 : smem;
+}
+
+extern "C" int stg_relattn_dense_supported(int L, int d, int need_bwd) {
+  int nw;
+  if (L < 1 || d < 4 || (d & 3)) return 0;
+  return dense_fwd_smem(L, d, &nw) != 0 && (!need_bwd || dense_bwd_smem(L, d, &nw) != 0);
+}
+
 extern "C" int stg_relattn_fwd(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel, float scale,
                                void* o, float* probs, stg_stream_t stream) {
   if (!qkv || !emb || !o || !probs || B < 1 || L < 1 || H < 1 || d < 4 || (d & 3) || max_rel < 1) return STG_EINVAL;
-  const int Lp = (L + 3) & ~3;
-  const int Lt = (L + 4 + 3) & ~3, pw = 4 * d + 4 * Lp + 4 * Lt;      // per-warp scratch (AR = 4 rows)
-  int nw = 16;                                          // 16 warps when their scratch fits beside the operand tiles, else 8
-  size_t smem = attn_smem(L, d, 2, pw, 0, nw);
-  if (smem > ATTN_SMEM_MAX) { nw = 8; smem = attn_smem(L, d, 2, pw, 0, nw); }
-  if (smem > ATTN_SMEM_MAX) return STG_EUNSUPPORTED;    // sequence too long for the one-CTA-per-head kernel
+  int nw;
+  const size_t smem = dense_fwd_smem(L, d, &nw);
+  if (!smem) return STG_EUNSUPPORTED;                   // sequence too long for the one-CTA-per-head kernel: stg_relattn_band_fwd
   AttnP p{B, L, H, d, max_rel, scale};
   if (dtype == STG_F32) {
     STG_CUDA_CHECK(cudaFuncSetAttribute(relattn_fwd_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
@@ -400,11 +709,9 @@ extern "C" int stg_relattn_fwd(const void* qkv, int dtype, const float* emb, int
 extern "C" int stg_relattn_bwd(const void* qkv, int dtype, const float* emb, const float* probs, const void* dout, int B, int L,
                                int H, int d, int max_rel, float scale, void* dqkv, stg_stream_t stream) {
   if (!qkv || !emb || !probs || !dout || !dqkv || B < 1 || L < 1 || H < 1 || d < 4 || (d & 3) || max_rel < 1) return STG_EINVAL;
-  const int Lp = (L + 3) & ~3;
-  int nw = 16;
-  size_t smem = attn_smem(L, d, 4, 4 * Lp, Lp, nw);
-  if (smem > ATTN_SMEM_MAX) { nw = 8; smem = attn_smem(L, d, 4, 4 * Lp, Lp, nw); }
-  if (smem > ATTN_SMEM_MAX) return STG_EUNSUPPORTED;
+  int nw;
+  const size_t smem = dense_bwd_smem(L, d, &nw);
+  if (!smem) return STG_EUNSUPPORTED;
   AttnP p{B, L, H, d, max_rel, scale};
   if (dtype == STG_F32) {
     STG_CUDA_CHECK(cudaFuncSetAttribute(relattn_bwd_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
@@ -415,6 +722,61 @@ extern "C" int stg_relattn_bwd(const void* qkv, int dtype, const float* emb, con
   } else return STG_EINVAL;
   STG_LAUNCH_CHECK();
   return STG_OK;
+}
+
+// Band kernels: argument checks, then the bounds of the kernels (d <= 128: one float4 of channels per lane; the grid's y / z
+// dimensions).  The sequence length is not bounded.  Shared memory depends on d and max_rel only: <= 182 KB at the bounds.
+static int band_params(int B, int L, int H, int d, int max_rel, float scale, BandP* p, dim3* grid) {
+  if (B < 1 || L < 1 || H < 1 || d < 4 || (d & 3) || max_rel < 1) return STG_EINVAL;
+  if (d > BAND_D_MAX || max_rel > BAND_M_MAX || B > 65535 || H > 65535) return STG_EUNSUPPORTED;
+  const int W = 2 * max_rel - 1, U = W + AR - 1;
+  *p = BandP{L, H, d, max_rel, W, U, (U + 3) & ~3, scale};
+  *grid = dim3((unsigned)((L + BQT - 1) / BQT), (unsigned)H, (unsigned)B);
+  return STG_OK;
+}
+static size_t band_smem(const BandP& p, int per_warp_rows) {
+  return sizeof(float) * ((size_t)BKC * (p.d + 4) + (size_t)BNW * (AR * p.d + per_warp_rows * AR * p.Up));
+}
+
+template <typename T>
+static int band_fwd(const T* qkv, const float* emb, const BandP& p, dim3 grid, T* o, float* probs, cudaStream_t s) {
+  const size_t smem = band_smem(p, 1);
+  STG_CUDA_CHECK(cudaFuncSetAttribute(relattn_band_fwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  relattn_band_fwd_kernel<T><<<grid, BNW * 32, smem, s>>>(qkv, emb, p, o, probs);
+  STG_LAUNCH_CHECK();
+  return STG_OK;
+}
+
+template <typename T>
+static int band_bwd(const T* qkv, const float* emb, const float* probs, const T* dout, const BandP& p, dim3 grid, T* dqkv,
+                    float* scratch, cudaStream_t s) {
+  const size_t sq = band_smem(p, 1), skv = band_smem(p, 2);
+  STG_CUDA_CHECK(cudaFuncSetAttribute(relattn_band_bwd_q_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sq));
+  STG_CUDA_CHECK(cudaFuncSetAttribute(relattn_band_bwd_kv_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)skv));
+  relattn_band_bwd_q_kernel<T><<<grid, BNW * 32, sq, s>>>(qkv, emb, probs, dout, p, dqkv, scratch);
+  STG_LAUNCH_CHECK();
+  relattn_band_bwd_kv_kernel<T><<<grid, BNW * 32, skv, s>>>(qkv, probs, dout, scratch, p, dqkv);
+  STG_LAUNCH_CHECK();
+  return STG_OK;
+}
+
+extern "C" int stg_relattn_band_fwd(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel,
+                                    float scale, void* o, float* probs_band, stg_stream_t stream) {
+  if (!qkv || !emb || !o || !probs_band || (dtype != STG_F32 && dtype != STG_BF16)) return STG_EINVAL;
+  BandP p; dim3 grid;
+  if (const int rc = band_params(B, L, H, d, max_rel, scale, &p, &grid)) return rc;
+  if (dtype == STG_F32) return band_fwd((const float*)qkv, emb, p, grid, (float*)o, probs_band, S_);
+  return band_fwd((const bf16*)qkv, emb, p, grid, (bf16*)o, probs_band, S_);
+}
+
+extern "C" int stg_relattn_band_bwd(const void* qkv, int dtype, const float* emb, const float* probs_band, const void* dout, int B,
+                                    int L, int H, int d, int max_rel, float scale, void* dqkv, float* scratch, stg_stream_t stream) {
+  if (!qkv || !emb || !probs_band || !dout || !dqkv || !scratch || (dtype != STG_F32 && dtype != STG_BF16)) return STG_EINVAL;
+  BandP p; dim3 grid;
+  if (const int rc = band_params(B, L, H, d, max_rel, scale, &p, &grid)) return rc;
+  if (dtype == STG_F32)
+    return band_bwd((const float*)qkv, emb, probs_band, (const float*)dout, p, grid, (float*)dqkv, scratch, S_);
+  return band_bwd((const bf16*)qkv, emb, probs_band, (const bf16*)dout, p, grid, (bf16*)dqkv, scratch, S_);
 }
 
 extern "C" int stg_encoder_losses(const float* unit_pred, const float* unit_target, const float* phoneme_logits,

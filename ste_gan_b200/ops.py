@@ -608,6 +608,38 @@ def relattn_bwd(qkv: Tensor, emb: Tensor, probs: Tensor, dout: Tensor, n_head: i
     return dqkv
 
 
+def relattn_dense_supported(L: int, d: int, need_bwd: bool) -> bool:
+    """Whether relattn_fwd (and, with need_bwd, relattn_bwd) take sequence length L at head dim d (host-only query)."""
+    return bool(_lib.load().stg_relattn_dense_supported(int(L), int(d), int(bool(need_bwd))))
+
+
+def relattn_band_fwd(qkv: Tensor, emb: Tensor, n_head: int, max_rel: int) -> Tuple[Tensor, Tensor]:
+    """relattn_fwd at any L -> (o [B, L, H*d], probs_band fp32 [B, H, L, 2*max_rel-1]): entry (i, w) is the probability of key
+    j = i + w - (max_rel - 1), 0 where that j is outside [0, L)."""
+    B, L, C3 = qkv.shape
+    d = C3 // (3 * n_head)
+    _need(qkv, B * L * C3, None, "qkv"); _need(emb, n_head * (2 * max_rel - 1) * d, torch.float32, "emb")
+    o = torch.empty((B, L, n_head * d), device=qkv.device, dtype=qkv.dtype)
+    probs = torch.empty((B, n_head, L, 2 * max_rel - 1), device=qkv.device, dtype=torch.float32)
+    check(_lib.load().stg_relattn_band_fwd(_ptr(qkv), code_of(qkv.dtype), _ptr(emb), B, L, n_head, d, max_rel, float(d) ** -0.5,
+                                           _ptr(o), _ptr(probs), _stream()), "stg_relattn_band_fwd")
+    return o, probs
+
+
+def relattn_band_bwd(qkv: Tensor, emb: Tensor, probs: Tensor, dout: Tensor, n_head: int, max_rel: int) -> Tensor:
+    """Input gradient of relattn_band_fwd from its band-layout probabilities."""
+    B, L, C3 = qkv.shape
+    d = C3 // (3 * n_head)
+    _need(qkv, B * L * C3, None, "qkv"); _need(dout, B * L * n_head * d, qkv.dtype, "dout")
+    _need(emb, n_head * (2 * max_rel - 1) * d, torch.float32, "emb")
+    _need(probs, B * n_head * L * (2 * max_rel - 1), torch.float32, "probs")
+    dqkv = torch.empty_like(qkv)
+    scratch = torch.empty((B, n_head, L), device=qkv.device, dtype=torch.float32)
+    check(_lib.load().stg_relattn_band_bwd(_ptr(qkv), code_of(qkv.dtype), _ptr(emb), _ptr(probs), _ptr(dout), B, L, n_head, d,
+                                           max_rel, float(d) ** -0.5, _ptr(dqkv), _ptr(scratch), _stream()), "stg_relattn_band_bwd")
+    return dqkv
+
+
 def encoder_losses(unit_pred: Tensor, unit_target: Tensor, logits: Tensor, phoneme_target: Tensor, slots: Tensor,
                    gs_units: float = 0.0, gs_phonemes: float = 0.0, grad_dtype: Optional[torch.dtype] = None):
     """slots[0] += speech-unit loss, slots[1] += phoneme loss; returns (d_units, d_logits) in grad_dtype (None: no gradients)."""

@@ -148,13 +148,15 @@ def encoder_forward(plan: EncoderPlan, emg: Tensor, need_ctx: bool = True):
     saved_layers = []
     for ly in plan.layers:
         qkv, _, _ = _fwd(ly.qkv, xl, B, L, want_raw=True)
-        o, probs = ops.relattn_fwd(qkv, ly.emb, ly.n_head, ly.max_rel)
+        # the one-CTA-per-head kernels where they take L (for the backward too, when it follows), the band-tiled ones beyond
+        band = not ops.relattn_dense_supported(L, qkv.shape[-1] // (3 * ly.n_head), need_ctx)
+        o, probs = (ops.relattn_band_fwd if band else ops.relattn_fwd)(qkv, ly.emb, ly.n_head, ly.max_rel)
         pre1, _, _ = _fwd(ly.out, o, B, L, want_raw=True, add_post=xl)                          # src + attn        (transformer.py:54-55)
         x1, st1 = ops.layernorm(pre1, ly.g1, ly.b1, LN_EPS)                                     # norm1             (:56)
         _, hff, _ = _fwd(ly.l1, x1, B, L, act=ACT_RELU, want_act=True)                          # relu(linear1)     (:57)
         pre2, _, _ = _fwd(ly.l2, hff, B, L, want_raw=True, add_post=x1)                         # src + linear2     (:57-58)
         x2, st2 = ops.layernorm(pre2, ly.g2, ly.b2, LN_EPS)                                     # norm2             (:59)
-        saved_layers.append(dict(qkv=qkv, probs=probs, pre1=pre1, st1=st1, hff=hff, pre2=pre2, st2=st2))
+        saved_layers.append(dict(qkv=qkv, probs=probs, band=band, pre1=pre1, st1=st1, hff=hff, pre2=pre2, st2=st2))
         xl = x2
     units, _, _ = _fwd(plan.w_out, xl, B, L, want_raw=True, out_f32=True)                       # emg_encoder.py:88
     logits, _, _ = _fwd(plan.w_aux, xl, B, L, want_raw=True, out_f32=True)
@@ -176,7 +178,7 @@ def encoder_backward(plan: EncoderPlan, ctx: EncCtx, d_units: Optional[Tensor], 
         dx1 = _dgrad(ly.l1, dh, B, L, L, add_post=dpre2)
         dpre1 = ops.layernorm_bwd(dx1, s["pre1"], s["st1"], ly.g1)
         do = _dgrad(ly.out, dpre1, B, L, L)
-        dqkv = ops.relattn_bwd(s["qkv"], ly.emb, s["probs"], do, ly.n_head, ly.max_rel)
+        dqkv = (ops.relattn_band_bwd if s["band"] else ops.relattn_bwd)(s["qkv"], ly.emb, s["probs"], do, ly.n_head, ly.max_rel)
         dx = _dgrad(ly.qkv, dqkv, B, L, L, add_post=dpre1)
     # w_raw_in, then the ReLU of the last ResBlock (its saved output is the mask)
     dz = _dgrad(plan.w_in, dx, B, L, L, mask=ctx.y_last, mask_mode=ACT_RELU)
