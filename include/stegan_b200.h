@@ -335,6 +335,18 @@ int stg_relattn_band_fwd(const void* qkv, int dtype, const float* emb, int B, in
 int stg_relattn_band_bwd(const void* qkv, int dtype, const float* emb, const float* probs_band, const void* dout, int B, int L,
                          int H, int d, int max_rel, float scale, void* dqkv, float* scratch, stg_stream_t stream);
 /*
+ * The two forwards with per-sample key-length masks, for batches of utterances padded to a common length L: sample b holds
+ * Lb = lengths[b] rows (a DEVICE array of B ints, read at execution time, so a captured graph serves any length mix; negative
+ * counts as 0, more than L as L).  Lb replaces L in every bound of the kernel, so each row i < Lb is bit-identical to the same
+ * call at B = 1, L = Lb; rows i >= Lb of o and of the probabilities are 0, and so are the probabilities of keys j >= Lb.  Padded
+ * q / k / v rows are never read into a kept row, NaN included.  L stays the row stride of qkv, o and the probabilities.
+ * Forward only.  STG_EINVAL on a NULL `lengths`, otherwise the arguments and return codes of the unmasked calls.
+ */
+int stg_relattn_fwd_masked(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel, float scale,
+                           void* o, float* probs, const int32_t* lengths, stg_stream_t stream);
+int stg_relattn_band_fwd_masked(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel, float scale,
+                                void* o, float* probs_band, const int32_t* lengths, stg_stream_t stream);
+/*
  * EMGEncoderLoss (losses/emg_encoder_loss.py:63-84) over N = B*T rows: slots[0] += mean_r ||target_r - pred_r + 1e-6||_2
  * (F.pairwise_distance), slots[1] += mean_r cross_entropy(logits_r, phoneme_r); d_units / d_logits (`grad_dtype`, may be
  * NULL) = gs_units * d slots[0] / d pred and gs_phonemes * d slots[1] / d logits.
@@ -342,6 +354,17 @@ int stg_relattn_band_bwd(const void* qkv, int dtype, const float* emb, const flo
 int stg_encoder_losses(const float* unit_pred, const float* unit_target, const float* phoneme_logits,
                        const int64_t* phoneme_target, int N, int Du, int P, float* slots, float gs_units, float gs_phonemes,
                        void* d_units, void* d_logits, int grad_dtype, stg_stream_t stream);
+/*
+ * EMGEncoderLoss per utterance of a padded batch (losses/emg_encoder_loss.py:19-84): unit_pred / unit_target [B][T][Du],
+ * phoneme_logits [B][T][P] float32, phoneme_target [B][T] int64; sample b holds n = clamp(lengths[b], 0, T) frames (DEVICE
+ * int32 [B]) and rows t >= n are never read.  sums [B][2] = (sum_t ||target_t - pred_t + 1e-6||_2, sum_t cross_entropy_t);
+ * counts [B][4] int32 = (n, argmax_t == target_t, target_t == silence_index, both of those and target_t != silence_index);
+ * argmax takes the first maximum, as torch.argmax.  A target outside [0, P) makes that utterance's cross-entropy sum NaN.
+ * Fixed-order reductions without atomics: replays are bit-identical.  STG_EINVAL: a NULL pointer, B, T, Du or P < 1.
+ */
+int stg_encoder_scores(const float* unit_pred, const float* unit_target, const float* phoneme_logits,
+                       const int64_t* phoneme_target, const int32_t* lengths, int B, int T, int Du, int P, int silence_index,
+                       float* sums, int32_t* counts, stg_stream_t stream);
 
 /* torch.optim.AdamW (ste_gan/constants.py:57; train.py:80-81,199,267) over one flat fp32 buffer.
  * step_count is a device int64 (incremented by the kernel) so the update is CUDA-graph capturable.

@@ -102,7 +102,10 @@ _SIGS = {
     "stg_relattn_dense_supported": [_I, _I, _I],
     "stg_relattn_band_fwd": [_P, _I, _P, _I, _I, _I, _I, _I, _F, _P, _P, _P],
     "stg_relattn_band_bwd": [_P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P, _P, _P],
+    "stg_relattn_fwd_masked": [_P, _I, _P, _I, _I, _I, _I, _I, _F, _P, _P, _P, _P],
+    "stg_relattn_band_fwd_masked": [_P, _I, _P, _I, _I, _I, _I, _I, _F, _P, _P, _P, _P],
     "stg_encoder_losses": [_P, _P, _P, _P, _I, _I, _I, _P, _F, _F, _P, _P, _I, _P],
+    "stg_encoder_scores": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P],
     "stg_adamw": [_P, _P, _P, _P, _L, _F, _P, _F, _F, _F, _F, _P, _F, _P, _I, _P],
 }
 EXPORTS = sorted(list(_SIGS) + ["stg_strerror", "stg_last_cuda_error", "stg_version", "stg_launch_count", "stg_set_sm_limit",

@@ -99,22 +99,42 @@ __device__ __forceinline__ void store4(T* p, const float4& v, float s) {
 // -> 4-row blocks: see DESIGN.md section 3.5.
 constexpr int AR = 4;
 
+// Key-length masks (kMask, stg_relattn_fwd_masked / stg_relattn_band_fwd_masked): sample b holds Lb = clamp(lengths[b], 0, L)
+// rows.  Lb replaces L in every bound of the arithmetic (L stays the memory stride), so a kept row runs the loops, lanes and
+// summation order of the same kernel at (B = 1, L = Lb) and is bit-identical to it; padded K / V rows are skipped, never
+// multiplied by a zero probability (0 * NaN = NaN).  Query rows >= Lb get o = 0 and an all-zero probability row.
+template <bool kMask>
+__device__ __forceinline__ int valid_len(const int32_t* __restrict__ lengths, int b, int L) {
+  if constexpr (kMask) return min(max(lengths[b], 0), L);
+  return L;
+}
+
 // shared memory (floats): K [L][ds] | V [L][ds] | per warp: q [AR][d] + logits/probs [AR][Lp] + positional logits [AR][Lt]
 // (d % 4 == 0, Lp = roundup4(L), Lt = roundup4(L + AR)); the head's embedding rows are read through L1.
-template <typename T>
+template <typename T, bool kMask>
 __global__ void __launch_bounds__(512, 1) relattn_fwd_kernel(const T* __restrict__ qkv, const float* __restrict__ emb, AttnP p,
-                                                          T* __restrict__ o, float* __restrict__ probs) {
+                                                          T* __restrict__ o, float* __restrict__ probs,
+                                                          const int32_t* __restrict__ lengths) {
   extern __shared__ __align__(16) float sm[];
   const int b = blockIdx.x / p.H, h = blockIdx.x - b * p.H;
-  const int L = p.L, d = p.d, ds = d + 4, d4 = d >> 2, M = p.M, HD = p.H * d, Lp = (L + 3) & ~3, Lt = (L + AR + 3) & ~3;
+  const int L = valid_len<kMask>(lengths, b, p.L), d = p.d, ds = d + 4, d4 = d >> 2, M = p.M, HD = p.H * d;
+  const int Ls = p.L, Lp = (Ls + 3) & ~3, Lt = (Ls + AR + 3) & ~3;     // L: rows of the sample; Ls: rows in memory
   float* Ks = sm; float* Vs = Ks + L * ds; float* wsc = Vs + L * ds;
   const int nw = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* qs = wsc + warp * (AR * d + AR * Lp + AR * Lt); float* lg = qs + AR * d; float* ts = lg + AR * Lp;
   const float* Eh = emb + (int64_t)h * (2 * M - 1) * d;
-  const T* base = qkv + (int64_t)b * L * 3 * HD + h * d;
+  const T* base = qkv + (int64_t)b * Ls * 3 * HD + h * d;
   load_rows(base + HD, 3 * HD, L, d, ds, Ks);
   load_rows(base + 2 * HD, 3 * HD, L, d, ds, Vs);
   __syncthreads();
+  if constexpr (kMask) {                                          // rows / keys past the sample's end: exactly 0
+    for (int i = warp; i < Ls; i += nw) {
+      float* pr = probs + (((int64_t)b * p.H + h) * Ls + i) * Ls;
+      for (int j = (i < L ? L : 0) + lane; j < Ls; j += 32) pr[j] = 0.f;
+      if (i >= L)
+        for (int c = lane; c < d; c += 32) o[((int64_t)b * Ls + i) * HD + h * d + c] = from_f<T>(0.f);
+    }
+  }
   for (int ib = warp * AR; ib < L; ib += nw * AR) {
     const int nr = min(AR, L - ib);
     for (int x = lane; x < AR * d; x += 32) {
@@ -164,7 +184,7 @@ __global__ void __launch_bounds__(512, 1) relattn_fwd_kernel(const T* __restrict
       for (int j = lane; j < L; j += 32) { const float e = __expf(row[j] - mx); row[j] = e; sum += e; }
       sum = warp_sum_f(sum);
       const float inv = 1.f / sum;
-      float* pr = probs + (((int64_t)b * p.H + h) * L + ib + r) * L;
+      float* pr = probs + (((int64_t)b * p.H + h) * Ls + ib + r) * Ls;
       for (int j = lane; j < L; j += 32) { const float pv = row[j] * inv; row[j] = pv; pr[j] = pv; }
     }
     __syncwarp();
@@ -178,7 +198,7 @@ __global__ void __launch_bounds__(512, 1) relattn_fwd_kernel(const T* __restrict
 #pragma unroll
         for (int r = 0; r < AR; ++r) axpy4(lg[r * Lp + j], v, acc[r]);
       }
-      for (int r = 0; r < nr; ++r) store4(o + ((int64_t)b * L + ib + r) * HD + h * d + 4 * c, acc[r], 1.f);
+      for (int r = 0; r < nr; ++r) store4(o + ((int64_t)b * Ls + ib + r) * HD + h * d + 4 * c, acc[r], 1.f);
     }
     __syncwarp();
   }
@@ -339,17 +359,30 @@ __device__ __forceinline__ void load_block(const T* __restrict__ base, int64_t s
 }
 
 // shared memory (floats): partner chunk [BKC][ds] | per warp: q [AR][d] + logits/probs [AR][Up]      (embedding rows through L1)
-template <typename T>
+template <typename T, bool kMask>
 __global__ void __launch_bounds__(BNW * 32) relattn_band_fwd_kernel(const T* __restrict__ qkv, const float* __restrict__ emb,
-                                                                    BandP p, T* __restrict__ o, float* __restrict__ probs) {
+                                                                    BandP p, T* __restrict__ o, float* __restrict__ probs,
+                                                                    const int32_t* __restrict__ lengths) {
   extern __shared__ __align__(16) float sm[];
-  const BandTile t(p);
-  const int L = p.L, d = p.d, ds = d + 4, d4 = d >> 2, M = p.M, W = p.W, U = p.U, Up = p.Up, HD = p.H * d;
+  const int L = valid_len<kMask>(lengths, blockIdx.z, p.L), Ls = p.L;  // L: rows of the sample; Ls: rows in memory
+  BandTile t(p);
+  if constexpr (kMask) {                                          // L replaces p.L in both bounds of the tile
+    t.nr = max(0, min(AR, L - t.r0));
+    t.hi = min(L, (int)blockIdx.x * BQT + BQT + p.M - 1);
+  }
+  const int d = p.d, ds = d + 4, d4 = d >> 2, M = p.M, W = p.W, U = p.U, Up = p.Up, HD = p.H * d;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nr = t.nr, s0 = t.s0;
   float* Cs = sm;
   float* qs = Cs + BKC * ds + warp * (AR * d + AR * Up); float* lg = qs + AR * d;
   const float* Eh = emb + (int64_t)t.h * W * d;
-  const T* base = qkv + (int64_t)t.b * L * 3 * HD + t.h * d;
+  const T* base = qkv + (int64_t)t.b * Ls * 3 * HD + t.h * d;
+  if constexpr (kMask) {                                          // this warp's rows in [L, Ls): o = 0, probabilities 0
+    for (int r = nr; r < min(AR, Ls - t.r0); ++r) {
+      float* pr = probs + (t.bh * Ls + t.r0 + r) * W;
+      for (int w = lane; w < W; w += 32) pr[w] = 0.f;
+      for (int c = lane; c < d; c += 32) o[((int64_t)t.b * Ls + t.r0 + r) * HD + t.h * d + c] = from_f<T>(0.f);
+    }
+  }
   load_block(base, 3 * HD, t.r0, nr, d, qs);
   for (int x = lane; x < AR * Up; x += 32) lg[x] = 0.f;                 // every slot defined before the += below
   __syncwarp();
@@ -403,7 +436,7 @@ __global__ void __launch_bounds__(BNW * 32) relattn_band_fwd_kernel(const T* __r
     }
     sum = warp_sum_f(sum);
     const float inv = 1.f / sum;
-    float* pr = probs + (t.bh * L + i) * W;
+    float* pr = probs + (t.bh * Ls + i) * W;
     for (int w = lane; w < W; w += 32) { const float pv = row[w] * inv; row[w] = pv; pr[w] = pv; }
     for (int s = lane; s < U; s += 32)
       if (s < r || s >= r + W) lg[r * Up + s] = 0.f;
@@ -426,7 +459,7 @@ __global__ void __launch_bounds__(BNW * 32) relattn_band_fwd_kernel(const T* __r
     }
   }
   if (lane < d4)
-    for (int r = 0; r < nr; ++r) store4(o + ((int64_t)t.b * L + t.r0 + r) * HD + t.h * d + 4 * lane, acc[r], 1.f);
+    for (int r = 0; r < nr; ++r) store4(o + ((int64_t)t.b * Ls + t.r0 + r) * HD + t.h * d + 4 * lane, acc[r], 1.f);
 }
 
 // Backward, query side: dP_ij = dO_i . v_j ; D_i = sum_j dP_ij P_ij (-> Dsc [B][H][L]) ; dS_ij = P_ij (dP_ij - D_i) ;
@@ -627,6 +660,62 @@ __global__ void __launch_bounds__(256) encoder_loss_kernel(const float* __restri
   }
 }
 
+// Per-utterance scores (stg_encoder_scores): one CTA of SC_W warps per sample b over its n_b = clamp(lengths[b], 0, T) rows;
+// warp w takes rows w, w + SC_W, ...  sums[b] = (sum_r ||tgt_r - pred_r + 1e-6||_2, sum_r CE_r); counts[b] = (rows, argmax ==
+// target, target == silence, both and target != silence).  Per-warp partial sums in a fixed row order, then a fixed-order sum
+// over the warps: no atomics, so replays are bit-identical.  A target outside [0, P) is not read through: its CE is NaN.
+constexpr int SC_W = 8;
+__global__ void __launch_bounds__(SC_W * 32) encoder_scores_kernel(const float* __restrict__ pred, const float* __restrict__ tgt,
+                                                                   const float* __restrict__ logits, const int64_t* __restrict__ ph,
+                                                                   const int32_t* __restrict__ lengths, int T, int Du, int P,
+                                                                   int silence, float* __restrict__ sums, int32_t* __restrict__ counts) {
+  __shared__ float s_sum[SC_W][2];
+  __shared__ int s_cnt[SC_W][3];
+  const int b = blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int n = min(max(lengths[b], 0), T);
+  float su = 0.f, ce = 0.f;
+  int correct = 0, sil = 0, correct_ns = 0;
+  for (int t = warp; t < n; t += SC_W) {
+    const int64_t row = (int64_t)b * T + t;
+    const float* pr = pred + row * Du; const float* tr = tgt + row * Du;
+    float ss = 0.f;
+    for (int i = lane; i < Du; i += 32) { const float df = tr[i] - pr[i] + 1e-6f; ss = fmaf(df, df, ss); }
+    su += sqrtf(warp_sum_f(ss));
+    const float* lr = logits + row * P;
+    float mx = -INFINITY;
+    int arg = P;
+    for (int i = lane; i < P; i += 32)
+      if (lr[i] > mx || arg == P) { mx = lr[i]; arg = i; }                   // first maximum of this lane's entries
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {                                      // first maximum of the row (torch.argmax)
+      const float m2 = __shfl_xor_sync(0xffffffffu, mx, o);
+      const int a2 = __shfl_xor_sync(0xffffffffu, arg, o);
+      if (m2 > mx || (m2 == mx && a2 < arg)) { mx = m2; arg = a2; }
+    }
+    float se = 0.f;
+    for (int i = lane; i < P; i += 32) se += __expf(lr[i] - mx);
+    se = warp_sum_f(se);
+    const int64_t k = ph[row];
+    const bool in = k >= 0 && k < P;
+    ce += in ? mx + __logf(se) - lr[in ? k : 0] : __int_as_float(0x7fffffff);
+    correct += arg == k;
+    sil += k == silence;
+    correct_ns += arg == k && k != silence;
+  }
+  if (lane == 0) {
+    s_sum[warp][0] = su; s_sum[warp][1] = ce;
+    s_cnt[warp][0] = correct; s_cnt[warp][1] = sil; s_cnt[warp][2] = correct_ns;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float a = 0.f, c = 0.f;
+    int k0 = 0, k1 = 0, k2 = 0;
+    for (int w = 0; w < SC_W; ++w) { a += s_sum[w][0]; c += s_sum[w][1]; k0 += s_cnt[w][0]; k1 += s_cnt[w][1]; k2 += s_cnt[w][2]; }
+    sums[2 * b] = a; sums[2 * b + 1] = c;
+    counts[4 * b] = n; counts[4 * b + 1] = k0; counts[4 * b + 2] = k1; counts[4 * b + 3] = k2;
+  }
+}
+
 }  // namespace
 }  // namespace stg
 
@@ -688,22 +777,37 @@ extern "C" int stg_relattn_dense_supported(int L, int d, int need_bwd) {
   return dense_fwd_smem(L, d, &nw) != 0 && (!need_bwd || dense_bwd_smem(L, d, &nw) != 0);
 }
 
-extern "C" int stg_relattn_fwd(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel, float scale,
-                               void* o, float* probs, stg_stream_t stream) {
+template <typename T, bool kMask>
+static int dense_fwd(const T* qkv, const float* emb, const AttnP& p, int nw, size_t smem, T* o, float* probs,
+                     const int32_t* lengths, cudaStream_t s) {
+  STG_CUDA_CHECK(cudaFuncSetAttribute(relattn_fwd_kernel<T, kMask>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  relattn_fwd_kernel<T, kMask><<<p.B * p.H, 32 * nw, smem, s>>>(qkv, emb, p, o, probs, lengths);
+  STG_LAUNCH_CHECK();
+  return STG_OK;
+}
+
+template <bool kMask>
+static int relattn_fwd_any(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel, float scale,
+                           void* o, float* probs, const int32_t* lengths, cudaStream_t s) {
   if (!qkv || !emb || !o || !probs || B < 1 || L < 1 || H < 1 || d < 4 || (d & 3) || max_rel < 1) return STG_EINVAL;
   int nw;
   const size_t smem = dense_fwd_smem(L, d, &nw);
   if (!smem) return STG_EUNSUPPORTED;                   // sequence too long for the one-CTA-per-head kernel: stg_relattn_band_fwd
+  if (dtype != STG_F32 && dtype != STG_BF16) return STG_EINVAL;
   AttnP p{B, L, H, d, max_rel, scale};
-  if (dtype == STG_F32) {
-    STG_CUDA_CHECK(cudaFuncSetAttribute(relattn_fwd_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    relattn_fwd_kernel<float><<<B * H, 32 * nw, smem, S_>>>((const float*)qkv, emb, p, (float*)o, probs);
-  } else if (dtype == STG_BF16) {
-    STG_CUDA_CHECK(cudaFuncSetAttribute(relattn_fwd_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    relattn_fwd_kernel<bf16><<<B * H, 32 * nw, smem, S_>>>((const bf16*)qkv, emb, p, (bf16*)o, probs);
-  } else return STG_EINVAL;
-  STG_LAUNCH_CHECK();
-  return STG_OK;
+  if (dtype == STG_F32) return dense_fwd<float, kMask>((const float*)qkv, emb, p, nw, smem, (float*)o, probs, lengths, s);
+  return dense_fwd<bf16, kMask>((const bf16*)qkv, emb, p, nw, smem, (bf16*)o, probs, lengths, s);
+}
+
+extern "C" int stg_relattn_fwd(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel, float scale,
+                               void* o, float* probs, stg_stream_t stream) {
+  return relattn_fwd_any<false>(qkv, dtype, emb, B, L, H, d, max_rel, scale, o, probs, nullptr, S_);
+}
+
+extern "C" int stg_relattn_fwd_masked(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel,
+                                      float scale, void* o, float* probs, const int32_t* lengths, stg_stream_t stream) {
+  if (!lengths) return STG_EINVAL;
+  return relattn_fwd_any<true>(qkv, dtype, emb, B, L, H, d, max_rel, scale, o, probs, lengths, S_);
 }
 
 extern "C" int stg_relattn_bwd(const void* qkv, int dtype, const float* emb, const float* probs, const void* dout, int B, int L,
@@ -738,11 +842,12 @@ static size_t band_smem(const BandP& p, int per_warp_rows) {
   return sizeof(float) * ((size_t)BKC * (p.d + 4) + (size_t)BNW * (AR * p.d + per_warp_rows * AR * p.Up));
 }
 
-template <typename T>
-static int band_fwd(const T* qkv, const float* emb, const BandP& p, dim3 grid, T* o, float* probs, cudaStream_t s) {
+template <typename T, bool kMask>
+static int band_fwd(const T* qkv, const float* emb, const BandP& p, dim3 grid, T* o, float* probs, const int32_t* lengths,
+                    cudaStream_t s) {
   const size_t smem = band_smem(p, 1);
-  STG_CUDA_CHECK(cudaFuncSetAttribute(relattn_band_fwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  relattn_band_fwd_kernel<T><<<grid, BNW * 32, smem, s>>>(qkv, emb, p, o, probs);
+  STG_CUDA_CHECK(cudaFuncSetAttribute(relattn_band_fwd_kernel<T, kMask>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  relattn_band_fwd_kernel<T, kMask><<<grid, BNW * 32, smem, s>>>(qkv, emb, p, o, probs, lengths);
   STG_LAUNCH_CHECK();
   return STG_OK;
 }
@@ -760,13 +865,25 @@ static int band_bwd(const T* qkv, const float* emb, const float* probs, const T*
   return STG_OK;
 }
 
-extern "C" int stg_relattn_band_fwd(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel,
-                                    float scale, void* o, float* probs_band, stg_stream_t stream) {
+template <bool kMask>
+static int band_fwd_any(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel, float scale, void* o,
+                        float* probs_band, const int32_t* lengths, cudaStream_t s) {
   if (!qkv || !emb || !o || !probs_band || (dtype != STG_F32 && dtype != STG_BF16)) return STG_EINVAL;
   BandP p; dim3 grid;
   if (const int rc = band_params(B, L, H, d, max_rel, scale, &p, &grid)) return rc;
-  if (dtype == STG_F32) return band_fwd((const float*)qkv, emb, p, grid, (float*)o, probs_band, S_);
-  return band_fwd((const bf16*)qkv, emb, p, grid, (bf16*)o, probs_band, S_);
+  if (dtype == STG_F32) return band_fwd<float, kMask>((const float*)qkv, emb, p, grid, (float*)o, probs_band, lengths, s);
+  return band_fwd<bf16, kMask>((const bf16*)qkv, emb, p, grid, (bf16*)o, probs_band, lengths, s);
+}
+
+extern "C" int stg_relattn_band_fwd(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel,
+                                    float scale, void* o, float* probs_band, stg_stream_t stream) {
+  return band_fwd_any<false>(qkv, dtype, emb, B, L, H, d, max_rel, scale, o, probs_band, nullptr, S_);
+}
+
+extern "C" int stg_relattn_band_fwd_masked(const void* qkv, int dtype, const float* emb, int B, int L, int H, int d, int max_rel,
+                                           float scale, void* o, float* probs_band, const int32_t* lengths, stg_stream_t stream) {
+  if (!lengths) return STG_EINVAL;
+  return band_fwd_any<true>(qkv, dtype, emb, B, L, H, d, max_rel, scale, o, probs_band, lengths, S_);
 }
 
 extern "C" int stg_relattn_band_bwd(const void* qkv, int dtype, const float* emb, const float* probs_band, const void* dout, int B,
@@ -787,6 +904,17 @@ extern "C" int stg_encoder_losses(const float* unit_pred, const float* unit_targ
   if (grad_dtype == STG_F32) encoder_loss_kernel<float><<<blocks, 256, 0, S_>>>(unit_pred, unit_target, phoneme_logits, phoneme_target, N, Du, P, slots, gs_units, gs_phonemes, (float*)d_units, (float*)d_logits);
   else if (grad_dtype == STG_BF16) encoder_loss_kernel<bf16><<<blocks, 256, 0, S_>>>(unit_pred, unit_target, phoneme_logits, phoneme_target, N, Du, P, slots, gs_units, gs_phonemes, (bf16*)d_units, (bf16*)d_logits);
   else return STG_EINVAL;
+  STG_LAUNCH_CHECK();
+  return STG_OK;
+}
+
+extern "C" int stg_encoder_scores(const float* unit_pred, const float* unit_target, const float* phoneme_logits,
+                                  const int64_t* phoneme_target, const int32_t* lengths, int B, int T, int Du, int P,
+                                  int silence_index, float* sums, int32_t* counts, stg_stream_t stream) {
+  if (!unit_pred || !unit_target || !phoneme_logits || !phoneme_target || !lengths || !sums || !counts) return STG_EINVAL;
+  if (B < 1 || T < 1 || Du < 1 || P < 1 || B > (1 << 30)) return STG_EINVAL;
+  encoder_scores_kernel<<<B, SC_W * 32, 0, S_>>>(unit_pred, unit_target, phoneme_logits, phoneme_target, lengths, T, Du, P,
+                                                 silence_index, sums, counts);
   STG_LAUNCH_CHECK();
   return STG_OK;
 }

@@ -3,16 +3,19 @@ ste_gan/train.py:394) as a serving loop: weights are folded once, each (batch, f
 is captured as a CUDA graph, utterances are sharded round-robin over ranks with no collective.
 serve_batched() pads utterances of similar length to a common bucket length and runs them as one
 batch with per-sample length masks (stg_conv_masked), which leaves each utterance's result exact.
+validate_batched() scores generated utterances with the frozen EMG encoder in the same padded batches.
 """
 from __future__ import annotations
 
 from collections import OrderedDict
-from typing import Dict, List, Optional, Sequence, Tuple
+from dataclasses import dataclass
+from typing import Dict, Iterable, List, Optional, Sequence, Tuple
 
 import torch
 
-from . import passes
+from . import passes, passes_encoder
 from .dist import round_robin
+from .models.emg_encoder import SILENCE_PHONEME_INDEX
 
 Tensor = torch.Tensor
 
@@ -50,6 +53,42 @@ def plan_batches(lengths: Sequence[int], max_batch: int = 8,
     return plan
 
 
+@dataclass
+class EncoderScore:
+    """EMGEncoderLoss (losses/emg_encoder_loss.py:19-84) of one generated utterance, or summed over several
+    (aggregate_scores): the sums over frames and the phone counts, from which the frame-weighted means follow."""
+    speech_unit_sum: float              # sum over frames of ||target - pred + 1e-6||_2
+    phoneme_sum: float                  # sum over frames of the phoneme cross-entropy
+    num_phones: int                     # frames
+    num_correct_phones: int
+    num_silence_phones: int
+    num_correct_phones_no_silence: int
+
+    @property
+    def speech_unit_loss(self) -> float:
+        """Mean speech-unit distance (NaN for zero frames, as the mean of nothing)."""
+        return self.speech_unit_sum / self.num_phones if self.num_phones else float("nan")
+
+    @property
+    def phoneme_loss(self) -> float:
+        """Mean phoneme cross-entropy (NaN for zero frames)."""
+        return self.phoneme_sum / self.num_phones if self.num_phones else float("nan")
+
+
+def aggregate_scores(scores: Iterable[EncoderScore]) -> EncoderScore:
+    """Frame-weighted totals over a set of utterances: the sums and counts added up (in double precision), so the means of
+    the result weight every frame equally.  Accepts the values of validate_batched dicts, also merged across ranks."""
+    total = EncoderScore(0.0, 0.0, 0, 0, 0, 0)
+    for sc in scores:
+        total.speech_unit_sum += sc.speech_unit_sum
+        total.phoneme_sum += sc.phoneme_sum
+        total.num_phones += sc.num_phones
+        total.num_correct_phones += sc.num_correct_phones
+        total.num_silence_phones += sc.num_silence_phones
+        total.num_correct_phones_no_silence += sc.num_correct_phones_no_silence
+    return total
+
+
 class UtteranceGenerator:
     """max_graphs bounds the per-shape CUDA-graph cache (least recently used shape is dropped): each captured (batch,
     frames) shape pins its activations, so serving arbitrary utterance lengths would otherwise grow without limit.
@@ -58,9 +97,11 @@ class UtteranceGenerator:
     convolution reads exactly the zero padding the utterance gets on its own.  serve() runs one utterance per call
     at its own length; serve_batched() pads utterances to a few bucket lengths and batches them with length masks.
     Graphs are cached per (batch, frames) shape, masked graphs under (batch, frames, True): a masked graph reads the
-    lengths from a device buffer refreshed before each replay, so one graph serves every length mix of its shape."""
+    lengths from a device buffer refreshed before each replay, so one graph serves every length mix of its shape.
+    emg_encoder (a frozen EMGEncoderTransformer on the same device): validate_batched() scores the generated EMG with it;
+    its graphs are cached under ("validate", batch, frames) in the same LRU cache."""
 
-    def __init__(self, net_g, precision: str = "bf16", max_graphs: int = 8, trainer=None):
+    def __init__(self, net_g, precision: str = "bf16", max_graphs: int = 8, trainer=None, emg_encoder=None):
         self.net_g = net_g
         self.dtype = torch.bfloat16 if precision == "bf16" else torch.float32
         self.device = next(net_g.parameters()).device
@@ -73,9 +114,10 @@ class UtteranceGenerator:
         self.max_graphs = max(1, int(max_graphs))
         self._graphs: "OrderedDict[tuple, tuple]" = OrderedDict()
         self._uses_mode = bool(getattr(net_g, "use_speaking_mode_embedding", False))
+        self.emg_encoder = emg_encoder
 
     def refold(self) -> None:
-        """Call after the generator's weights changed."""
+        """Call after the generator's weights changed (drops every captured graph, the validation graphs included)."""
         if self.trainer is not None:
             self.trainer.flush()          # (pipelined step_graph defers the last generator AdamW)
         self.folds = passes.fold_generator(self.net_g, self.dtype, want_dgrad=False)
@@ -170,4 +212,77 @@ class UtteranceGenerator:
             host = y[:len(idx)].to("cpu", non_blocking=False)     # one copy per batch
             for j, i in enumerate(idx):
                 out[i] = host[j, :r * lengths[i]].clone()
+        return out
+
+    @torch.no_grad()
+    def _score(self, su: Tensor, sess: Tensor, lens: Tensor, ut: Tensor, ph: Tensor) -> Tuple[Tensor, Tensor]:
+        """Masked generate -> masked encode -> per-utterance scores, all on the device (see validate_batched)."""
+        x, _ = passes.generator_forward(self.net_g, su, sess, None, self.dtype, False, folds=self.folds, lengths=lens)
+        plan = self.emg_encoder.plan(self.dtype)
+        if x.shape[1] != plan.frame_rows * su.shape[1]:
+            raise ValueError(f"validate_batched: the generator gives {x.shape[1] // su.shape[1]} EMG rows per frame, the "
+                             f"encoder takes {plan.frame_rows}")
+        return passes_encoder.encoder_scores(plan, x, ut, ph, lens)
+
+    @torch.no_grad()
+    def _capture_validate(self, batch: int, frames: int, unit_dim: int, target_dim: int) -> None:
+        while len(self._graphs) >= self.max_graphs:      # LRU bound, shared with the serving graphs
+            self._graphs.popitem(last=False)
+        dev = self.device
+        su = torch.zeros(batch, frames, unit_dim, device=dev)
+        sess = torch.zeros(batch, device=dev, dtype=torch.int64)
+        lens = torch.full((batch,), frames, device=dev, dtype=torch.int32)
+        ut = torch.zeros(batch, frames, target_dim, device=dev)
+        ph = torch.zeros(batch, frames, device=dev, dtype=torch.int64)
+        side = torch.cuda.Stream()
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side):
+            for _ in range(2):
+                self._score(su, sess, lens, ut, ph)
+        torch.cuda.current_stream().wait_stream(side)
+        torch.cuda.synchronize()
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            sums, counts = self._score(su, sess, lens, ut, ph)
+        self._graphs[("validate", batch, frames)] = (g, su, sess, lens, ut, ph, sums, counts)
+
+    def validate_batched(self, utterances: List[Tuple[Tensor, Tensor, Tensor, Tensor]], rank: int = 0, world: int = 1,
+                         max_batch: int = 8, per_octave: int = BUCKETS_PER_OCTAVE) -> Dict[int, EncoderScore]:
+        """Score generated utterances with the frozen EMG encoder: this rank's share of (generator input [n, D], session_id,
+        unit_target [n, Du], phoneme_target [n]) items -> {utterance index: EncoderScore}, each equal to EMGEncoderLoss on
+        that utterance's generated EMG alone.  Batches as serve_batched (plan_batches, round-robin by batch); each bucket
+        replays one captured graph of masked generate -> masked encode -> scores, so the EMG never leaves the device and
+        only the [max_batch] sums and counts come back per batch.  Merge the dicts of several ranks with aggregate_scores."""
+        if self.emg_encoder is None:
+            raise ValueError("validate_batched: construct UtteranceGenerator with emg_encoder=")
+        if self._uses_mode:
+            raise ValueError("validate_batched: speaking-mode generators are not supported (as in serve_batched)")
+        lengths = [int(u[0].shape[0]) for u in utterances]
+        plan = plan_batches(lengths, max_batch, per_octave)
+        out = {}
+        for T, idx in plan[rank::world]:
+            D, Du = utterances[idx[0]][0].shape[1], utterances[idx[0]][2].shape[1]
+            key = ("validate", max_batch, T)
+            if key not in self._graphs:
+                self._capture_validate(max_batch, T, D, Du)
+            self._graphs.move_to_end(key)
+            g, su_d, sess_d, lens_d, ut_d, ph_d, sums_d, counts_d = self._graphs[key]
+            su = torch.zeros(max_batch, T, D)
+            sess = torch.zeros(max_batch, dtype=torch.int64)
+            lens = torch.zeros(max_batch, dtype=torch.int32)
+            ut = torch.zeros(max_batch, T, Du)
+            ph = torch.zeros(max_batch, T, dtype=torch.int64)
+            for j, i in enumerate(idx):
+                units, sid, u_t, p_t = utterances[i]
+                n = lengths[i]
+                if u_t.shape[0] != n or p_t.shape[0] != n:
+                    raise ValueError(f"validate_batched: utterance {i} has {n} input frames but targets of "
+                                     f"{u_t.shape[0]} / {p_t.shape[0]} frames")
+                su[j, :n], sess[j], lens[j], ut[j, :n], ph[j, :n] = units, sid.reshape(()), n, u_t, p_t
+            for dst, src in ((su_d, su), (sess_d, sess), (lens_d, lens), (ut_d, ut), (ph_d, ph)):
+                dst.copy_(src, non_blocking=True)
+            g.replay()
+            sums, counts = sums_d.to("cpu").tolist(), counts_d.to("cpu").tolist()      # the only copies back per batch
+            for j, i in enumerate(idx):
+                out[i] = EncoderScore(sums[j][0], sums[j][1], *counts[j])
         return out

@@ -585,15 +585,21 @@ def layernorm_bwd(dy: Tensor, x: Tensor, stats: Tensor, gamma: Tensor) -> Tensor
     return dx
 
 
-def relattn_fwd(qkv: Tensor, emb: Tensor, n_head: int, max_rel: int) -> Tuple[Tensor, Tensor]:
-    """qkv [B, L, 3*H*d] -> (o [B, L, H*d], probs fp32 [B, H, L, L]); emb fp32 [H, 2*max_rel-1, d]."""
+def relattn_fwd(qkv: Tensor, emb: Tensor, n_head: int, max_rel: int, lengths: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
+    """qkv [B, L, 3*H*d] -> (o [B, L, H*d], probs fp32 [B, H, L, L]); emb fp32 [H, 2*max_rel-1, d].
+    lengths (int32 [B] on the device): stg_relattn_fwd_masked - sample b attends over its first lengths[b] rows only, its
+    rows past them are 0."""
     B, L, C3 = qkv.shape
     d = C3 // (3 * n_head)
     _need(qkv, B * L * C3, None, "qkv"); _need(emb, n_head * (2 * max_rel - 1) * d, torch.float32, "emb")
+    _need(lengths, B, torch.int32, "lengths")
     o = torch.empty((B, L, n_head * d), device=qkv.device, dtype=qkv.dtype)
     probs = torch.empty((B, n_head, L, L), device=qkv.device, dtype=torch.float32)
-    check(_lib.load().stg_relattn_fwd(_ptr(qkv), code_of(qkv.dtype), _ptr(emb), B, L, n_head, d, max_rel, float(d) ** -0.5, _ptr(o),
-                                      _ptr(probs), _stream()), "stg_relattn_fwd")
+    args = (_ptr(qkv), code_of(qkv.dtype), _ptr(emb), B, L, n_head, d, max_rel, float(d) ** -0.5, _ptr(o), _ptr(probs))
+    if lengths is None:
+        check(_lib.load().stg_relattn_fwd(*args, _stream()), "stg_relattn_fwd")
+    else:
+        check(_lib.load().stg_relattn_fwd_masked(*args, _ptr(lengths), _stream()), "stg_relattn_fwd_masked")
     return o, probs
 
 
@@ -613,16 +619,21 @@ def relattn_dense_supported(L: int, d: int, need_bwd: bool) -> bool:
     return bool(_lib.load().stg_relattn_dense_supported(int(L), int(d), int(bool(need_bwd))))
 
 
-def relattn_band_fwd(qkv: Tensor, emb: Tensor, n_head: int, max_rel: int) -> Tuple[Tensor, Tensor]:
+def relattn_band_fwd(qkv: Tensor, emb: Tensor, n_head: int, max_rel: int,
+                     lengths: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
     """relattn_fwd at any L -> (o [B, L, H*d], probs_band fp32 [B, H, L, 2*max_rel-1]): entry (i, w) is the probability of key
-    j = i + w - (max_rel - 1), 0 where that j is outside [0, L)."""
+    j = i + w - (max_rel - 1), 0 where that j is outside [0, L).  lengths: as relattn_fwd (stg_relattn_band_fwd_masked)."""
     B, L, C3 = qkv.shape
     d = C3 // (3 * n_head)
     _need(qkv, B * L * C3, None, "qkv"); _need(emb, n_head * (2 * max_rel - 1) * d, torch.float32, "emb")
+    _need(lengths, B, torch.int32, "lengths")
     o = torch.empty((B, L, n_head * d), device=qkv.device, dtype=qkv.dtype)
     probs = torch.empty((B, n_head, L, 2 * max_rel - 1), device=qkv.device, dtype=torch.float32)
-    check(_lib.load().stg_relattn_band_fwd(_ptr(qkv), code_of(qkv.dtype), _ptr(emb), B, L, n_head, d, max_rel, float(d) ** -0.5,
-                                           _ptr(o), _ptr(probs), _stream()), "stg_relattn_band_fwd")
+    args = (_ptr(qkv), code_of(qkv.dtype), _ptr(emb), B, L, n_head, d, max_rel, float(d) ** -0.5, _ptr(o), _ptr(probs))
+    if lengths is None:
+        check(_lib.load().stg_relattn_band_fwd(*args, _stream()), "stg_relattn_band_fwd")
+    else:
+        check(_lib.load().stg_relattn_band_fwd_masked(*args, _ptr(lengths), _stream()), "stg_relattn_band_fwd_masked")
     return o, probs
 
 
@@ -654,3 +665,22 @@ def encoder_losses(unit_pred: Tensor, unit_target: Tensor, logits: Tensor, phone
                                          float(gs_units), float(gs_phonemes), _ptr(du), _ptr(dl),
                                          code_of(grad_dtype) if grad_dtype is not None else F32, _stream()), "stg_encoder_losses")
     return du, dl
+
+
+def encoder_scores(unit_pred: Tensor, unit_target: Tensor, logits: Tensor, phoneme_target: Tensor, lengths: Tensor,
+                   silence_index: int) -> Tuple[Tensor, Tensor]:
+    """Per-utterance EMGEncoderLoss of a padded batch (stg_encoder_scores): unit_pred / unit_target fp32 [B, T, Du], logits fp32
+    [B, T, P], phoneme_target int64 [B, T], lengths int32 [B] (frames; rows past them are never read) ->
+    (sums fp32 [B, 2] = (sum of unit distances, sum of cross-entropies), counts int32 [B, 4] = (frames, correct phones,
+    silence phones, correct non-silence phones))."""
+    B, T, Du = unit_pred.shape
+    P_ = logits.shape[-1]
+    _need(unit_pred, B * T * Du, torch.float32, "unit_pred"); _need(unit_target, B * T * Du, torch.float32, "unit_target")
+    _need(logits, B * T * P_, torch.float32, "logits"); _need(phoneme_target, B * T, torch.int64, "phoneme_target")
+    _need(lengths, B, torch.int32, "lengths")
+    sums = torch.empty((B, 2), device=unit_pred.device, dtype=torch.float32)
+    counts = torch.empty((B, 4), device=unit_pred.device, dtype=torch.int32)
+    check(_lib.load().stg_encoder_scores(_ptr(unit_pred), _ptr(unit_target), _ptr(logits), _ptr(phoneme_target), _ptr(lengths),
+                                         B, T, Du, P_, int(silence_index), _ptr(sums), _ptr(counts), _stream()),
+          "stg_encoder_scores")
+    return sums, counts

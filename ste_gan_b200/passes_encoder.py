@@ -92,6 +92,9 @@ class EncoderPlan:
             c2 = _pack(*_bn_fold(blk.conv2, blk.bn2), 1, 1, dtype)
             res = _pack(*_bn_fold(blk.residual_path, blk.res_norm), blk.stride, 0, dtype) if blk.residual_path is not None else None
             self.blocks.append((c1, c2, res))
+        self.frame_rows = 1                 # EMG rows per encoder frame: the product of the ResBlock strides (16)
+        for c1, _, _ in self.blocks:
+            self.frame_rows *= c1.mod.stride
         self.w_in = lin(enc.w_raw_in)
         self.layers: List[_Layer] = []
         for lyr in enc.transformer.layers:
@@ -127,39 +130,56 @@ def _src(f: Folded, x: Tensor, B: int, t: int) -> Tensor:
     return unfold_input(f, x, B, t) if f.unfold else x
 
 
-def encoder_forward(plan: EncoderPlan, emg: Tensor, need_ctx: bool = True):
-    """emg fp32 [B, T, C] -> (speech-unit prediction fp32 [B, T/16, 256], phoneme logits fp32 [B, T/16, P], ctx)."""
+def encoder_forward(plan: EncoderPlan, emg: Tensor, need_ctx: bool = True, lengths: Optional[Tensor] = None):
+    """emg fp32 [B, T, C] -> (speech-unit prediction fp32 [B, T/16, 256], phoneme logits fp32 [B, T/16, P], ctx).
+    lengths (int32 [B] on the device, frames; forward only): sample b is an utterance of lengths[b] frames (16 * lengths[b]
+    EMG rows) padded to T / 16 frames with anything, NaN included.  Rows [0, lengths[b]) of both heads are what the utterance
+    gives on its own, the rows after them are 0.  Why output masks alone make this exact: every conv writes 0 at its rows
+    past the sample's end (rates of 8, 4, 2, 1 rows per frame after blocks 1-4), so each conv reads 0 there, which is the
+    zero padding the utterance gets alone.  Only conv2 of a ResBlock (k = 3, pad 1, stride 1) reads a row past the end, and
+    that row is conv1's masked output.  The stride-2 convs on even lengths read rows <= 2o + 1 (k = 3, pad 1) or 2o (k = 1)
+    for a kept output row o: all inside the sample.  The transformer is row-local except attention, which skips the padded
+    keys (stg_relattn_fwd_masked); the padded rows of the LayerNorm outputs hold beta, but no kept row reads them."""
+    if lengths is not None:
+        if need_ctx:
+            raise ValueError("encoder_forward: length masks are forward-only (need_ctx=True with lengths)")
+        if emg.shape[1] % plan.frame_rows != 0:
+            raise ValueError(f"encoder_forward: with lengths, T = {emg.shape[1]} must be a multiple of {plan.frame_rows} "
+                             "(EMG rows per frame)")
     dt = plan.dtype
     x = emg.contiguous().float()
     B, T, _ = x.shape
     h_in, t = ops.cast(x, dt), T
+    rate = plan.frame_rows                  # rows per frame of the current activations
     saved_blocks = []
     for (c1, c2, res) in plan.blocks:
-        _, h, t1 = _fwd(c1, _src(c1, h_in, B, t), B, t, act=ACT_RELU, want_act=True)            # relu(bn1(conv1 x))
+        m = dict(lengths=lengths, rate=rate // c1.mod.stride)
+        _, h, t1 = _fwd(c1, _src(c1, h_in, B, t), B, t, act=ACT_RELU, want_act=True, **m)      # relu(bn1(conv1 x))
         if res is not None:
-            r, _, _ = _fwd(res, _src(res, h_in, B, t), B, t, want_raw=True)                     # res_norm(residual_path x)
+            r, _, _ = _fwd(res, _src(res, h_in, B, t), B, t, want_raw=True, **m)                # res_norm(residual_path x)
         else:
             r = h_in
-        _, y, _ = _fwd(c2, h, B, t1, act=ACT_RELU, want_act=True, add_post=r)                   # relu(bn2(conv2 h) + res)
+        _, y, _ = _fwd(c2, h, B, t1, act=ACT_RELU, want_act=True, add_post=r, **m)              # relu(bn2(conv2 h) + res)
         saved_blocks.append(dict(x_in=h_in, h=h, y=y, t_in=t, t_out=t1))
-        h_in, t = y, t1
+        h_in, t, rate = y, t1, m["rate"]
     L = t
-    xl, _, _ = _fwd(plan.w_in, h_in, B, L, want_raw=True)                                       # emg_encoder.py:80
+    m = dict(lengths=lengths, rate=rate)
+    xl, _, _ = _fwd(plan.w_in, h_in, B, L, want_raw=True, **m)                                  # emg_encoder.py:80
     saved_layers = []
     for ly in plan.layers:
-        qkv, _, _ = _fwd(ly.qkv, xl, B, L, want_raw=True)
+        qkv, _, _ = _fwd(ly.qkv, xl, B, L, want_raw=True, **m)
         # the one-CTA-per-head kernels where they take L (for the backward too, when it follows), the band-tiled ones beyond
         band = not ops.relattn_dense_supported(L, qkv.shape[-1] // (3 * ly.n_head), need_ctx)
-        o, probs = (ops.relattn_band_fwd if band else ops.relattn_fwd)(qkv, ly.emb, ly.n_head, ly.max_rel)
-        pre1, _, _ = _fwd(ly.out, o, B, L, want_raw=True, add_post=xl)                          # src + attn        (transformer.py:54-55)
+        o, probs = (ops.relattn_band_fwd if band else ops.relattn_fwd)(qkv, ly.emb, ly.n_head, ly.max_rel, lengths=lengths)
+        pre1, _, _ = _fwd(ly.out, o, B, L, want_raw=True, add_post=xl, **m)                     # src + attn        (transformer.py:54-55)
         x1, st1 = ops.layernorm(pre1, ly.g1, ly.b1, LN_EPS)                                     # norm1             (:56)
-        _, hff, _ = _fwd(ly.l1, x1, B, L, act=ACT_RELU, want_act=True)                          # relu(linear1)     (:57)
-        pre2, _, _ = _fwd(ly.l2, hff, B, L, want_raw=True, add_post=x1)                         # src + linear2     (:57-58)
+        _, hff, _ = _fwd(ly.l1, x1, B, L, act=ACT_RELU, want_act=True, **m)                     # relu(linear1)     (:57)
+        pre2, _, _ = _fwd(ly.l2, hff, B, L, want_raw=True, add_post=x1, **m)                    # src + linear2     (:57-58)
         x2, st2 = ops.layernorm(pre2, ly.g2, ly.b2, LN_EPS)                                     # norm2             (:59)
         saved_layers.append(dict(qkv=qkv, probs=probs, band=band, pre1=pre1, st1=st1, hff=hff, pre2=pre2, st2=st2))
         xl = x2
-    units, _, _ = _fwd(plan.w_out, xl, B, L, want_raw=True, out_f32=True)                       # emg_encoder.py:88
-    logits, _, _ = _fwd(plan.w_aux, xl, B, L, want_raw=True, out_f32=True)
+    units, _, _ = _fwd(plan.w_out, xl, B, L, want_raw=True, out_f32=True, **m)                  # emg_encoder.py:88
+    logits, _, _ = _fwd(plan.w_aux, xl, B, L, want_raw=True, out_f32=True, **m)
     ctx = EncCtx(B=B, T=T, blocks=saved_blocks, y_last=h_in, t_last=L, layers=saved_layers, x_final=xl) if need_ctx else None
     return units, logits, ctx
 
@@ -218,3 +238,13 @@ def encoder_losses(plan: EncoderPlan, emg: Tensor, unit_target: Tensor, phoneme_
     if not want_grad:
         return None, units, logits
     return encoder_backward(plan, ctx, du if use_units else None, dl if use_phonemes else None), units, logits
+
+
+def encoder_scores(plan: EncoderPlan, emg: Tensor, unit_target: Tensor, phoneme_target: Tensor, lengths: Tensor):
+    """EMGEncoderLoss per utterance of a padded batch, forward only: emg fp32 [B, T, C], unit_target [B, T/16, Du],
+    phoneme_target [B, T/16], lengths int32 [B] on the device (frames).  Returns the device tensors (sums fp32 [B, 2],
+    counts int32 [B, 4]) of ops.encoder_scores; rows past an utterance's end are never read."""
+    from .models.emg_encoder import SILENCE_PHONEME_INDEX
+    units, logits, _ = encoder_forward(plan, emg, need_ctx=False, lengths=lengths)
+    return ops.encoder_scores(units, unit_target.contiguous().float(), logits, phoneme_target.contiguous().to(torch.int64),
+                              lengths, SILENCE_PHONEME_INDEX)
