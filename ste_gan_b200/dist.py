@@ -64,8 +64,7 @@ class GradReducer:
         # Our own NCCL communicator (ste_gan_b200/nccl.py): all-reduces on explicit streams, capturable inside the CUDA
         # graphs of the train step.  GPU + NCCL backend only; the gloo tests exercise the torch.distributed path.
         self.comm = None
-        if self.enabled and torch.cuda.is_available() and dist.get_backend(group) == "nccl" and \
-                os.environ.get("STG_OWN_NCCL", "1") != "0":
+        if self.enabled and torch.cuda.is_available() and dist.get_backend(group) == "nccl":
             from .nccl import NcclComm
             self.comm = NcclComm(group)
 

@@ -119,7 +119,7 @@ class UtteranceGenerator:
     def refold(self) -> None:
         """Call after the generator's weights changed (drops every captured graph, the validation graphs included)."""
         if self.trainer is not None:
-            self.trainer.flush()          # (pipelined step_graph defers the last generator AdamW)
+            self.trainer.flush()          # (step_graph defers the last generator AdamW)
         self.folds = passes.fold_generator(self.net_g, self.dtype, want_dgrad=False)
         self._graphs.clear()
 

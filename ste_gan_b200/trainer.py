@@ -127,7 +127,8 @@ class GanTrainer:
         self._d_folded = False                  # d_plan packs match the current D weights
         self.reducer = GradReducer(group, enabled=data_parallel)
         # data parallel with the own NCCL communicator: the all-reduces are stream-ordered launches issued INSIDE the phases
-        # (and therefore inside the captured graphs); without it (STG_OWN_NCCL=0) torch.distributed calls between the graphs
+        # (and therefore inside the captured graph); without it (a group that is not CUDA + NCCL) the eager step() calls
+        # torch.distributed between its phases, and capture() refuses
         self._inline = self.reducer.comm is not None
         dev = self.G.flat.device
         self.device = dev
@@ -140,9 +141,6 @@ class GanTrainer:
         self.slots = torch.zeros(8, device=dev, dtype=torch.float32)
         self.d_folds: Optional[Dict[int, passes.Folded]] = None
         self._d_persist: Dict[int, passes.Folded] = {}
-        self._graphs = None
-        self._d_graphs = None
-        self._pending_g = None                  # handles of a deferred generator-gradient all-reduce (pipelined step_graph)
         self._static = None
         self.x_pred: Optional[Tensor] = None
         # the discriminator passes on x_pred and on x_real are independent: they run on two streams (forked from and
@@ -158,20 +156,11 @@ class GanTrainer:
         self._enc = torch.cuda.Stream(device=dev)                                     # EMG-encoder losses beside the D passes
         self._comm = torch.cuda.Stream(device=dev)                                    # gradient all-reduces (own NCCL communicator)
         self._pend = torch.zeros(1, device=dev, dtype=torch.int32)                    # device flag: a generator AdamW is pending (fused graph)
-        self._fused = None                                                            # (step graph, flush graph) of the fused capture
+        self._fused = None                                                            # (step graph, flush graph) of capture()
         self._pending_host = False
-        self._sm_reserve, self._n_sm = 0, torch.cuda.get_device_properties(dev).multi_processor_count
-        self.concurrent_d = True
-        import os
-        self._d_slices = self._disc_grad_slices() if os.environ.get("STG_D_BUCKETS", "1") != "0" else None
-        # Gradient buckets of the generator, back to front (= the order its backward completes them).  GBlocks
-        # [k2, n) + last_conv | [k1, k2) | [0, k1) + gblocks.0 + embeddings, cut where the parameter count from the
-        # front passes 1/3 and 2/3 (base model: GB3..GB8 | GB2 | GB1, ~8 M parameters each).  Each entry:
-        # (first GBlock, end GBlock, first conv, end conv of passes.generator_convs, flat-gradient slice).
+        self._d_slices = self._disc_grad_slices()
         self.g_buckets = generator_grad_buckets(self.G.offsets, self.G.numel, len(list(net_g.gblocks)) - 1)
-        # without a data-parallel group there is nothing to overlap: one bucket (one fold-backward launch, one graph)
-        if grad_buckets is None and os.environ.get("STG_G_BUCKETS"):
-            grad_buckets = int(os.environ["STG_G_BUCKETS"])
+        # without a data-parallel group there is nothing to overlap: one bucket (one fold-backward launch)
         if (grad_buckets if grad_buckets is not None else (3 if self.reducer.enabled else 1)) == 1:
             nblk = len(list(net_g.gblocks)) - 1
             self.g_buckets = [(0, nblk, 0, 5 * nblk + 2, (0, self.G.numel))]
@@ -230,12 +219,9 @@ class GanTrainer:
             return None
         return out
 
-    def _s2(self, i: int):
-        return self._side2[i] if self.concurrent_d else None
-
     def _fold_d(self, refold: bool):
         return passes.fold_discriminator(self.net_d, self.dtype, training=True, plan=self.d_plan, refold=refold,
-                                         sn_streams=self._sn if self.concurrent_d else None)
+                                         sn_streams=self._sn)
 
     def _reduce(self, flat_slice: Tensor):
         """Data parallel: all-reduce (sum) a slice of a flat gradient on the communication stream, ordered after
@@ -257,14 +243,6 @@ class GanTrainer:
             if e is not None:
                 torch.cuda.current_stream().wait_event(e)
 
-    def _sm_scope(self, on: bool) -> None:
-        """Data-parallel fused capture only (self._sm_reserve > 0): the tcgen05 launches captured while `on` leave
-        `_sm_reserve` SMs to the communicator - the pieces of the step that run beside a gradient all-reduce; everything
-        else gets the whole chip."""
-        if self._sm_reserve > 0:
-            from . import _lib as _l
-            _l.load().stg_set_sm_limit(self._n_sm - self._sm_reserve if on else 0)
-
     def _fork(self) -> None:
         ev = torch.cuda.Event()
         ev.record(torch.cuda.current_stream())
@@ -276,39 +254,37 @@ class GanTrainer:
         torch.cuda.current_stream().wait_event(ev)
 
     # ------------------------------------------------------------------ phases
-    # Phase D is five pieces with three dependencies between them:
-    #     _d_folds -> _d_real --------------\
-    #        \ (f1)                         v
-    #   _g_forward -> _d_fake -----------> _d_update
-    # Eager steps (and the single-graph capture) run the top row on the side stream; the pipelined capture makes each
-    # piece its own CUDA graph so that the top row of step k+1 can start while step k's gradient all-reduce and
-    # generator optimiser are still running (step_graph).
-    def _d_folds(self) -> None:
-        """Discriminator folds of the fake pass (f1) and of the real pass (f2): the spectral-norm power iterations of
-        the two forwards happen in that order (train.py:190-191)."""
-        refold_d = not self._d_folded
-        self._d_folded = True
-        self._f1 = self._fold_d(refold_d)
-        self._ev_f1 = torch.cuda.Event()
-        self._ev_f1.record(torch.cuda.current_stream())
-        self._f2 = self._fold_d(False)
-
-    # The fake and the real pass share their weights except in the spectral-norm sub-discriminator (the full-rate scale
-    # stack: its sigma advances between the two forwards).  With `concurrent_d` that stack runs once per pass and all
-    # the others run ONCE, forward and backward, on the concatenated batch [x_pred | x_real]: half the launches, twice
-    # the rows per launch (their layers have too few tiles to fill the chip), one weight-gradient contraction over both.
+    # The fake and the real pass of a discriminator forward share their weights except in the spectral-norm
+    # sub-discriminator (the full-rate scale stack: its sigma advances between the two forwards).  That stack runs once per
+    # pass and all the others run ONCE, forward and backward, on the concatenated batch [x_pred | x_real]: half the
+    # launches, twice the rows per launch (their layers have too few tiles to fill the chip), one weight-gradient
+    # contraction over both.
     def _split_subs(self):
         subs = passes.disc_subnets(self.net_d)
         heavy, rest = passes._heavy_split(subs)
         return subs, heavy, [i for i in rest if subs[i][0] == "P"], [i for i in rest if subs[i][0] == "S"]
 
-    def _d_real(self, x_real: Tensor) -> None:
-        self._x_real = x_real
-        if self.concurrent_d:      # only the spectral-norm stack: the rest waits for x_pred and runs batched (_d_fake)
-            _, heavy, _, _ = self._split_subs()
-            self._real = passes.discriminator_forward(self.net_d, x_real, self.dtype, self._f2, subset=heavy) if heavy else (None, None)
-        else:
-            self._real = passes.discriminator_forward(self.net_d, x_real, self.dtype, self._f2)
+    def _disc_forward(self, x: Tensor, folds, idx: list, spread=None):
+        """Forward of the sub-discriminators `idx` (none: (None, None)), dealt over the `spread` streams."""
+        if not idx:
+            return None, None
+        return passes.discriminator_forward(self.net_d, x, self.dtype, folds, subset=idx, spread=spread)
+
+    def _per_pass(self, heavy: list, fake_h, real_h, batched):
+        """Per-pass views of every sub-discriminator's feature maps: the batched stacks (`batched`: pairs of a forward over
+        [x_pred | x_real] and its indices) split behind x_pred's rows, the spectral-norm stack from its two own passes
+        (fake_h, real_h).  Returns (fake maps, real maps, per-sub contexts of the fake pass); views only, no launches."""
+        nd, Bq = len(passes.disc_subnets(self.net_d)), self.x_pred.shape[0]
+        res_f, res_r, sub_f = [None] * nd, [None] * nd, [None] * nd
+        for (r_b, c_b), idx in batched:
+            if idx:
+                a, b, sa = passes.split_disc_batch(r_b, c_b, idx, Bq)
+                for i in idx:
+                    res_f[i], res_r[i], sub_f[i] = a[i], b[i], sa[i]
+        (rh_f, ch_f), (rh_r, _) = fake_h, real_h
+        for i in heavy:
+            res_f[i], res_r[i], sub_f[i] = rh_f[i], rh_r[i], ch_f.subs[i]
+        return res_f, res_r, sub_f
 
     def _g_forward(self, su: Tensor, sess: Tensor, mode: Optional[Tensor], x_pred: Optional[Tensor] = None) -> None:
         self.slots.zero_()
@@ -319,54 +295,17 @@ class GanTrainer:
             self.x_pred = x_pred
             return
         self.x_pred, self._gctx = passes.generator_forward(self.net_g, su, sess, mode, self.dtype, True, folds=self.g_plan.fold(),
-                                                           side=self._s2(1) if self.use_adv else None)
+                                                           side=self._side2[1] if self.use_adv else None)
 
-    def _d_fake(self) -> None:
+    def _d_update(self, fake_h, real_h, p_b, s_b) -> None:
+        """loss_D of the two passes, its backward (weight gradients only) and the data-parallel exchange of the
+        discriminator gradient."""
         dt = self.dtype
-        if not self.concurrent_d:
-            self._fake = passes.discriminator_forward(self.net_d, self.x_pred, dt, self._f1)
-            return
-        _, heavy, p_idx, s_idx = self._split_subs()
-        fwd = lambda x, idx: passes.discriminator_forward(self.net_d, x, dt, self._f1, subset=idx,
-                                                          spread=self._ps if idx is p_idx else (self._ss if idx is s_idx else None)) if idx else (None, None)
-        x_cat = torch.cat([self.x_pred, self._x_real], 0)
-        # current: fake pass of the spectral-norm stack | side2[1]: S stacks batched | side2[0]: P stacks batched
-        ((rs, cs), (rp, cp)), (rh, ch) = passes.fork_join(
-            self._s2(1), lambda: passes.fork_join(self._s2(0), lambda: fwd(x_cat, p_idx), lambda: fwd(x_cat, s_idx))[::-1],
-            lambda: fwd(self.x_pred, heavy))
-        self._fake = (rh, ch)
-        self._batched = (rp, cp, rs, cs, x_cat)
-
-    def _d_update(self) -> None:
-        dt = self.dtype
-        if not self.concurrent_d:
-            (res_f, ctx_f), (res_r, ctx_r) = self._fake, self._real
-            self._fake = self._real = None
-            self._last_d_fmaps = (res_f, res_r, ctx_f)      # kept for the parity tests (references only)
-            nd = len(res_f)
-            dl = ops.mse_const_multi([fm[-1] for fm in res_f] + [fm[-1] for fm in res_r], [0.0] * nd + [1.0] * nd, self.slots,
-                                     [0] * (2 * nd), 1.0, dt)
-            self.d_plan.zero()
-            passes.discriminator_backward(self.net_d, ctx_f, dl[:nd], None, want_input_grad=False, want_weight_grad=True, plan=self.d_plan)
-            passes.discriminator_backward(self.net_d, ctx_r, dl[nd:], None, want_input_grad=False, want_weight_grad=True, plan=self.d_plan)
-            self.d_plan.backward(accumulate=False)
-            self._reduce_d()
-            return
         subs, heavy, p_idx, s_idx = self._split_subs()
-        (rh_f, ch_f), (rh_r, ch_r) = self._fake, self._real
-        rp, cp, rs, cs, x_cat = self._batched
-        self._fake = self._real = self._batched = None
+        ch_f, ch_r, cp, cs = fake_h[1], real_h[1], p_b[1], s_b[1]
         Bq, nd = self.x_pred.shape[0], len(subs)
-        # per-pass views of every feature map (parity tests; the loss below needs the logits of each pass)
-        res_f, res_r = [None] * nd, [None] * nd
-        for r_b, c_b, idx in ((rp, cp, p_idx), (rs, cs, s_idx)):
-            if idx:
-                a, b, _ = passes.split_disc_batch(r_b, c_b, idx, Bq)
-                for i in idx:
-                    res_f[i], res_r[i] = a[i], b[i]
-        for i in heavy:
-            res_f[i], res_r[i] = rh_f[i], rh_r[i]
-        self._last_d_fmaps = (res_f, res_r, ch_f)
+        res_f, res_r, _ = self._per_pass(heavy, fake_h, real_h, ((p_b, p_idx), (s_b, s_idx)))
+        self._last_d_fmaps = (res_f, res_r, ch_f)      # kept for the parity tests (references only)
         # loss_D = sum_i mse(fake_i, 0) + mse(real_i, 1) and its gradients, one launch      train.py:192-196
         # (batched stacks: the two gradients land in the two halves of one [2B, rows, 1] tensor)
         dcat = {i: torch.empty((2 * Bq,) + tuple(res_f[i][-1].shape[1:]), device=self.device, dtype=dt) for i in p_idx + s_idx}
@@ -387,9 +326,9 @@ class GanTrainer:
         only = lambda dlog, idx: [dlog[i] if i in idx else None for i in range(nd)]
         self._fork()
         with torch.cuda.stream(self._side):       # side: spectral-norm stack, fake | its side: spectral-norm stack, real
-            passes.fork_join(self._s2(0), lambda: bwd(ch_r, only(dl_r, heavy)), lambda: bwd(ch_f, only(dl_f, heavy)))
+            passes.fork_join(self._side2[0], lambda: bwd(ch_r, only(dl_r, heavy)), lambda: bwd(ch_f, only(dl_f, heavy)))
         # current: P stacks, batched | its side: S stacks, batched
-        passes.fork_join(self._s2(1), lambda: bwd(cs, only(dl_b, s_idx)), lambda: bwd(cp, only(dl_b, p_idx)))
+        passes.fork_join(self._side2[1], lambda: bwd(cs, only(dl_b, s_idx)), lambda: bwd(cp, only(dl_b, p_idx)))
         early = []
         if self._inline and heavy and self._d_slices is not None:
             # data parallel: the period stacks and the two coarse scale stacks are through (the spectral-norm stack, half
@@ -407,55 +346,52 @@ class GanTrainer:
             self._wait_events(early + [self._reduce(self.D.grad[g_lo:g_hi])])
             return
         self.d_plan.backward(accumulate=False)    # the only contribution since zero_grad: overwrite
-        self._reduce_d()
-
-    def _reduce_d(self) -> None:
-        """Data parallel: the discriminator gradient is exchanged in one piece right behind its backward pass - everything
-        that follows (D AdamW, the passes of phase G) depends on it.  (own communicator: in-stream, also under capture)"""
         if self._inline:
+            # data parallel, one piece right behind the backward: everything that follows (D AdamW, phase G) depends on it
             self._wait_events([self._reduce(self.D.grad)])
 
     def _phase_d(self, su: Tensor, sess: Tensor, mode: Optional[Tensor], x_real: Tensor, x_pred: Optional[Tensor] = None,
                  head=None) -> None:
-        """`head` (fused graph): runs on the current stream right before the generator fold + forward - the pending
-        generator update of the previous step - while the discriminator folds and the real pass of the spectral-norm
-        stack, which do not depend on the generator, already run on the side stream."""
+        """Phase D.  The discriminator folds and the real pass of the spectral-norm stack need neither the generator nor
+        x_pred: they run on the side stream while the current stream runs `head`, the generator fold + forward and - once
+        the fake pass's folds are there - the fake pass.  `head` (captured step): the pending generator update of the
+        previous step."""
         head = head or (lambda: None)
         if not self.use_adv:
             head()
             self._g_forward(su, sess, mode, x_pred)
             return
-        if self.concurrent_d:
-            # side stream: D folds and the real pass, which needs neither G nor x_pred; current stream: G fold +
-            # generator forward, then - once the fake pass's folds are there - the fake pass
-            cur = torch.cuda.current_stream()
-            self._fork()
-            self._sm_scope(True)           # beside the deferred exchange of the previous step's last generator bucket (head)
-            with torch.cuda.stream(self._side):
-                self._d_folds()
-                self._d_real(x_real)
-            head()
-            self._sm_scope(False)
-            self._g_forward(su, sess, mode, x_pred)
-            cur.wait_event(self._ev_f1)
-            self._d_fake()
-            self._join()
-        else:
-            self._d_folds()
-            head()
-            self._g_forward(su, sess, mode, x_pred)
-            self._d_fake()
-            self._d_real(x_real)
-        self._sm_scope(True)               # the discriminator gradient is exchanged group by group during its backward
-        self._d_update()
-        self._sm_scope(False)
+        _, heavy, p_idx, s_idx = self._split_subs()
+        cur = torch.cuda.current_stream()
+        self._fork()
+        with torch.cuda.stream(self._side):
+            # folds of the fake pass (f1) and of the real pass (f2): the spectral-norm power iterations of the two
+            # forwards happen in that order (train.py:190-191)
+            refold_d = not self._d_folded
+            self._d_folded = True
+            f1 = self._fold_d(refold_d)
+            ev_f1 = torch.cuda.Event()
+            ev_f1.record(self._side)
+            f2 = self._fold_d(False)
+            real_h = self._disc_forward(x_real, f2, heavy)
+        head()
+        self._g_forward(su, sess, mode, x_pred)
+        cur.wait_event(ev_f1)
+        x_cat = torch.cat([self.x_pred, x_real], 0)
+        # current: fake pass of the spectral-norm stack | side2[1]: S stacks batched | side2[0]: P stacks batched
+        (s_b, p_b), fake_h = passes.fork_join(
+            self._side2[1], lambda: passes.fork_join(self._side2[0], lambda: self._disc_forward(x_cat, f1, p_idx, self._ps),
+                                                     lambda: self._disc_forward(x_cat, f1, s_idx, self._ss))[::-1],
+            lambda: self._disc_forward(self.x_pred, f1, heavy))
+        self._join()
+        self._d_update(fake_h, real_h, p_b, s_b)
 
     def _phase_g_head(self, x_real: Tensor, update_d: bool = True) -> None:
         """Phase G up to and including the generator backward of the first (rearmost) gradient bucket."""
         dx_pred = self._g_losses(x_real, update_d)
         # generator backward, bucket by bucket (G.grad was zeroed in phase D and this is its only writer: overwrite)
         self._last_gctx = self._gctx                       # kept for the parity tests (references only)
-        self._gb = passes.GenBackward(self.net_g, self._gctx, dx_pred, plan=self.g_plan, side=self._s2(1), res_side=self._s2(0),
+        self._gb = passes.GenBackward(self.net_g, self._gctx, dx_pred, plan=self.g_plan, side=self._side2[1], res_side=self._side2[0],
                                       overwrite_grads=True)
         self._g_bucket(0)
 
@@ -477,13 +413,13 @@ class GanTrainer:
             ev = torch.cuda.Event()
             ev.record(torch.cuda.current_stream())
             self._enc.wait_event(ev)
-            with torch.cuda.stream(self._enc if self.concurrent_d else torch.cuda.current_stream()):
+            with torch.cuda.stream(self._enc):
                 dx_enc, self._enc_units, self._enc_logits = pe.encoder_losses(
                     self._enc_plan, x_pred, self._cur_su, self._cur_ph, self.slots[6:8], self.w_su, self.w_ph, True,
                     self.use_su, self.use_ph)
                 enc_ev = torch.cuda.Event()
                 enc_ev.record(torch.cuda.current_stream())
-        if self.use_td and self.use_adv and self.concurrent_d:
+        if self.use_td and self.use_adv:
             # the time-domain loss needs only x_real / x_pred: it runs on its own stream beside the discriminator passes
             ev = torch.cuda.Event()
             ev.record(torch.cuda.current_stream())
@@ -497,43 +433,23 @@ class GanTrainer:
                 self.D.adamw(self.lr_dev, grad_scale=self.reducer.grad_scale)   # train.py:199
             refold_d = update_d or not self._d_folded
             self._d_folded = True
-            if self.concurrent_d:
-                # The fake and the real pass use the same weights - except in the spectral-norm sub-discriminator (the
-                # full-rate scale stack), whose sigma advances between the two forwards.  So: that sub-discriminator
-                # runs once per pass (fake on the side stream as soon as its folds are there, real after the second
-                # power iteration), and ALL THE OTHERS run ONCE on the concatenated batch [x_pred | x_real]: half the
-                # launches and twice the rows per launch for layers that had too few tiles to fill the chip.
-                subs = passes.disc_subnets(self.net_d)
-                heavy, rest = passes._heavy_split(subs)
-                p_idx = [i for i in rest if subs[i][0] == "P"]
-                s_idx = [i for i in rest if subs[i][0] == "S"]
-                Bq = x_pred.shape[0]
-                f3 = self._fold_d(refold_d)
-                x_cat = torch.cat([x_pred, x_real], 0)
-                fwd = lambda x, f, idx: passes.discriminator_forward(self.net_d, x, dt, f, subset=idx,
-                                                                     spread=self._ps if idx is p_idx else (self._ss if idx is s_idx else None)) if idx else (None, None)
-                self._fork()
-                with torch.cuda.stream(self._side):       # side: fake pass of the spectral-norm stack | its side: S stacks, batched
-                    (rs, cs), (rh_f, ch_f) = passes.fork_join(self._s2(0), lambda: fwd(x_cat, f3, s_idx), lambda: fwd(x_pred, f3, heavy))
-                f4 = self._fold_d(False)                  # current: second power iteration, then real pass of that stack | P stacks, batched
-                (rh_r, _), (rp, cp) = passes.fork_join(self._s2(1), lambda: fwd(x_real, f4, heavy), lambda: fwd(x_cat, f3, p_idx))
-                self._join()
-                res_f, res_r, sub_f = [None] * len(subs), [None] * len(subs), [None] * len(subs)
-                for r_b, c_b, idx in ((rp, cp, p_idx), (rs, cs, s_idx)):
-                    if idx:
-                        a, b, sa = passes.split_disc_batch(r_b, c_b, idx, Bq)
-                        for i in idx:
-                            res_f[i], res_r[i], sub_f[i] = a[i], b[i], sa[i]
-                for i in heavy:
-                    res_f[i], res_r[i], sub_f[i] = rh_f[i], rh_r[i], ch_f.subs[i]
-                assert all(r is not None for r in res_f)
-                ctx_f = passes.DiscCtx(B=Bq, T=x_pred.shape[1], C=x_pred.shape[2], dtype=dt, folds=f3, subs=sub_f)
-                ctx_f.keep = (ch_f, cp, cs, x_cat)
-            else:
-                f3 = self._fold_d(refold_d)
-                f4 = self._fold_d(False)
-                res_f, ctx_f = passes.discriminator_forward(self.net_d, x_pred, dt, f3)
-                res_r, _ = passes.discriminator_forward(self.net_d, x_real, dt, f4)
+            # the split of phase D: the spectral-norm stack once per pass (fake on the side stream, real after the second
+            # power iteration), all the others once on [x_pred | x_real]
+            _, heavy, p_idx, s_idx = self._split_subs()
+            f3 = self._fold_d(refold_d)
+            x_cat = torch.cat([x_pred, x_real], 0)
+            self._fork()
+            with torch.cuda.stream(self._side):       # side: fake pass of the spectral-norm stack | its side: S stacks, batched
+                s_b, fake_h = passes.fork_join(self._side2[0], lambda: self._disc_forward(x_cat, f3, s_idx, self._ss),
+                                               lambda: self._disc_forward(x_pred, f3, heavy))
+            f4 = self._fold_d(False)                  # current: second power iteration, then real pass of that stack | P stacks, batched
+            real_h, p_b = passes.fork_join(self._side2[1], lambda: self._disc_forward(x_real, f4, heavy),
+                                           lambda: self._disc_forward(x_cat, f3, p_idx, self._ps))
+            self._join()
+            res_f, res_r, sub_f = self._per_pass(heavy, fake_h, real_h, ((p_b, p_idx), (s_b, s_idx)))
+            assert all(r is not None for r in res_f)
+            ctx_f = passes.DiscCtx(B=x_pred.shape[0], T=x_pred.shape[1], C=x_pred.shape[2], dtype=dt, folds=f3, subs=sub_f)
+            ctx_f.keep = (fake_h[1], p_b[1], s_b[1], x_cat)
             self.d_folds = f4
             self._last_g_fmaps = (res_f, res_r)             # kept for the parity tests (references only)
             nd = len(res_f)
@@ -547,7 +463,7 @@ class GanTrainer:
             else:
                 dfm = [[None] * (len(fm_f) - 1) for fm_f in res_f]
             dx_d = passes.discriminator_backward(self.net_d, ctx_f, dlog, dfm, want_input_grad=True, want_weight_grad=False,
-                                                 side=self._s2(0), spread=self._ps if self.concurrent_d else None)
+                                                 side=self._side2[0], spread=self._ps)
             if td_ev is not None:
                 torch.cuda.current_stream().wait_event(td_ev)
             ops.axpy_f32(dx_pred, dx_d, 1.0)
@@ -569,17 +485,16 @@ class GanTrainer:
         if i == len(self.g_buckets) - 1:
             self._gb = self._gctx = None
 
-    def _phase_g(self, x_real: Tensor, update_d: bool = True, reduce: bool = False, defer_last: bool = False) -> list:
+    def _phase_g(self, x_real: Tensor, update_d: bool = True, reduce: bool = False) -> list:
         """Phase G; with reduce=True the all-reduce of each generator-gradient bucket is issued as soon as the bucket is
         final (it then overlaps the backward of the buckets in front of it).  Returns the pending all-reduce handles
-        (own communicator: events).  defer_last: the last bucket is NOT exchanged here (see _opt_g_head)."""
+        (own communicator: events)."""
         handles = []
         self._phase_g_head(x_real, update_d)
-        n = len(self.g_buckets)
-        for i in range(n):
+        for i in range(len(self.g_buckets)):
             if i > 0:
                 self._g_bucket(i)
-            if reduce and not (defer_last and i == n - 1):
+            if reduce:
                 handles += self._reduce_g_bucket(i)
         return handles
 
@@ -624,7 +539,6 @@ class GanTrainer:
                 self._g_bucket(i)
             lo, hi = self.g_buckets[i][4]
             ev = self._reduce(self.G.grad[lo:hi])
-            self._sm_scope(True)           # the buckets in front run their backward beside this exchange
             if ev is None:                      # no data-parallel group: the slice is final now, fork the side stream here
                 ev = torch.cuda.Event()
                 ev.record(torch.cuda.current_stream())
@@ -636,7 +550,6 @@ class GanTrainer:
             evs.append(done)
         if n > 1:
             self._g_bucket(n - 1)
-        self._sm_scope(False)
         self._wait_events(evs)
         self._pend.fill_(1)
 
@@ -665,32 +578,23 @@ class GanTrainer:
         self._phase_d(None, None, None, x_real, x_pred=x_pred)
         return self._g_losses(x_real, update_d=True)
 
-    def capture(self, batch: int, frames: int, unit_dim: int = 256, hop: int = 16, channels: int = 8,
-                pipelined: Optional[bool] = None, fused: Optional[bool] = None) -> None:
-        """Capture the step as CUDA graphs over static input buffers.  Two eager
-        warm-up steps run first (allocator / lazy-initialisation warm-up, on all-zero inputs); the trainer's state -
-        parameters, AdamW moments and step counters, spectral-norm u / v, loss slots - is snapshotted before and
+    def capture(self, batch: int, frames: int, unit_dim: int = 256, hop: int = 16, channels: int = 8) -> None:
+        """Capture the whole step (_fused_step) as ONE CUDA graph over static input buffers, plus the graph that flush()
+        replays.  With the own NCCL communicator the gradient all-reduces are graph nodes too, so a replay has no
+        host-side seam; data parallelism over any other process group is refused (train with step() there).  The
+        generator update of step k is left pending on the device (flag `_pend`) and runs at the head of replay k+1,
+        beside that step's discriminator folds and real pass, which depend on neither the generator nor its gradient;
+        flush() applies a pending update on its own (the eager step(), checkpointing, `lr` changes and the inference
+        engine call it).
+
+        Two eager warm-up steps run first (allocator / lazy-initialisation warm-up, on all-zero inputs); the trainer's
+        state - parameters, AdamW moments and step counters, spectral-norm u / v, loss slots - is snapshotted before and
         restored after them, so capture() leaves the training state exactly as it found it (resume-then-capture is
-        safe, and `steps` in the next checkpoint still counts real steps only).
-
-        fused (the default; STG_FUSED_GRAPH=0 or an explicit `pipelined` switch it off): the WHOLE step is ONE graph
-        (_fused_step) - with the own NCCL communicator the gradient all-reduces are graph nodes too, so a replay has no
-        host-side seam.  The generator update of step k is left pending on the device (flag `_pend`) and runs at the head
-        of replay k+1, beside that step's discriminator folds and real pass, which depend on neither the generator nor its
-        gradient; flush() applies a pending update on its own (the eager step(), checkpointing, `lr` changes and the
-        inference engine call it).  Measured on one B200 (tools/piece_times.py): the five-plus-two graphs of the
-        pipelined form cost ~0.2 ms per step in launch seams (pieces 3.80 ms, step 4.02 ms).
-
-        pipelined (round-1 form): phase D is captured as its five pieces (see _d_folds) and step_graph()
-        software-pipelines consecutive steps on the host: the all-reduce of the generator gradient and the generator's
-        AdamW of step k run WHILE step k+1's discriminator folds and real pass are already executing; pipelined=False:
-        three graphs (phase D, phase G per bucket, generator AdamW) replayed back to back."""
+        safe, and `steps` in the next checkpoint still counts real steps only)."""
+        if self.reducer.enabled and not self._inline:
+            raise RuntimeError("GanTrainer.capture: data-parallel graph capture needs the own NCCL communicator, i.e. a "
+                               "process group with the nccl backend on CUDA devices; train with step() over this group")
         dev = self.device
-        import os
-        if fused is None:
-            fused = pipelined is None and os.environ.get("STG_FUSED_GRAPH", "1") != "0"
-        if pipelined is None:
-            pipelined = self.concurrent_d and self.use_adv and os.environ.get("STG_PIPELINE", "1") != "0"
         self.flush()
         self._fused = None
         self._static = dict(
@@ -710,95 +614,33 @@ class GanTrainer:
         torch.cuda.synchronize()
         self._restore_state(snap)
         torch.cuda.synchronize()
-        pool = torch.cuda.graph_pool_handle()
-        G = torch.cuda.CUDAGraph
-        # (data parallel: the process group's watchdog thread may touch the CUDA API while we capture)
-        gkw = dict(capture_error_mode="thread_local") if self.reducer.enabled else {}
-        if fused:
-            # Data parallel: the persistent conv / wgrad kernels take one CTA per SM with (nearly) the whole register file,
-            # so a concurrent NCCL kernel only finds room on SMs that a launch leaves idle - measured at N = 8, the
-            # all-reduces then cost their full stand-alone time (0.67 ms for the 141 MB of a step) however they are
-            # overlapped.  STG_NCCL_SMS=R keeps R SMs free of them for the communicator inside this graph.
-            from . import _lib as _l
-            # Measured at N = 2 (bench.py, ms per step): R = 0: 4.32, 8: 4.70 (with 8 NCCL channels), 16: 4.25, 24: 4.31; capping
-            # NCCL's channel count to R always lost.  Default 16.
-            reserve = int(os.environ.get("STG_NCCL_SMS", "16")) if self.reducer.enabled else 0
-            n_sm = torch.cuda.get_device_properties(dev).multi_processor_count
-            step_g, flush_g = G(), G()
-            self._pend.zero_()
-            # STG_NCCL_SCOPE=1: reserve only in the pieces that run beside an exchange (_sm_scope) instead of the whole graph.
-            # Measured at N = 2: 4.27 ms scoped vs 4.25 ms whole-graph - the step does not notice 16 SMs more or less
-            # (DESIGN.md 3.4), so the simpler whole-graph reservation stays the default.
-            scoped = os.environ.get("STG_NCCL_SCOPE", "0") == "1"
-            if reserve > 0:
-                if scoped:
-                    self._sm_reserve = reserve
-                else:
-                    _l.load().stg_set_sm_limit(n_sm - reserve)
-            try:
-                with torch.cuda.graph(step_g, pool=pool, **gkw):
-                    self._fused_step(s)
-            finally:
-                self._sm_reserve = 0
-                if reserve > 0:
-                    _l.load().stg_set_sm_limit(0)
-            with torch.cuda.graph(flush_g, pool=pool, **gkw):
-                self._opt_g_head()
-            self._pend.zero_()
-            self._fused, self._graphs, self._d_graphs, self._pending_host = (step_g, flush_g), None, None, False
-            return
-        # graphs that replay beside a gradient all-reduce leave a few SMs to the communicator (STG_NCCL_SMS, default 0 =
-        # off: the persistent conv kernels otherwise hold every SM and the NCCL CTAs only get in between launches)
-        import contextlib, os
+        gkw = dict(pool=torch.cuda.graph_pool_handle())
+        if self.reducer.enabled:      # the process group's watchdog thread may touch the CUDA API while we capture
+            gkw["capture_error_mode"] = "thread_local"
+        # Data parallel: the persistent conv / wgrad kernels take one CTA per SM with (nearly) the whole register file,
+        # so a concurrent NCCL kernel only finds room on SMs that a launch leaves idle - measured at N = 8, the
+        # all-reduces then cost their full stand-alone time (0.67 ms for the 141 MB of a step) however they are
+        # overlapped.  STG_NCCL_SMS=R keeps R SMs free of them for the communicator inside this graph.
+        # Measured at N = 2 (bench.py, ms per step): R = 0: 4.32, 8: 4.70 (with 8 NCCL channels), 16: 4.25, 24: 4.31; capping
+        # NCCL's channel count to R always lost.  Default 16.
+        import os
         from . import _lib
-        reserve = int(os.environ.get("STG_NCCL_SMS", "0")) if self.reducer.enabled else 0
+        reserve = int(os.environ.get("STG_NCCL_SMS", "16")) if self.reducer.enabled else 0
         n_sm = torch.cuda.get_device_properties(dev).multi_processor_count
-
-        @contextlib.contextmanager
-        def beside_allreduce():
+        step_g, flush_g = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
+        self._pend.zero_()
+        if reserve > 0:
+            _lib.load().stg_set_sm_limit(n_sm - reserve)
+        try:
+            with torch.cuda.graph(step_g, **gkw):
+                self._fused_step(s)
+        finally:
             if reserve > 0:
-                _lib.load().stg_set_sm_limit(n_sm - reserve)
-            try:
-                yield
-            finally:
-                if reserve > 0:
-                    _lib.load().stg_set_sm_limit(0)
-        if pipelined:
-            # the two rows of phase D replay CONCURRENTLY: they must not share a memory pool (blocks freed while one
-            # was captured would be handed to the other)
-            pool_a = torch.cuda.graph_pool_handle()
-            a1, a2, b1, b2, b3 = G(), G(), G(), G(), G()
-            with beside_allreduce():      # (the deferred last bucket of the previous step)
-                with torch.cuda.graph(a1, pool=pool_a, **gkw):
-                    self._d_folds()
-                with torch.cuda.graph(a2, pool=pool_a, **gkw):
-                    self._d_real(s["x_real"])
-            with torch.cuda.graph(b1, pool=pool, **gkw):
-                self._g_forward(s["su"], s["sess"], s["mode"])
-            with torch.cuda.graph(b2, pool=pool, **gkw):
-                self._d_fake()
-            with torch.cuda.graph(b3, pool=pool, **gkw):
-                self._d_update()
-            self._d_graphs = (a1, a2, b1, b2, b3)
-            self._pipe = torch.cuda.Stream(device=dev)
-            self._pipe_ev = [torch.cuda.Event() for _ in range(3)]
-            g1 = None
-        else:
-            self._d_graphs = None
-            g1 = G()
-            with torch.cuda.graph(g1, pool=pool, **gkw):
-                self._phase_d(s["su"], s["sess"], s["mode"], s["x_real"])
-        # phase G: one graph per generator-gradient bucket (the bucket's all-reduce is issued between them)
-        g2 = [G() for _ in self.g_buckets]
-        with torch.cuda.graph(g2[0], pool=pool, **gkw):
-            self._phase_g_head(s["x_real"])
-        for i in range(1, len(g2)):
-            with beside_allreduce(), torch.cuda.graph(g2[i], pool=pool, **gkw):
-                self._g_bucket(i)
-        g3 = G()
-        with torch.cuda.graph(g3, pool=pool, **gkw):
-            self._phase_opt_g()
-        self._graphs = (g1, g2, g3)
+                _lib.load().stg_set_sm_limit(0)
+        with torch.cuda.graph(flush_g, **gkw):
+            self._opt_g_head()
+        self._pend.zero_()
+        self._fused, self._pending_host = (step_g, flush_g), False
 
     def _sn_buffers(self) -> list:
         return [b for c in passes.discriminator_convs(self.net_d) if c.norm != "weight_norm" for b in (c.weight_u, c.weight_v)]
@@ -827,20 +669,16 @@ class GanTrainer:
         self._d_folded = True
 
     def flush(self) -> None:
-        """Complete a deferred generator update (fused graph: the device flag `_pend` is set; pipelined graphs: wait for
-        the generator-gradient all-reduce, then the optimiser graph)."""
-        if self._pending_host and self._fused is not None:
+        """Complete the generator update that the last step_graph() left pending: exchange of the last gradient bucket
+        (data parallel) and its AdamW, under the device flag `_pend`, which it clears."""
+        if self._pending_host:
             self._pending_host = False
-            self._fused[1].replay()           # (exchange of the last bucket +) AdamW under the flag, which it clears
-        if self._pending_g is not None:
-            self._wait_handles(self._pending_g)
-            self._pending_g = None
-            self._graphs[2].replay()
+            self._fused[1].replay()
 
     def step_graph(self, speech_units: Tensor, session_ids: Tensor, x_real: Tensor,
                    speaking_mode_ids: Optional[Tensor] = None, phoneme_targets: Optional[Tensor] = None) -> Tensor:
         """Replay the captured step; inputs may be pinned-host or device tensors (copied into the static buffers).
-        With a pipelined capture the generator optimiser of this step is deferred into the next call (or flush())."""
+        The generator update of this step stays pending until the next replay or flush()."""
         s = self._static
         s["su"].copy_(speech_units, non_blocking=True)
         s["sess"].copy_(session_ids, non_blocking=True)
@@ -853,41 +691,8 @@ class GanTrainer:
             if phoneme_targets is None:
                 raise ValueError("step_graph: the EMG-encoder losses are on - pass phoneme_targets")
             s["ph"].copy_(phoneme_targets, non_blocking=True)
-        if self._fused is not None:
-            self._fused[0].replay()
-            self._pending_host = True
-            return self.slots
-        g1, g2, g3 = self._graphs
-        def phase_g() -> list:
-            handles = []
-            for i, gr in enumerate(g2):
-                gr.replay()
-                handles += self._reduce_g_bucket(i)     # overlaps the next bucket's backward
-            return handles
-        if self._d_graphs is None:
-            g1.replay()
-            if not self._inline:
-                self.reducer.all_reduce(self.D.grad)
-            self._wait_handles(phase_g())
-            g3.replay()
-            return self.slots
-        a1, a2, b1, b2, b3 = self._d_graphs
-        ev0, ev_f, ev_r = self._pipe_ev
-        cur = torch.cuda.current_stream()
-        ev0.record(cur)                       # inputs copied, previous step's phase G done
-        self._pipe.wait_event(ev0)
-        with torch.cuda.stream(self._pipe):
-            a1.replay(); ev_f.record(self._pipe)
-            a2.replay(); ev_r.record(self._pipe)
-        self.flush()                          # previous step: all-reduce(G) + AdamW(G), beside a1 / a2
-        b1.replay()
-        cur.wait_event(ev_f)
-        b2.replay()
-        cur.wait_event(ev_r)
-        b3.replay()
-        if not self._inline:
-            self.reducer.all_reduce(self.D.grad)
-        self._pending_g = phase_g()
+        self._fused[0].replay()
+        self._pending_host = True
         return self.slots
 
     def save_checkpoint(self, directory, steps: int, epoch: int, final: bool = False) -> None:

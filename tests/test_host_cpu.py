@@ -92,7 +92,7 @@ def _dp_worker(rank, world, port, out):
     flat = torch.arange(8.0) * (r + 1)
     red.broadcast(flat, src=0)
     # the bucket-by-bucket exchange of the generator gradient: slices reduced asynchronously, back to front, waited on
-    # together (trainer._reduce_g_bucket / flush)
+    # together (trainer._reduce_g_bucket / _wait_handles)
     g2 = torch.full((900,), float(r + 1))
     handles = []
     for lo_, hi_ in ((600, 900), (300, 600), (0, 300)):
@@ -112,6 +112,16 @@ def test_data_parallel_gloo_world2():
     out = mgr.dict()
     mp.spawn(_dp_worker, args=(2, port, out), nprocs=2, join=True)
     assert out[0] == (True, 0, 16) and out[1] == (True, 16, 32)
+
+
+def test_capture_refuses_data_parallel_without_own_communicator():
+    """Over a group that is not CUDA + NCCL (no own communicator) the gradient exchange cannot be captured: capture()
+    says so before it runs anything (here: on a trainer with nothing but its reducer set)."""
+    from ste_gan_b200.trainer import GanTrainer
+    tr = object.__new__(GanTrainer)
+    tr.reducer, tr._inline = types.SimpleNamespace(enabled=True, comm=None), False
+    with pytest.raises(RuntimeError, match="own NCCL communicator"):
+        tr.capture(2, 64)
 
 
 def test_precision_context():

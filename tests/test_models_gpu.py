@@ -363,7 +363,7 @@ def test_cuda_graph_step_matches_eager():
     a, b = t1.losses(), t2.losses()
     for k in a:
         assert abs(a[k] - b[k]) <= 2e-2 * max(1.0, abs(a[k])), (k, a[k], b[k])
-    # the pipelined replay defers the last generator optimiser step: flush(), then the parameters agree as well
+    # the replay defers the last generator optimiser step: flush(), then the parameters agree as well
     assert t2._fused is not None and t2._pending_host      # the default capture: ONE graph per step, generator update pending
     t2.flush()
     # Tolerance: the weight-gradient reductions (TMA reduce-add, atomics) are order-nondeterministic, and AdamW's first
@@ -372,19 +372,18 @@ def test_cuda_graph_step_matches_eager():
     assert O.rel_l2(t2.G.flat, t1.G.flat) < 3e-3 and O.rel_l2(t2.D.flat, t1.D.flat) < 3e-3
 
 
-def test_cuda_graph_step_unpipelined_matches_pipelined():
-    """The round-1 capture forms stay available: single-graph phase D (pipelined=False) and the five-graph pipelined replay
-    run the same kernels."""
+def test_cuda_graph_step_three_buckets_matches_eager():
+    """The three-bucket generator backward under capture - AdamW per bucket on the communication stream (keep_step for
+    all but the first), the last bucket deferred behind the device flag - against the eager one-bucket step."""
     from ste_gan_b200.trainer import GanTrainer
     su, sess, x_real = (t.cuda() for t in O.synthetic_batch(2, 100, seed=7))
     g1, d1 = _fresh_nets(); g2, d2 = _fresh_nets()
     t1 = GanTrainer(g1.cuda(), d1.cuda(), precision="bf16")                    # one gradient bucket (no data-parallel group)
     t2 = GanTrainer(g2.cuda(), d2.cuda(), precision="bf16", grad_buckets=3)    # the three-bucket generator backward
     assert len(t1.g_buckets) == 1 and len(t2.g_buckets) == 3
-    t1.capture(2, 100, pipelined=False)
-    t2.capture(2, 100, pipelined=True)
+    t2.capture(2, 100)
     for _ in range(3):
-        t1.step_graph(su, sess, x_real)
+        t1.step(su, sess, x_real)
         t2.step_graph(su, sess, x_real)
     t2.flush()
     a, b = t1.losses(), t2.losses()
@@ -588,7 +587,7 @@ def test_average_filter_module(window, pad):
 
 
 def test_data_parallel_matches_single_process():
-    """N ranks through the bucketed, pipelined graph step == one process on the global batch (tools/dp_check.py under
+    """N ranks through the bucketed graph step == one process on the global batch (tools/dp_check.py under
     torchrun, 2 GPUs, fp32).  Skipped on single-GPU boxes; the log of the last multi-GPU run is kept under profiles/."""
     import subprocess, sys
     if torch.cuda.device_count() < 2:

@@ -1,4 +1,4 @@
-"""Data-parallel correctness check (GPU, 2+ ranks): N ranks x B samples through the pipelined / bucketed graph step vs ONE
+"""Data-parallel correctness check (GPU, 2+ ranks): N ranks x B samples through the bucketed graph step vs ONE
 process on the global batch (eager step, no exchange).  fp32 validation mode, 2 optimiser steps.
     torchrun --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 tools/dp_check.py"""
 import os, sys
