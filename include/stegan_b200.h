@@ -416,10 +416,10 @@ int stg_debug_row_classes(int t_dst, int* out);
 int stg_debug_tma_bw(const void* buf, long long n_rows, int box_rows, int n_iters, int mode, int stages, int grid, long long* clk,
                      stg_stream_t stream);
 /* Host-only diagnostic: the plan the tcgen05 convolution engine would launch for `d` (only the geometry is read; pointers
- * just need to be non-NULL where the call would use them).  out[16] = { column tile bn, staged epilogue, taps per stage (tap
- * window), main-loop stages, dynamic shared memory bytes, two CTAs per SM, CTA pairs, row classes, tiles, grid, compact-group K
- * (0: none), 64-channel chunks per tap, TMEM columns, epilogue-operand ring depth (0: no operands), output ring depth,
- * output-row residue classes }.  STG_EUNSUPPORTED when the engine does not take the shape.  No GPU needed. */
+ * just need to be non-NULL where the call would use them).  out[15] = { column tile bn, staged epilogue, taps per stage (tap
+ * window), main-loop stages, dynamic shared memory bytes, two CTAs per SM, row classes, tiles, grid, compact-group K (0: none),
+ * 64-channel chunks per tap, TMEM columns, epilogue-operand ring depth (0: no operands), output ring depth, output-row
+ * residue classes }.  STG_EUNSUPPORTED when the engine does not take the shape.  No GPU needed. */
 int stg_debug_conv_plan(const StgConv* d, int* out);
 /* debug accounting (host side): bytes the tcgen05 launches since the last reset were planned to pull into shared memory
  * through TMA (main-loop operands + epilogue operands). */

@@ -1,5 +1,4 @@
 // extern "C" entry points that dispatch between the engines, plus diagnostics.
-#include <stdlib.h>
 #include <string.h>
 
 #include <string>
@@ -11,7 +10,7 @@ namespace stg {
 static thread_local std::string g_last_error;
 unsigned long long g_launch_count = 0;
 double g_ingest_bytes = 0.0;
-int g_sm_limit = getenv("STG_SM_LIMIT") ? atoi(getenv("STG_SM_LIMIT")) : 0;   // stg_set_sm_limit: SMs the persistent tcgen05 kernels may occupy (0 = all)
+int g_sm_limit = 0;   // stg_set_sm_limit: SMs the persistent tcgen05 kernels may occupy (0 = all)
 
 void set_cuda_error(cudaError_t e, const char* where) {
   g_last_error = std::string(cudaGetErrorName(e)) + ": " + cudaGetErrorString(e) + " at " + where;

@@ -28,8 +28,6 @@
 //           wavefront per 16 bytes and made the epilogue, not the MMAs, the critical path).
 //   DIRECT  (fp32 outputs, 1-channel logits, strided data-gradients): 8 warps, row-per-thread global
 //           loads/stores with the next chunk's operands prefetched.
-#include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "tc_common.cuh"
@@ -76,10 +74,7 @@ struct TcP {
   int cs_g, cd_g;          // source / destination channels per (packed) group
   int n_res, tiles_m;      // output-row residues (1 unless transposed && stride > 1), row tiles per residue
   int tiles_n, n_tiles;    // column tiles, total tiles = B * n_res * tiles_m * tiles_n
-  // CTA pairs (cta_group::2, kPair kernels): a "tile" is a PAIR tile = 2 row tiles x one column tile; the row tiles of a
-  // residue class are numbered mt = b * tiles_m + tm and the CTA of cluster rank r takes mt = 2 * pair + r.  An odd count
-  // leaves the last pair's rank-1 CTA with b == n_samples: its loads are zero-filled and its stores clipped by the TMA unit.
-  int n_samples, pairs_per_res;
+  int n_samples;           // a row-class tail tile may gather rows past the last sample (zero-filled loads, clipped stores)
   // Row classes (staged, stride-1, single-phase kernels): T rows per sample rarely fill whole 128-row tiles (T = 100 /
   // 200 / 400: 78 %).  The rows of a sample are cut into 128-row tiles plus a binary tail (64 / 32 / 16 / 8 rows), and a
   // tail tile gathers the SAME seg-row slice of 128 / seg consecutive samples with one (C, seg rows, samples) TMA box -
@@ -196,18 +191,13 @@ __device__ __forceinline__ void life_ev(long long* tr, int tag) {
 struct Tile {
   int b, res, h0, col0, ch0, wcol0, g0, n_iters, cls;
 };
-template <bool kPair>
-__device__ __forceinline__ Tile decode_tile(const TcP& p, int t, int rank) {
+__device__ __forceinline__ Tile decode_tile(const TcP& p, int t) {
   Tile x;
   const int tn = t % p.tiles_n; int u = t / p.tiles_n;
   int tm;
   // strided data-gradient: output rows h = h' * n_res + res are produced per residue class `res` from the
   // taps j with (res + pad - j*dilation) % stride == 0, as a stride-1 correlation over h'
-  if constexpr (kPair) {
-    const int pm = u % p.pairs_per_res; x.res = u / p.pairs_per_res;
-    const int mt = 2 * pm + rank;
-    x.b = mt / p.tiles_m; tm = mt - x.b * p.tiles_m;
-  } else if (p.n_cls > 1) {
+  if (p.n_cls > 1) {
     int c = 0;
     while (c + 1 < p.n_cls && u >= p.cls_mt0[c + 1]) ++c;
     const int idx = u - p.cls_mt0[c];
@@ -318,22 +308,19 @@ __device__ __forceinline__ void epi_store(const TcEpi& e, int b, int row, int co
 
 // ---------------------------------------------------------------------------------------------- kernel
 // kMask: stg_conv_masked (per-sample length masks in both epilogues); the unmasked instances compile without them
-template <bool kStaged, bool kPair, bool kMask>
-__global__ void __launch_bounds__(kStaged ? 384 : 352, (kStaged && !kPair) ? 2 : 1)
+template <bool kStaged, bool kMask>
+__global__ void __launch_bounds__(kStaged ? 384 : 352, kStaged ? 2 : 1)
 conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtensorMap tmW,
                const __grid_constant__ EpiMaps em, const TcP p) {
   constexpr int EPI_WARPS = 8;   // warps that read the accumulator (arrivals on tmem_empty)
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment for SWIZZLE_128B tiles
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  // B tile bytes staged by THIS CTA per tap (a pair splits the columns; compact groups: only the rows of the chunk's units)
-  const int b_bytes = p.cu_k ? p.cu_fpc * p.cu_n * p.cu_k * 2 : (kPair ? p.bn / 2 : p.bn) * KC * 2;
+  // B tile bytes per tap (compact groups: only the rows of the chunk's units)
+  const int b_bytes = p.cu_k ? p.cu_fpc * p.cu_n * p.cu_k * 2 : p.bn * KC * 2;
   const int stage_bytes = p.a_bytes + p.max_ntaps * b_bytes;
   const TcEpi& e = p.e;
-  // pair kernels: cluster rank (0 = leader: issues the MMAs, owns the full / tmem_empty barriers), pair tile walk
-  const int rank = kPair ? __shfl_sync(0xffffffffu, (int)cluster_ctarank(), 0) : 0;
-  const int tile0 = kPair ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
-  const int tstep = kPair ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+  const int tile0 = (int)blockIdx.x, tstep = (int)gridDim.x;
   const uint32_t epi_base = smem_base + p.stages * stage_bytes;           // staged: (n_in << in_sh) + 3 n_out slots + bias
   const uint32_t bias_base = epi_base + (kStaged ? ((e.n_in << e.in_sh) + p.out_ring * e.n_out) * SLOT : 0);
   const uint32_t bar_base = bias_base + (kStaged ? 2048 : 0);   // one bias copy per epilogue team
@@ -355,30 +342,19 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
     for (int c = 0; c < p.n_cls; ++c) prefetch_tmap(&tmA4.m[c]);
     prefetch_tmap(&tmW);
     for (int s = 0; s < p.stages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-    for (int a = 0; a < 2; ++a) { mbar_init(tmem_full_bar(a), 1); mbar_init(tmem_empty_bar(a), kPair ? 2 * EPI_WARPS : EPI_WARPS); }
+    for (int a = 0; a < 2; ++a) { mbar_init(tmem_full_bar(a), 1); mbar_init(tmem_empty_bar(a), EPI_WARPS); }
     for (int a = 0; a < 8; ++a) mbar_init(in_bar(a), 1);
     fence_barrier_init();
   }
-  if (warp == 1) {
-    if constexpr (kPair) { tmem_alloc_2sm(tmem_slot, (uint32_t)p.tmem_cols); tmem_relinquish_2sm(); }
-    else { tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols); tmem_relinquish(); }
-  }
+  if (warp == 1) { tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols); tmem_relinquish(); }
   tc_fence_before();
-  if constexpr (kPair) cluster_sync_all();   // the peer's barriers are initialised before anything arrives on them
-  else __syncthreads();
+  __syncthreads();
   tc_fence_after();
   life_ev(p.trace, 31);
   pdl_wait();      // everything above overlapped the previous kernel's tail; no global memory is touched before this line
   life_ev(p.trace, 32);
   uint32_t tmem_base;
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
-  // pair: stage-full barriers and the accumulator-drained barriers that count live in the LEADER's shared memory
-  const uint32_t lead_bars = kPair ? mapa_u32(bar_base, 0) : bar_base;
-  auto lead_full_bar = [&](int s) { return lead_bars + 8u * s; };
-  auto lead_tmem_empty_bar = [&](int a) { return lead_bars + 8u * (2 * MAX_STAGES + 2 + a); };
-  auto arrive_tmem_empty = [&](int a) {
-    if constexpr (kPair) mbar_arrive_cluster(lead_tmem_empty_bar(a)); else mbar_arrive(tmem_empty_bar(a));
-  };
 
   // Two producer warps: warp 0 loads the A (activation) boxes and posts the stage's expect_tx, the LAST warp of the CTA
   // loads the W boxes of the same stage onto the same barrier (its complete_tx may land before the expect_tx - both
@@ -395,19 +371,18 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
     const bool lead = lane == 0;
     Tracer trc(lead && do_a ? p.trace : nullptr, 0);
     const uint32_t a_box_bytes = (uint32_t)(p.hb * p.pack * KC * 2);
-    const uint32_t tx_bytes = (kPair ? 2u : 1u) * ((uint32_t)p.a_boxes * a_box_bytes + (uint32_t)b_bytes);
+    const uint32_t tx_bytes = (uint32_t)p.a_boxes * a_box_bytes + (uint32_t)b_bytes;
     const int row_step = p.hb * p.stride;
     int s = 0; uint32_t phs = 0;   // ring position, continuous across tiles
 #ifdef STG_PROF_LOOP
     long long prof[4] = {0, 0, 0, 0};   // clocks in: empty wait | expect_tx + A loads | W loads + advance ; stages
 #endif
     for (int t = tile0; t < p.n_tiles; t += tstep) {
-      const Tile x = decode_tile<kPair>(p, t, rank);
+      const Tile x = decode_tile(p, t);
       trc.ev(1, t);
       const int n_groups = p.res_gfirst[x.res + 1] - x.g0;
-      // W coordinate of this CTA's (half) tile along the destination-channel axis
-      const int wc = p.b_mn == 0 ? x.col0 + (kPair ? rank * (p.bn / 2) : 0)
-                   : p.b_mn == 2 ? x.wcol0 / 64 + (kPair ? rank * (p.bn / 128) : 0) : x.wcol0;
+      // W coordinate of the tile along the destination-channel axis
+      const int wc = p.b_mn == 0 ? x.col0 : p.b_mn == 2 ? x.wcol0 / 64 : x.wcol0;
       for (int gi = 0; gi < n_groups; ++gi) {
         const int g = x.g0 + gi;
         const int row0 = x.h0 * p.stride + p.tt.g_off[g];
@@ -422,29 +397,28 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
           const long long pc1 = clock64();
 #endif
           const uint32_t a_dst = smem_base + (uint32_t)(s * stage_bytes);
-          const uint32_t fb = kPair ? lead_full_bar(s) : full_bar(s);
+          const uint32_t fb = full_bar(s);
           const int c0 = x.ch0 + chunk * KC;
           if (do_a) {
-            // pair: both CTAs' bytes complete on the leader's barrier, which expects the sum
-            if (rank == 0) mbar_expect_tx_el(full_bar(s), tx_bytes);
+            mbar_expect_tx_el(fb, tx_bytes);
 #pragma unroll 1
             for (int bx = 0; bx < p.a_boxes; ++bx)
-              tma_load_4d_el<kPair>(a_dst + bx * a_box_bytes, &tmA4.m[x.cls], fb, c0, 0, row0 + bx * row_step, x.b);
+              tma_load_4d_el(a_dst + bx * a_box_bytes, &tmA4.m[x.cls], fb, c0, 0, row0 + bx * row_step, x.b);
           }
 #ifdef STG_PROF_LOOP
           const long long pc2 = clock64();
 #endif
           if (do_a) {
           } else if (p.cu_k) {       // compact groups: [cu_fpc * cu_n rows][cu_k] block of the units of this chunk
-            tma_load_3d_el<kPair>(a_dst + p.a_bytes, &tmW, fb, 0, x.col0 + chunk * p.cu_fpc * p.cu_n, tap);
+            tma_load_3d_el(a_dst + p.a_bytes, &tmW, fb, 0, x.col0 + chunk * p.cu_fpc * p.cu_n, tap);
           } else if (p.b_mn == 0) {
-            tma_load_3d_el<kPair>(a_dst + p.a_bytes, &tmW, fb, chunk * KC, wc, tap);
+            tma_load_3d_el(a_dst + p.a_bytes, &tmW, fb, chunk * KC, wc, tap);
           } else if (p.b_mn == 2) {  // forward pack seen as (64, co row, ci/64, tap): one box = the whole [bn/64][64][64] tile
-            tma_load_4d_el<kPair>(a_dst + p.a_bytes, &tmW, fb, 0, c0, wc, tap);
+            tma_load_4d_el(a_dst + p.a_bytes, &tmW, fb, 0, c0, wc, tap);
           } else {  // forward pack [k][c_src][c_dst/g]: bn/64 boxes of (64 destination channels x 64 source-channel rows)
 #pragma unroll 1
             for (int nb = 0; nb < p.bn / 64; ++nb)
-              tma_load_3d_el<kPair>(a_dst + p.a_bytes + nb * 8192, &tmW, fb, wc + nb * 64, c0, tap);
+              tma_load_3d_el(a_dst + p.a_bytes + nb * 8192, &tmW, fb, wc + nb * 64, c0, tap);
           }
           if (++s == p.stages) { s = 0; phs ^= 1u; }
 #ifdef STG_PROF_LOOP
@@ -458,9 +432,9 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
     if (lead && do_a && p.trace && blockIdx.x == 0) for (int i = 0; i < 4; ++i) p.trace[1 + 3 * 5200 + i] = prof[i];
 #endif
   } else if (warp == 1 && p.max_ntaps == 1) {
-    // ===== MMA issuer, one tap per stage (warp-uniform control flow; pair: the leader issues for both CTAs) =====
+    // ===== MMA issuer, one tap per stage (warp-uniform control flow) =====
     const bool lead = lane == 0;
-    const uint32_t idesc = idesc_bf16_f32(kPair ? 2 * TM : TM, p.bn, 0, p.b_mn ? 1 : 0);
+    const uint32_t idesc = idesc_bf16_f32(TM, p.bn, 0, p.b_mn ? 1 : 0);
     const uint32_t idesc_u = idesc_bf16_f32(TM, p.cu_k ? p.cu_n : p.bn, 0, 0);   // compact groups: N = one unit's columns
     // ... K steps per unit = 1 << cu_ks, B descriptor without its start address, start-address step between units
     const int cu_ks = p.cu_k == 16 ? 0 : (p.cu_k == 32 ? 1 : 2), cu_km = (1 << cu_ks) - 1;
@@ -477,8 +451,8 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
 #ifdef STG_PROF_LOOP
     long long mprof[3] = {0, 0, 0};     // clocks in: full wait | MMA issue + commits ; stages
 #endif
-    for (int t = tile0; t < p.n_tiles && rank == 0; t += tstep) {
-      const Tile x = decode_tile<kPair>(p, t, rank);
+    for (int t = tile0; t < p.n_tiles; t += tstep) {
+      const Tile x = decode_tile(p, t);
       if (x.n_iters == 0) continue;
       const int as = acc_i & 1, aph = (acc_i >> 1) & 1;
       mbar_wait(tmem_empty_bar(as), aph ^ 1);  // epilogue(s) have drained this accumulator buffer
@@ -508,15 +482,15 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
 #pragma unroll
           for (int i = 0; i < KC / 16; ++i) {
             const int q = i >> cu_ks, ks = i & cu_km;
-            umma_bf16_el<kPair>(dcol + (uint32_t)(q * p.cu_n), ad + 2 * i, bu + (uint64_t)(q * cu_bq + 2 * ks), idesc_u, (acc0 | (uint32_t)(ks > 0)));
+            umma_bf16_el(dcol + (uint32_t)(q * p.cu_n), ad + 2 * i, bu + (uint64_t)(q * cu_bq + 2 * ks), idesc_u, (acc0 | (uint32_t)(ks > 0)));
           }
         } else {
 #pragma unroll
           for (int ks = 0; ks < KC / 16; ++ks)
-            umma_bf16_el<kPair>(d_tmem, ad + 2 * ks, bd + bstep * ks, idesc, (it > 0 || ks > 0) ? 1u : 0u);
+            umma_bf16_el(d_tmem, ad + 2 * ks, bd + bstep * ks, idesc, (it > 0 || ks > 0) ? 1u : 0u);
         }
-        umma_commit_el<kPair>(empty_bar(s));
-        if (it == x.n_iters - 1) umma_commit_el<kPair>(tmem_full_bar(as));
+        umma_commit_el(empty_bar(s));
+        if (it == x.n_iters - 1) umma_commit_el(tmem_full_bar(as));
         if (++s == p.stages) { s = 0; phs ^= 1u; }
 #ifdef STG_PROF_LOOP
         const long long mc2 = clock64();
@@ -534,7 +508,7 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
     const bool do_a = warp == 0;
     int s = 0; uint32_t phs = 0;
     for (int t = tile0; t < p.n_tiles; t += tstep) {
-      const Tile x = decode_tile<kPair>(p, t, rank);
+      const Tile x = decode_tile(p, t);
       const int n_groups = p.res_gfirst[x.res + 1] - x.g0;
       for (int gi = 0; gi < n_groups; ++gi) {
        const int g = x.g0 + gi;
@@ -579,7 +553,7 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
     const int cu_bq = (p.cu_n * p.cu_k * 2) >> 4;
     int s = 0, acc_i = 0; uint32_t phs = 0;
     for (int t = tile0; t < p.n_tiles; t += tstep) {
-      const Tile x = decode_tile<kPair>(p, t, rank);
+      const Tile x = decode_tile(p, t);
       if (x.n_iters == 0) continue;
       const int as = acc_i & 1, aph = (acc_i >> 1) & 1;
       mbar_wait(tmem_empty_bar(as), aph ^ 1);
@@ -652,7 +626,7 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
       // iterator over (tile, sub-tile) pairs for the operand loads, which run 1 << in_sh sub-tiles ahead of the math (a load
       // takes 0.6-0.8 us to land, a team turns a sub-tile around in ~0.25 us: two in flight left the math waiting)
       int ld_t = tile0, ld_s = 0, ld_q = 0;
-      Tile lx = decode_tile<kPair>(p, ld_t < p.n_tiles ? ld_t : tile0, rank);
+      Tile lx = decode_tile(p, ld_t < p.n_tiles ? ld_t : tile0);
       auto issue_loads = [&]() {
         if (e.n_in == 0 || ld_t >= p.n_tiles) return;
         const int buf = ld_q & in_mask;
@@ -667,13 +641,13 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
         ++ld_q;
         if (++ld_s == n_sub) {
           ld_s = 0; ld_t += tstep;
-          if (ld_t < p.n_tiles) lx = decode_tile<kPair>(p, ld_t, rank);
+          if (ld_t < p.n_tiles) lx = decode_tile(p, ld_t);
         }
       };
       for (int i = 0; i <= in_mask; ++i) issue_loads();
       int q = 0;
       for (int t = tile0; t < p.n_tiles; t += tstep) {
-        const Tile x = decode_tile<kPair>(p, t, rank);
+        const Tile x = decode_tile(p, t);
         const int r0_out = x.h0 >> rsh;
         for (int s = 0; s < n_sub; ++s, ++q) {
           const int obuf = ring(q);
@@ -705,7 +679,7 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
       Tracer trc(threadIdx.x == 64 ? p.trace : nullptr, 2);
       int acc_i = 0, qbase = 0;
       for (int t = tile0; t < p.n_tiles; t += tstep) {
-        const Tile x = decode_tile<kPair>(p, t, rank);
+        const Tile x = decode_tile(p, t);
         const int as = acc_i & 1, aph = (acc_i >> 1) & 1;
         trc.ev(10, t);
         // length mask: my row is (x.b, x.h0 + m), or in a row-class tail tile, which stacks seg-row slices of 128 / seg
@@ -744,7 +718,7 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
         if (last_s < 0 && x.n_iters > 0) {   // nothing to read: hand the buffer back (after tmem_full, so the arrival lands in this tile's phase)
           tc_fence_before();
           __syncwarp();
-          if (lane == 0) arrive_tmem_empty(as);
+          if (lane == 0) mbar_arrive(tmem_empty_bar(as));
         }
 #pragma unroll 1
         for (int s = (qbase & 1) == team ? 0 : 1; s < n_sub; s += 2) {
@@ -761,7 +735,7 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
           if (s == last_s && x.n_iters > 0) {  // my team's part of the accumulator is read: hand the TMEM buffer back to the MMA warp
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) arrive_tmem_empty(as);
+            if (lane == 0) mbar_arrive(tmem_empty_bar(as));
           }
           if (e.bias) {
 #pragma unroll
@@ -850,7 +824,7 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
     const int c_lo = (half == 0) ? 0 : (n_chunks + 1) / 2, c_hi = (half == 0) ? (n_chunks + 1) / 2 : n_chunks;
     int acc_i = 0;
     for (int t = tile0; t < p.n_tiles; t += tstep) {
-      const Tile x = decode_tile<kPair>(p, t, rank);
+      const Tile x = decode_tile(p, t);
       const int as = acc_i & 1, aph = (acc_i >> 1) & 1;
       const int arow = out_row(p, x, sub * 32 + lane);  // output row of this thread (before pair_sum)
       const bool row_ok = arow >= 0 && (!e.pair_sum || (lane & 1) == 0);
@@ -895,19 +869,14 @@ conv_tc_kernel(const __grid_constant__ TmA4 tmA4, const __grid_constant__ CUtens
       if (x.n_iters > 0) {
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) arrive_tmem_empty(as);
+        if (lane == 0) mbar_arrive(tmem_empty_bar(as));
         ++acc_i;
       }
     }
   }
   tc_fence_before();
-  if constexpr (kPair) {
-    cluster_sync_all();   // the peer may still read this CTA's shared memory / arrive on its barriers until here
-    if (warp == 1) tmem_dealloc_2sm(tmem_base, (uint32_t)p.tmem_cols);
-  } else {
-    __syncthreads();
-    if (warp == 1) tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
-  }
+  __syncthreads();
+  if (warp == 1) tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
   life_ev(p.trace, 33);
 }
 
@@ -954,46 +923,33 @@ static int sm_count() {
   return (g_sm_limit > 0 && g_sm_limit < n) ? g_sm_limit : n;   // stg_set_sm_limit: leave SMs to a concurrent communicator
 }
 
-// Cost model for the column-tile width (STG_BN_MODEL=0: the ">= min tiles" rule below).  One CTA per SM walks
-// ceil(tiles / SMs) tiles; a tile's main loop costs n_stages x (max(2 bn, 200) + 60) clk (the MMAs of a 64-deep stage against the
-// producers' issue floor), epilogues hide behind the next tile's main loop except the last one (bn / 32 sub-tiles of
-// ~200 clk with two teams).  Picks the divisor of cd_g with the smallest makespan; ties go to the wider tile.
+// Cost model for the column-tile width.  One CTA per SM walks ceil(tiles / SMs) tiles; a tile's main loop costs
+// n_stages x (max(2 bn, 200) + 60) clk (the MMAs of a 64-deep stage against the producers' issue floor), epilogues hide
+// behind the next tile's main loop except the last one (bn / 32 sub-tiles of ~200 clk with two teams).  Picks the
+// multiple of `step` dividing cd_g with the smallest makespan (0: none divides); ties go to the wider tile.
 static int pick_bn_model(int cd_g, int groups, int64_t row_tiles, int n_stages, int step) {
-  // STG_BN_FEED (B/clk an SM ingests through TMA, 0 = not modelled) and STG_BN_ALPHA (weight of the SM-time objective
-  // against the launch's own makespan): see the note on work conservation in DESIGN.md 3.x
-  static const double feed = getenv("STG_BN_FEED") ? atof(getenv("STG_BN_FEED")) : 0.0;
-  static const double alpha = getenv("STG_BN_ALPHA") ? atof(getenv("STG_BN_ALPHA")) : 0.0;
   int best = 0;
   double best_t = 0;
   for (int bn = 256; bn >= step; bn -= step) {
     if (cd_g % bn) continue;
     const int64_t tiles = row_tiles * (cd_g / bn) * groups;
     const double waves = (double)((tiles + sm_count() - 1) / sm_count());
-    double mma = 2.0 * bn > 200.0 ? 2.0 * bn : 200.0;
-    if (feed > 0.0) { const double ld = (TM * KC * 2 + bn * KC * 2) / feed; if (ld > mma) mma = ld; }
+    const double mma = 2.0 * bn > 200.0 ? 2.0 * bn : 200.0;
     const double stage = mma + 60.0;   // + barrier round trip / commit latency per stage
     const double epi = (bn / 32.0) * 200.0;
-    const double makespan = waves * n_stages * stage + epi;
-    const double smtime = (double)tiles * (n_stages * stage + epi) / sm_count();
-    const double t = alpha * smtime + (1.0 - alpha) * makespan;
+    const double t = waves * n_stages * stage + epi;
     if (best == 0 || t < best_t * 0.999) { best = bn; best_t = t; }
   }
   return best;
 }
-static bool bn_model_on() {
-  static const bool on = !(getenv("STG_BN_MODEL") && atoi(getenv("STG_BN_MODEL")) == 0);
-  return on;
-}
 
 static int pick_bn(int cd_g, int groups, int64_t row_tiles, int n_stages) {
   if (groups == 1 && (cd_g % 16) != 0) return cd_g <= 16 ? 16 : (cd_g <= 128 ? ((cd_g + 15) / 16) * 16 : 128);
-  static const int env_bn = getenv("STG_BN") ? atoi(getenv("STG_BN")) : 0;  // tuning overrides
-  static const int min_tiles = getenv("STG_MIN_TILES") ? atoi(getenv("STG_MIN_TILES")) : 128;
-  if (env_bn > 0 && cd_g % env_bn == 0) return env_bn;
-  if (bn_model_on()) {
-    const int b = pick_bn_model(cd_g, groups, row_tiles, n_stages, 32);   // multiples of 32: staged-epilogue sub-tiles
-    if (b > 0) return b;
-  }
+  const int b = pick_bn_model(cd_g, groups, row_tiles, n_stages, 32);   // multiples of 32: staged-epilogue sub-tiles
+  if (b > 0) return b;
+  // no multiple of 32 divides cd_g (cd_g = 16 mod 32): the widest dividing multiple of 16, narrower (down to 128) while
+  // the launch has fewer than min_tiles tiles
+  constexpr int min_tiles = 128;
   int best = 0;
   for (int bn = 256; bn >= 16; bn -= 16) {
     if (cd_g % bn) continue;
@@ -1006,19 +962,8 @@ static int pick_bn(int cd_g, int groups, int64_t row_tiles, int n_stages) {
 
 // data-gradient column tiles are whole 64-channel boxes of the forward pack
 static int pick_bn_mn(int cd_g, int groups, int64_t row_tiles, int n_stages) {
-  static const int min_tiles = getenv("STG_MIN_TILES") ? atoi(getenv("STG_MIN_TILES")) : 128;
   if (cd_g % 64 != 0) return groups == 1 ? (cd_g <= 64 ? 64 : 128) : 0;
-  if (bn_model_on()) {
-    const int b = pick_bn_model(cd_g, groups, row_tiles, n_stages, 64);
-    if (b > 0) return b;
-  }
-  int best = 0;
-  for (int bn = 256; bn >= 64; bn -= 64) {
-    if (cd_g % bn) continue;
-    best = bn;
-    if (row_tiles * (cd_g / bn) * groups >= min_tiles) break;
-  }
-  return best;
+  return pick_bn_model(cd_g, groups, row_tiles, n_stages, 64);   // 64 divides cd_g: never 0
 }
 
 // Row classes of a sample of t_dst rows (TcP::n_cls): whole 128-row tiles, then a binary tail (64 / 32 / 16 / 8 rows) whose
@@ -1102,15 +1047,9 @@ int tc_pack_groups(int c_in, int c_out, int groups) {
   // channels on BOTH sides - the forward conv contracts over the input side, the data-gradient over the output side, and
   // an MMA K step is 16 channels.  The packs are block-diagonal only inside a unit (m > 1: groups of 8 channels).
   auto side_ok = [](int c) { return c == 16 || c == 32 || (c % KC) == 0; };
-  static const int env_legacy = getenv("STG_GROUP_MERGE") ? atoi(getenv("STG_GROUP_MERGE")) : 0;   // 1: round-1 block-diagonal packs
-  for (int m = 1; m <= groups && !env_legacy; ++m) {
+  for (int m = 1; m <= groups; ++m) {
     if (groups % m) continue;
     if (side_ok(cin_g * m) && side_ok(cout_g * m)) return groups / m;
-  }
-  // fallback: merge to whole 64-channel K chunks on both sides (redundant MMAs on the zeros)
-  for (int f = 1; f <= groups; ++f) {
-    if (groups % f) continue;
-    if ((cin_g * f) % KC == 0 && (cout_g * f) % KC == 0) return groups / f;
   }
   return groups;
 }
@@ -1205,8 +1144,7 @@ int conv_tc(const StgConv* d, cudaStream_t s, const int32_t* valid_units, int ro
   RowCls rc[4];
   int n_rc = 0;
   int64_t cls_tiles = 0;
-  static const int env_cls = getenv("STG_ROWCLS") ? atoi(getenv("STG_ROWCLS")) : 1;
-  if (env_cls && staged && d->phases == 1 && p.n_res == 1 && d->stride == 1) {
+  if (staged && d->phases == 1 && p.n_res == 1 && d->stride == 1) {
     n_rc = row_classes(d->t_dst, rc);
     for (int c = 0; c < n_rc; ++c)
       cls_tiles += rc[c].tps > 0 ? (int64_t)d->n_samples * rc[c].tps : ceil_div(d->n_samples, TM / rc[c].seg);
@@ -1221,25 +1159,13 @@ int conv_tc(const StgConv* d, cudaStream_t s, const int32_t* valid_units, int ro
   // ---- tap groups (A windows) and pipeline depth.  Taps of a group must lie on one row lattice of the strided
   // A box (same offset mod stride) and close enough for the window to fit its boxes; candidates: <= ng taps per
   // group, pick the ng with the least shared-memory ingest per tile among those that leave >= 3 (else 2) stages.
-  // CTA pairs: two row tiles of one column tile run as ONE cta_group::2 MMA, each CTA staging half of the W columns
-  // (opt-in, see below).  Needs >= 2 row tiles per residue class, whole 16-column (K-major W) / 64-column (MN-major W,
-  // data-gradient) halves, and the one-tap-per-stage pipeline.
-  // Measured (tools/conv_bench.py, profiles/r1c_pair_vs_single.txt): with the issue loops fixed the single-CTA kernel is
-  // no longer operand-feed-bound and pairs are 0-15 % SLOWER (cluster launch + the M = 256 MMA issues at ~100 clk per
-  // instruction), so pairs are opt-in (STG_PAIR=1).
-  static const int env_pair = getenv("STG_PAIR") ? atoi(getenv("STG_PAIR")) : 0;
   p.n_samples = d->n_samples;
-  const int n_mt = d->n_samples * p.tiles_m;
-  bool pair = env_pair != 0 && p.cu_k == 0 && n_rc == 0 && n_mt >= 2 && (p.b_mn ? (p.cd_g % 64 == 0 && p.bn % 128 == 0) : (p.bn % 32 == 0));
-  p.pairs_per_res = (n_mt + 1) / 2;
-  int b_bytes = p.cu_k ? p.cu_fpc * p.cu_n * p.cu_k * 2 : (pair ? p.bn / 2 : p.bn) * KC * 2;
+  const int b_bytes = p.cu_k ? p.cu_fpc * p.cu_n * p.cu_k * 2 : p.bn * KC * 2;
   // epilogue-operand ring: as deep as a column tile has sub-tiles (<= 8) while the main loop keeps >= 4 stages of the
   // one-tap-per-stage plan (or all the stages a tile has), else 4, else 2
-  static const int env_insh = getenv("STG_IN_DEPTH_SH") ? atoi(getenv("STG_IN_DEPTH_SH")) : -1;
   // shared memory for main-loop stages + epilogue staging (the launch adds ~1.5 KB of alignment slack, barriers and tap tables;
   // the SM gives one CTA 227 KB)
-  static const int smem_budget = (getenv("STG_SMEM_BUDGET_KB") ? atoi(getenv("STG_SMEM_BUDGET_KB")) : 224) * 1024;
-  static const int win_min_stages = getenv("STG_WIN_MIN_STAGES") ? atoi(getenv("STG_WIN_MIN_STAGES")) : 3;
+  constexpr int smem_budget = 224 * 1024;
   e.in_sh = 1;
   if (staged && e.n_in > 0) {
     const int stage1 = TM * KC * 2 + (p.cu_k ? p.cu_fpc * p.cu_n * p.cu_k * 2 : p.bn * KC * 2);
@@ -1249,7 +1175,6 @@ int conv_tc(const StgConv* d, cudaStream_t s, const int32_t* valid_units, int ro
       const int epi = ((e.n_in << sh) + 3 * e.n_out) * SLOT + 2048;
       if ((smem_budget - epi) / stage1 >= want) { e.in_sh = sh; break; }
     }
-    if (env_insh >= 1 && env_insh <= 3) e.in_sh = env_insh;
   }
   int epi_bytes = staged ? ((e.n_in << e.in_sh) + 3 * e.n_out) * SLOT + 2048 : 0;
   int avail = smem_budget - epi_bytes;
@@ -1259,11 +1184,9 @@ int conv_tc(const StgConv* d, cudaStream_t s, const int32_t* valid_units, int ro
   // in flight per SM stay the same, the rings get shallower), but the issue-bound data-gradients of the compact-group layers
   // gain 10-25 % (two issuing threads per SM) and grouped layers whose tiles hold few rows (1024 channels in 16 groups,
   // T = 25: 256 mostly empty tiles) run in one wave instead of two (2.0x).  So: those two classes only.
-  // STG_OCC2=0 never, 1 whenever it fits.
-  static const int env_occ2 = getenv("STG_OCC2") ? atoi(getenv("STG_OCC2")) : -1;
   const bool occ2_class = (p.cu_k != 0 && d->transposed) || (tile_groups > 1 && p.cu_k == 0 && p.bn <= 64);
   bool occ2 = false;
-  if ((env_occ2 > 0 || (env_occ2 < 0 && occ2_class)) && staged && !pair && p.bn <= 128) {
+  if (occ2_class && staged && p.bn <= 128) {
     const int epi2 = ((e.n_in << 1) + 2 * e.n_out) * SLOT + 2048;
     const int avail2 = 110 * 1024 - epi2;
     if (avail2 / (TM * KC * 2 + b_bytes) >= 2) { occ2 = true; e.in_sh = 1; epi_bytes = epi2; avail = avail2; }
@@ -1321,37 +1244,20 @@ int conv_tc(const StgConv* d, cudaStream_t s, const int32_t* valid_units, int ro
     pl.ok = pl.stages >= 2;
     return pl;
   };
-  static const int env_ng = getenv("STG_NG") ? atoi(getenv("STG_NG")) : 0;  // tuning override
   Plan best{0, 0, 0, 0, 0, 0, 0, false};
   const long long base_traffic = build(1, nullptr).traffic;
   const int cands[] = {1, 2, 3, 4, 5, 6, 8, 10};
   for (int ci = 0; ci < 8; ++ci) {
     const int ng = cands[ci];
-    if (env_ng > 0 && ng != env_ng && d->k >= env_ng) continue;
     if (ng > d->k && ng != 1) continue;
     Plan pl = build(ng, nullptr);
     if (!pl.ok) continue;
     if (!best.ok) { best = pl; continue; }           // ng = 1 comes first: the baseline
     // a window plan replaces the one-tap-per-stage baseline only if it still pipelines (>= 3 stages) and moves
     // at least 35 % fewer bytes: for k = 3 the saving is ~25 % and the coarser stages cost more than that
-    if (pl.stages >= win_min_stages && pl.traffic * 100 <= base_traffic * 65 && pl.traffic < best.traffic) best = pl;
+    if (pl.stages >= 3 && pl.traffic * 100 <= base_traffic * 65 && pl.traffic < best.traffic) best = pl;
   }
   if (!best.ok) return STG_EUNSUPPORTED;
-  if (pair && best.ng != 1) {   // tap windows keep the single-CTA pipeline: plan again with whole W tiles
-    pair = false;
-    b_bytes = p.bn * KC * 2;
-    best = Plan{0, 0, 0, 0, 0, 0, 0, false};
-    for (int ci = 0; ci < 8; ++ci) {
-      const int ng = cands[ci];
-      if (env_ng > 0 && ng != env_ng && d->k >= env_ng) continue;
-      if (ng > d->k && ng != 1) continue;
-      Plan pl = build(ng, nullptr);
-      if (!pl.ok) continue;
-      if (!best.ok) { best = pl; continue; }
-      if (pl.stages >= win_min_stages && pl.traffic * 100 <= base_traffic * 65 && pl.traffic < best.traffic) best = pl;
-    }
-    if (!best.ok) return STG_EUNSUPPORTED;
-  }
   if (n_rc && best.ng != 1) n_rc = 0;   // tap windows load (128 + shift)-row boxes of one sample: classic tiles
   p.n_cls = n_rc ? n_rc : 1;
   p.cls_mt0[0] = 0;
@@ -1363,21 +1269,14 @@ int conv_tc(const StgConv* d, cudaStream_t s, const int32_t* valid_units, int ro
   p.hb = best.hb; p.a_boxes = best.a_boxes; p.a_bytes = best.a_bytes; p.max_ntaps = best.ng; p.stages = best.stages;
   const int stage_bytes = p.a_bytes + p.max_ntaps * b_bytes;
   const size_t smem = (size_t)p.stages * stage_bytes + epi_bytes + 1024 /*align slack*/ + 8 * (2 * MAX_STAGES + 16) + sizeof(TapTables) + 16;
-  static const bool dbg_plan = getenv("STG_DEBUG_PLAN") != nullptr;
-  if (dbg_plan)
-    fprintf(stderr, "[conv_tc] c %d->%d k%d s%d d%d g%d ph%d T %d->%d tr%d | bn %d staged %d ng %d stages %d hb %d a_boxes %d a_bytes %d "
-            "groups %d tiles_m %d res %d smem %zu occ2 %d\n", d->c_src, d->c_dst, d->k, d->stride, d->dilation, d->groups, d->phases, d->t_src,
-            d->t_dst, d->transposed, p.bn, (int)staged, p.max_ntaps, p.stages, p.hb, p.a_boxes, p.a_bytes, p.res_gfirst[p.n_res],
-            p.tiles_m, p.n_res, smem, (int)occ2);
   if (g_plan_out) {   // host-only query (no tensor maps, no launch): see stg_debug_conv_plan in include/stegan_b200.h
     const int tiles_n = ceil_div(d->c_dst, p.bn);
-    const int64_t nt = pair ? (int64_t)p.n_res * p.pairs_per_res * tiles_n
-                     : n_rc ? (int64_t)p.cls_mt0[p.n_cls] * tiles_n : (int64_t)d->n_samples * p.n_res * p.tiles_m * tiles_n;
-    const int64_t slots = pair ? sm_count() / 2 : (occ2 ? 2 : 1) * sm_count();
+    const int64_t nt = n_rc ? (int64_t)p.cls_mt0[p.n_cls] * tiles_n : (int64_t)d->n_samples * p.n_res * p.tiles_m * tiles_n;
+    const int64_t slots = (occ2 ? 2 : 1) * sm_count();
     int* o = g_plan_out;
-    o[0] = p.bn; o[1] = staged; o[2] = p.max_ntaps; o[3] = p.stages; o[4] = (int)smem; o[5] = occ2; o[6] = pair; o[7] = p.n_cls;
-    o[8] = (int)nt; o[9] = (int)((nt < slots ? nt : slots) * (pair ? 2 : 1)); o[10] = p.cu_k; o[11] = p.k_chunks; o[12] = p.tmem_cols;
-    o[13] = staged && e.n_in > 0 ? 1 << e.in_sh : 0; o[14] = p.out_ring; o[15] = p.n_res;
+    o[0] = p.bn; o[1] = staged; o[2] = p.max_ntaps; o[3] = p.stages; o[4] = (int)smem; o[5] = occ2; o[6] = p.n_cls;
+    o[7] = (int)nt; o[8] = (int)(nt < slots ? nt : slots); o[9] = p.cu_k; o[10] = p.k_chunks; o[11] = p.tmem_cols;
+    o[12] = staged && e.n_in > 0 ? 1 << e.in_sh : 0; o[13] = p.out_ring; o[14] = p.n_res;
     return STG_OK;
   }
 
@@ -1410,7 +1309,7 @@ int conv_tc(const StgConv* d, cudaStream_t s, const int32_t* valid_units, int ro
     const uint64_t C = p.cs_g, N = d->c_dst, K = d->k;
     const uint64_t dims[3] = {C, N, K};
     const uint64_t strides[2] = {C * 2, N * C * 2};
-    const uint32_t box[3] = {(uint32_t)KC, (uint32_t)(pair ? p.bn / 2 : p.bn), 1};
+    const uint32_t box[3] = {(uint32_t)KC, (uint32_t)p.bn, 1};
     int r = make_tmap_bf16(&tmW, d->w, 3, dims, strides, box, nullptr);
     if (r) return r;
   } else if (p.cd_g % 64 == 0) {
@@ -1420,7 +1319,7 @@ int conv_tc(const StgConv* d, cudaStream_t s, const int32_t* valid_units, int ro
     const uint64_t N = p.cd_g, R = d->c_src, K = d->k;
     const uint64_t dims[4] = {64, R, N / 64, K};
     const uint64_t strides[3] = {N * 2, 128, R * N * 2};
-    const uint32_t box[4] = {64, (uint32_t)KC, (uint32_t)((pair ? p.bn / 2 : p.bn) / 64), 1};
+    const uint32_t box[4] = {64, (uint32_t)KC, (uint32_t)(p.bn / 64), 1};
     int r = make_tmap_bf16(&tmW, d->w, 4, dims, strides, box, nullptr);
     if (r) return r;
   } else {  // (destination channel within group, source channel row, tap); bn/64 boxes per tile, partial last box zero-filled
@@ -1454,52 +1353,33 @@ int conv_tc(const StgConv* d, cudaStream_t s, const int32_t* valid_units, int ro
     }
     if (r) return STG_ECUDA;
   }
-  using Kernel = decltype(&conv_tc_kernel<true, false, false>);
-  // [kPair][kStaged][kMask]
-  static const Kernel kernels[2][2][2] = {
-      {{conv_tc_kernel<false, false, false>, conv_tc_kernel<false, false, true>},
-       {conv_tc_kernel<true, false, false>, conv_tc_kernel<true, false, true>}},
-      {{conv_tc_kernel<false, true, false>, conv_tc_kernel<false, true, true>},
-       {conv_tc_kernel<true, true, false>, conv_tc_kernel<true, true, true>}}};
+  using Kernel = decltype(&conv_tc_kernel<true, false>);
+  // [kStaged][kMask]
+  static const Kernel kernels[2][2] = {{conv_tc_kernel<false, false>, conv_tc_kernel<false, true>},
+                                       {conv_tc_kernel<true, false>, conv_tc_kernel<true, true>}};
   static bool attr_set = false;
   if (!attr_set) {
-    for (int i = 0; i < 8; ++i) {
-      const Kernel k = kernels[i >> 2][(i >> 1) & 1][i & 1];
+    for (int i = 0; i < 4; ++i) {
+      const Kernel k = kernels[i >> 1][i & 1];
       STG_CUDA_CHECK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-      if ((i >> 1) == 1)   // staged single-CTA kernels: two may share an SM
+      if (i >> 1)   // staged kernels: two may share an SM
         STG_CUDA_CHECK(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     }
     attr_set = true;
   }
   const bool masked = valid_units != nullptr;
   p.tiles_n = ceil_div(d->c_dst, p.bn);
-  if (pair) {
-    const int64_t n_tiles = (int64_t)p.n_res * p.pairs_per_res * p.tiles_n;
-    if (n_tiles > 0x7fffffff) return STG_EINVAL;
-    p.n_tiles = (int)n_tiles;
-    const int max_pairs = sm_count() / 2;
-    const int n_pairs = p.n_tiles < max_pairs ? p.n_tiles : max_pairs;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2 * n_pairs); cfg.blockDim = dim3(staged ? 384 : 352); cfg.dynamicSmemBytes = smem; cfg.stream = s;
-    cudaLaunchAttribute at[2];
-    cfg.attrs = at; cfg.numAttrs = tc_launch_attrs(at, true);
-    STG_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernels[1][staged][masked], tmA, tmW, em, p));
-    STG_LAUNCH_CHECK();
-    return STG_OK;
-  }
   const int64_t n_tiles = n_rc ? (int64_t)p.cls_mt0[p.n_cls] * p.tiles_n : (int64_t)d->n_samples * p.n_res * p.tiles_m * p.tiles_n;
   if (n_tiles > 0x7fffffff) return STG_EINVAL;
   p.n_tiles = (int)n_tiles;
   g_ingest_bytes += (double)n_tiles * ((double)best.traffic * p.k_chunks / p.n_res + (staged ? (double)e.n_in * p.mrows * p.bn * 2 : 0.0));
-  static const int env_cap = getenv("STG_GRID_CAP") ? atoi(getenv("STG_GRID_CAP")) : 0;   // tuning: CTAs per launch
   const int slots = (occ2 ? 2 : 1) * sm_count();
-  int grid = p.n_tiles < slots ? p.n_tiles : slots;
-  if (env_cap > 0 && grid > env_cap) grid = env_cap;
+  const int grid = p.n_tiles < slots ? p.n_tiles : slots;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid); cfg.blockDim = dim3(staged ? 384 : 352); cfg.dynamicSmemBytes = smem; cfg.stream = s;
-  cudaLaunchAttribute at[2];
-  cfg.attrs = at; cfg.numAttrs = tc_launch_attrs(at, false);
-  STG_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernels[0][staged][masked], tmA, tmW, em, p));
+  cudaLaunchAttribute at[1];
+  cfg.attrs = at; cfg.numAttrs = tc_launch_attrs(at);
+  STG_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernels[staged][masked], tmA, tmW, em, p));
   STG_LAUNCH_CHECK();
   return STG_OK;
 }

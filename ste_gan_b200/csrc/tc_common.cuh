@@ -3,7 +3,6 @@
 // shared-memory and instruction descriptors.  Inline PTX only.
 #pragma once
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -71,48 +70,6 @@ template <int N>
 __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
-// Predicated forms: the producer / MMA warps keep WARP-UNIFORM control flow (every lane runs the loop, one lane's
-// instructions take effect), so addresses, descriptors and table look-ups stay in the uniform datapath.  Inside an
-// `if (lane == 0)` region the compiler moves every operand through R2UR + ELECT loops, which made the MMA issuer
-// ~0.2 us slower per pipeline stage.
-__device__ __forceinline__ void mbar_expect_tx_if(bool pred, uint32_t bar, uint32_t bytes) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %2, 0;\n\t@p mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n\t}"
-               ::"r"(bar), "r"(bytes), "r"((uint32_t)pred) : "memory");
-}
-// k2sm: CTA-pair form (.cta_group::2): `bar` is a shared::cluster address and may be the peer's (leader's) barrier
-template <bool k2sm = false>
-__device__ __forceinline__ void tma_load_3d_if(bool pred, uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2) {
-  if constexpr (k2sm) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %6, 0;\n\t"
-        "@p cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];\n\t}"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"((uint32_t)pred)
-        : "memory");
-    return;
-  }
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %6, 0;\n\t"
-      "@p cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];\n\t}"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"((uint32_t)pred)
-      : "memory");
-}
-template <bool k2sm = false>
-__device__ __forceinline__ void tma_load_4d_if(bool pred, uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2, int c3) {
-  if constexpr (k2sm) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %7, 0;\n\t"
-        "@p cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];\n\t}"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"((uint32_t)pred)
-        : "memory");
-    return;
-  }
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %7, 0;\n\t"
-      "@p cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];\n\t}"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"((uint32_t)pred)
-      : "memory");
-}
-
 // Elected forms for WARP-UNIFORM code (all 32 lanes converged, operands uniform): elect.sync picks one lane and only its
 // instruction takes effect.  ptxas knows the elected predicate selects exactly one thread, so it emits the single-issuer
 // instruction (UTMALDG / UTCHMMA / UTCBAR) directly with uniform-register operands - a `lane == 0` predicate makes it
@@ -121,50 +78,23 @@ __device__ __forceinline__ void tma_load_4d_if(bool pred, uint32_t dst, const CU
 __device__ __forceinline__ void mbar_expect_tx_el(uint32_t bar, uint32_t bytes) {
   asm volatile(STG_EL_BEGIN "@P_el mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n\t}" ::"r"(bar), "r"(bytes) : "memory");
 }
-template <bool k2sm = false>
 __device__ __forceinline__ void tma_load_3d_el(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2) {
-  if constexpr (k2sm) {
-    asm volatile(STG_EL_BEGIN
-        "@P_el cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];\n\t}"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
-  } else {
-    asm volatile(STG_EL_BEGIN
-        "@P_el cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];\n\t}"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
-  }
+  asm volatile(STG_EL_BEGIN
+      "@P_el cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];\n\t}"
+      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
-template <bool k2sm = false>
 __device__ __forceinline__ void tma_load_4d_el(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2, int c3) {
-  if constexpr (k2sm) {
-    asm volatile(STG_EL_BEGIN
-        "@P_el cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];\n\t}"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-  } else {
-    asm volatile(STG_EL_BEGIN
-        "@P_el cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];\n\t}"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-  }
+  asm volatile(STG_EL_BEGIN
+      "@P_el cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];\n\t}"
+      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
 }
-template <bool k2sm = false>
 __device__ __forceinline__ void umma_bf16_el(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  if constexpr (k2sm) {
-    asm volatile(STG_EL_BEGIN ".reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                 "@P_el tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                 ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-  } else {
-    asm volatile(STG_EL_BEGIN ".reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                 "@P_el tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                 ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-  }
+  asm volatile(STG_EL_BEGIN ".reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+               "@P_el tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+               ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
-template <bool k2sm = false>
 __device__ __forceinline__ void umma_commit_el(uint32_t bar) {
-  if constexpr (k2sm) {   // arrives on the barrier at this offset in BOTH CTAs of the pair
-    asm volatile(STG_EL_BEGIN "@P_el tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;\n\t}"
-                 ::"r"(bar), "h"((uint16_t)3) : "memory");
-  } else {
-    asm volatile(STG_EL_BEGIN "@P_el tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n\t}" ::"r"(bar) : "memory");
-  }
+  asm volatile(STG_EL_BEGIN "@P_el tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n\t}" ::"r"(bar) : "memory");
 }
 
 // elected TMA stores / bulk-group bookkeeping (bulk groups belong to the issuing THREAD: elect.sync with a full mask
@@ -207,35 +137,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-template <bool k2sm = false>
-__device__ __forceinline__ void umma_bf16_if(bool pred, uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  if constexpr (k2sm) {
-    asm volatile(
-        "{\n\t.reg .pred p, q;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\tsetp.ne.b32 q, %5, 0;\n\t"
-        "@q tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"((uint32_t)pred)
-        : "memory");
-    return;
-  }
-  asm volatile(
-      "{\n\t.reg .pred p, q;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\tsetp.ne.b32 q, %5, 0;\n\t"
-      "@q tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"((uint32_t)pred)
-      : "memory");
-}
-template <bool k2sm = false>
-__device__ __forceinline__ void umma_commit_if(bool pred, uint32_t bar) {
-  if constexpr (k2sm) {   // arrives on the barrier at this offset in BOTH CTAs of the pair
-    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %1, 0;\n\t"
-                 "@q tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %2;\n\t}"
-                 ::"r"(bar), "r"((uint32_t)pred), "h"((uint16_t)3) : "memory");
-    return;
-  }
-  asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %1, 0;\n\t"
-               "@q tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n\t}" ::"r"(bar), "r"((uint32_t)pred) : "memory");
-}
 // arrive on an mbarrier when all previously issued tcgen05.mma of this thread have completed
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
@@ -252,64 +153,6 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
   for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-// ---- CTA pairs (cta_group::2): two CTAs of one cluster (same TPC) run ONE M = 256 MMA.  Each CTA stages its own
-// 128 A rows and HALF of the B tile; the leader (cluster rank 0) issues the MMA, which reads both CTAs' shared memory and
-// writes 128 accumulator lanes in each CTA's TMEM.  Per-SM operand ingest drops from A + B to A + B/2.
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {   // every thread of the CTA
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// shared::cta address of this CTA -> shared::cluster address of the same offset in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// TMA loads of a pair: destination = this CTA's shared memory, completion bytes signalled on the LEADER's mbarrier
-// (`bar` is a shared::cluster address from mapa_u32(.., 0)); .cta_group::2 is what allows the barrier to live in the peer.
-__device__ __forceinline__ void tma_load_3d_2sm(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_2sm(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-// one warp of EACH CTA of the pair
-__device__ __forceinline__ void tmem_alloc_2sm(uint32_t smem_slot, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_slot), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish_2sm() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_2sm(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void umma_bf16_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrive on the mbarrier at this shared::cta offset in BOTH CTAs of the pair once the MMAs issued so far have completed
-__device__ __forceinline__ void umma_commit_2sm(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"((uint16_t)3) : "memory");
 }
 
 // ---- descriptors
@@ -358,15 +201,13 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 PFN_encodeTiled get_encode_tiled();
-// bf16 tensor, dims[0] contiguous; strides_bytes[i] is the stride of dims[i+1]
-// Launch attribute list for the tcgen05 kernels: PDL (STG_PDL=0 disables) and, for CTA pairs, cluster dimension 2.
-inline int tc_launch_attrs(cudaLaunchAttribute* at, bool pair) {
-  static const bool pdl = !(getenv("STG_PDL") && atoi(getenv("STG_PDL")) == 0);
-  int n = 0;
-  if (pdl) { at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[n].val.programmaticStreamSerializationAllowed = 1; ++n; }
-  if (pair) { at[n].id = cudaLaunchAttributeClusterDimension; at[n].val.clusterDim.x = 2; at[n].val.clusterDim.y = 1; at[n].val.clusterDim.z = 1; ++n; }
-  return n;
+// Launch attribute of the tcgen05 kernels: programmatic dependent launch (see pdl_wait / pdl_trigger).
+inline int tc_launch_attrs(cudaLaunchAttribute* at) {
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;
+  return 1;
 }
+// bf16 tensor, dims[0] contiguous; strides_bytes[i] is the stride of dims[i+1]
 int make_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                    const uint32_t* box, const uint32_t* elem_strides, int swizzle_bytes = 128);
 

@@ -337,8 +337,8 @@ int wgrad_tc(const StgWgrad* d, cudaStream_t s) {
   g_ingest_bytes += (double)gx * gy * nsplit * p.chunks_per_split * stage_bytes;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = dim3(192); cfg.dynamicSmemBytes = smem; cfg.stream = s;
-  cudaLaunchAttribute at[2];
-  cfg.attrs = at; cfg.numAttrs = tc_launch_attrs(at, false);
+  cudaLaunchAttribute at[1];
+  cfg.attrs = at; cfg.numAttrs = tc_launch_attrs(at);
   STG_CUDA_CHECK(cudaLaunchKernelEx(&cfg, wgrad_tc_kernel, tmY, tmX, tmD, p));
   STG_LAUNCH_CHECK();
   return STG_OK;

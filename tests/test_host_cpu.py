@@ -193,17 +193,17 @@ def _conv_plan(**kw):
     import ctypes as C
     import torch
     from ste_gan_b200 import _lib, ops
-    names = ("bn", "staged", "taps_per_stage", "stages", "smem", "occ2", "pair", "row_classes", "tiles", "grid", "compact_k",
-             "k_chunks", "tmem_cols", "in_ring", "out_ring", "residues")
+    names = ("bn", "staged", "taps_per_stage", "stages", "smem", "occ2", "row_classes", "tiles", "grid", "compact_k", "k_chunks",
+             "tmem_cols", "in_ring", "out_ring", "residues")
     ptrs = {k: 8 for k in ("src", "w")}
     ptrs.update({k: 8 for k in kw.pop("ptrs", ("y_raw",))})
     d = ops.StgConv(dtype=ops.code_of(torch.bfloat16), engine=ops.ENGINE_AUTO, **ptrs, **kw)
-    out = (C.c_int * 16)()
+    out = (C.c_int * 15)()
     rc = _lib.load().stg_debug_conv_plan(C.byref(d), out)
     return rc, dict(zip(names, out))
 
 
-def test_conv_engine_plans_of_the_bench_shapes():
+def test_conv_plans_of_every_bench_layer_class():
     """Host-only check of the tcgen05 convolution planner (stg_debug_conv_plan) on every layer class of the benchmarked
     configurations (SURVEY.md 8 a7 / a8 / a9 / a11, B = 16 and the batched 32): the plan fits the hardware (227 KB of shared
     memory, 512 TMEM columns, <= 2 x 148 CTAs), pipelines (>= 2 stages, >= 3 with a tap window), tiles the channels exactly,

@@ -4,8 +4,6 @@ forward against each utterance run alone and against the oracle, and serve_batch
 Tolerances: a masked row is exactly 0 and a kept row is bit-identical to the unmasked call (the mask is a select in the
 epilogue); a masked batch against the same utterance alone: rel-L2 1e-6 (fp32) / 1e-2 (bf16, other tile shapes); against
 the oracle: 1e-4 / 2e-2 (BASELINE.json north_star)."""
-import os
-
 import pytest
 import torch
 
@@ -36,11 +34,9 @@ CASES = [
     ("T896_k1_post0_nan", 896, 128, 128, 1, 1, False, 0, "relu", True, True),
     ("T1024_k1_tanh_dup_nan", 1024, 128, 128, 1, 1, True, None, "tanh", True, True),
 ]
-# expected tcgen05 plan per case: (staged epilogue, CTA pairs with STG_PAIR=1 [, with STG_ROWCLS=0 too]).  With 15 samples,
-# T896 has 105 row tiles: the last pair's rank-1 CTA has no sample (b == n_samples); T1024 runs pairs with the direct epilogue.
-PLANS = {"T100_k1_nan": (1, 0, 1), "T400_dup_post1": (1, 0, 0), "T400_k1_post1_nan": (1, 0, 1), "T1500_d9": (1, 0, 0),
-         "T3000_post0": (1, 0, 0), "T1500_tanh_f32": (0, 0, 0), "T3000_cdst12": (0, 0, 0), "T400_cdst12_dup_post1": (0, 0, 0),
-         "T896_k1_post0_nan": (1, 1, 1), "T1024_k1_tanh_dup_nan": (0, 1, 1)}
+# expected tcgen05 plan per case: staged (1) or direct (0) epilogue
+PLANS = {"T100_k1_nan": 1, "T400_dup_post1": 1, "T400_k1_post1_nan": 1, "T1500_d9": 1, "T3000_post0": 1, "T1500_tanh_f32": 0,
+         "T3000_cdst12": 0, "T400_cdst12_dup_post1": 0, "T896_k1_post0_nan": 1, "T1024_k1_tanh_dup_nan": 0}
 
 
 def _run(ops, engine, dtype, case, x, w, bias, post, lens=None, rpu=1):
@@ -116,9 +112,9 @@ def test_conv_masked_rejects_backward_shapes():
 
 
 @pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
-def test_conv_masked_plans(case):
-    """The tcgen05 cases above reach every kernel instance: staged and direct epilogues, single CTAs and (in the child
-    processes below, STG_PAIR=1) CTA pairs.  The masked call launches the plan of the same unmasked descriptor."""
+def test_conv_masked_epilogue_plans(case):
+    """The tcgen05 cases above reach both masked kernel instances: staged and direct epilogues.  The masked call launches
+    the plan of the same unmasked descriptor."""
     import ctypes as C
     from ste_gan_b200 import _lib
     name, T, ci, co, k, d, dup, post_shift, act, has_bias, _ = case
@@ -127,24 +123,9 @@ def test_conv_masked_plans(case):
                         k=k, dilation=d, stride=1, pad=d * (k // 2), post_shift=post_shift or 0, act=3 if tanh else 1,
                         dup_rows=int(dup), out_f32=int(tanh), src=1, w=1, bias=1 if has_bias else None,
                         add_post=None if post_shift is None else 1, y_raw=None if tanh else 1, y_act=1)
-    out = (C.c_int * 16)()
+    out = (C.c_int * 15)()
     assert _lib.load().stg_debug_conv_plan(C.byref(desc), out) == 0
-    staged, pair, pair_classic = PLANS[name]
-    want_pair = 0 if os.environ.get("STG_PAIR") != "1" else (pair_classic if os.environ.get("STG_ROWCLS") == "0" else pair)
-    assert (out[1], out[6]) == (staged, want_pair), (name, list(out))
-
-
-@pytest.mark.parametrize("env", [{"STG_PAIR": "1"}, {"STG_PAIR": "1", "STG_ROWCLS": "0"}], ids=["cta_pairs", "cta_pairs_classic"])
-def test_conv_masked_cta_pairs_in_a_child_process(env):
-    """CTA pairs (cta_group::2) and the classic tiling are chosen once per process from the environment: re-run the
-    tcgen05 mask cases there, with the plan check that shows which of them run as pairs."""
-    import subprocess, sys
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-q", "-x", "-p", "no:cacheprovider",
-                        "-k", "(test_conv_masked_equals and tcgen05) or test_conv_masked_plans"],
-                       env=dict(os.environ, **env), capture_output=True, text=True, timeout=900,
-                       cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-1000:]
-    assert " passed" in r.stdout and "skipped" not in r.stdout, r.stdout[-1000:]
+    assert out[1] == PLANS[name], (name, list(out))
 
 
 # ---------------------------------------------------------------------------------------------
