@@ -259,6 +259,20 @@ int stg_td_loss(const float* x_real, const float* x_gen, int B, int T, int C, fl
 int stg_td_loss_ex(const float* x_real, const float* x_gen, int B, int T, int C, int n_res, const int* wins,
                    const int* shifts, int pad_windows, int avg_window, float* losses, const float* grad_scale,
                    const float* grad_scale_dev, float* dx_gen, float* scratch, stg_stream_t stream);
+/* Per-utterance TimeDomainFeatureLoss of a padded batch, forward only.  Sample b holds n_b = clamp(valid_units[b], 0,
+ * T / rows_per_unit) * rows_per_unit rows (valid_units: DEVICE int32 [B], read at execution time, so a captured graph serves
+ * any length mix - the convention of stg_conv_masked).  out[b][i] (float32 [B][n_res]) = TimeDomainFeatureLoss(wins[i],
+ * shifts[i], pad_windows, avg_window).time_domain_loss(x_real[b, :n_b], x_gen[b, :n_b]): the filter reflects at n_b and the
+ * L1 mean runs over the F_b * C * 4 features of an n_b-row signal.  No row >= n_b of either input is read (NaN there cannot
+ * reach a kept value).  Where the reference's reflect padding raises (n_b <= avg_window / 2, or n_b <= win / 2 with padded
+ * windows; zero-length samples included) or n_b is shorter than one window, out[b][i] is NaN.  Fixed-order sums without
+ * atomics: a sample's value is bit-identical to the same call at B = 1, T = n_b, and across replays.
+ * scratch: float[4*B*T*C + 8*B*ceil((T+1)*C/256)]; rows >= n_b of its filtered copies are neither written nor read.
+ * STG_EINVAL (before any CUDA call): a NULL pointer, B, T or C < 1, n_res outside [1, 8], a win or shift < 1, an even or
+ * non-positive avg_window, rows_per_unit < 1, T % rows_per_unit != 0.  STG_EUNSUPPORTED: B > 65535. */
+int stg_td_scores(const float* x_real, const float* x_gen, int B, int T, int C, const int32_t* valid_units,
+                  int32_t rows_per_unit, int n_res, const int* wins, const int* shifts, int pad_windows, int avg_window,
+                  float* out, float* scratch, stg_stream_t stream);
 /* TimeDomainFeatureLoss.calculate_time_domain_features (time_domain_loss.py:57-68): x [B][T][C] -> feats [B][F][C][4] =
  * [mean(low), sum(low^2), sum(hi^2), mean(hi)] per frame, low = avg(avg(x)), hi = |x - low|.  scratch: float[2*B*T*C]. */
 int stg_td_features(const float* x, int B, int T, int C, int win, int shift, int pad_windows, int avg_window,

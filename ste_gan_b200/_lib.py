@@ -89,6 +89,7 @@ _SIGS = {
     "stg_axpy_f32": [_P, _P, _I, _F, _L, _P],
     "stg_td_loss": [_P, _P, _I, _I, _I, _P, C.POINTER(C.c_float), _P, _P, _P],
     "stg_td_loss_ex": [_P, _P, _I, _I, _I, _I, C.POINTER(C.c_int), C.POINTER(C.c_int), _I, _I, _P, C.POINTER(C.c_float), _P, _P, _P, _P],
+    "stg_td_scores": [_P, _P, _I, _I, _I, _P, C.c_int32, _I, C.POINTER(C.c_int), C.POINTER(C.c_int), _I, _I, _P, _P, _P],
     "stg_td_features": [_P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P],
     "stg_frame_stats": [_P, _I, _I, _I, _I, _I, _I, _P, _P, _P],
     "stg_window_signal": [_P, _I, _I, _I, _I, _I, _I, _P, _P],

@@ -1,6 +1,7 @@
-// Loss kernels: multi-resolution time-domain feature loss (fwd + bwd), LSGAN MSE-to-constant
-// and feature-matching L1 reductions (fwd + bwd).  HBM-bound; vectorised loads where the
-// layout allows, warp-shuffle + one atomic per block reductions, fp32 arithmetic throughout.
+// Loss kernels: multi-resolution time-domain feature loss (fwd + bwd) and its per-utterance scores on length-masked
+// batches (fwd), LSGAN MSE-to-constant and feature-matching L1 reductions (fwd + bwd).  HBM-bound; vectorised loads where
+// the layout allows, warp-shuffle + one atomic per block reductions (fixed-order, atomic-free for the per-utterance
+// scores), fp32 arithmetic throughout.
 #include "common.cuh"
 
 namespace stg {
@@ -250,6 +251,99 @@ __global__ void window_signal_kernel(const float* __restrict__ x, int B, int T_,
   }
 }
 
+// ---- per-utterance scores of a padded batch (stg_td_scores).  Sample b holds n_b rows and no row >= n_b of either input is
+// read: the filter reflects at n_b and the frames are those of an n_b-row signal.  The features of (b, resolution i) are summed
+// in chunks of TS_ITEMS (frame, channel) items, one CTA per chunk, then the chunks in order by one thread: fixed-order sums
+// without atomics, so a sample's value does not depend on the batch, on T or on the replay.
+constexpr int TS_ITEMS = 256;    // (frame, channel) items per chunk = threads per CTA
+struct TdResSet { TdRes r[8]; };
+
+__device__ __forceinline__ int ts_rows(const int32_t* valid_units, int b, int rows_per_unit, int T_) {
+  return min(max(valid_units[b], 0), T_ / rows_per_unit) * rows_per_unit;
+}
+// frames of an n-row signal, 0 where the reference's reflect padding (or unfold) raises: n <= avg_window / 2, n <= win / 2
+// with padded windows, or fewer rows than one window
+__device__ __forceinline__ int ts_frames(int n, int half, const TdRes& r) {
+  const int p = -r.start0;
+  if (n <= half || p >= n) return 0;
+  const int padded = n + 2 * p;
+  return padded < r.win ? 0 : (padded - r.win) / r.shift + 1;
+}
+
+// low = avg(avg(x)), hi = |x - low| of both inputs (filt = low_r | hi_r | low_g | hi_g, [B][T][C] each); rows >= n_b of filt
+// are left as they are
+__global__ void td_filter_masked_kernel(const float* __restrict__ x_real, const float* __restrict__ x_gen, int T_, int C,
+                                        int64_t n, const int32_t* __restrict__ valid_units, int rows_per_unit, int half,
+                                        float* __restrict__ filt) {
+  const float iw = 1.f / (float)(2 * half + 1);
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < 2 * n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int gen = i >= n;
+    const int64_t e = gen ? i - n : i;
+    const int c = (int)(e % C);
+    const int64_t bt = e / C;
+    const int t = (int)(bt % T_);
+    const int nb = ts_rows(valid_units, (int)(bt / T_), rows_per_unit, T_);
+    if (t >= nb || nb <= half) continue;
+    const float* xs = (gen ? x_gen : x_real) + (bt - t) * C + c;
+    float s2 = 0.f;
+    for (int a = -half; a <= half; ++a) {
+      const int u = reflect(t + a, nb);
+      float s1 = 0.f;
+      for (int q = -half; q <= half; ++q) s1 += xs[(int64_t)reflect(u + q, nb) * C];
+      s2 += s1 * iw;
+    }
+    const float lw = s2 * iw;
+    float* low = filt + 2 * gen * n;
+    low[e] = lw;
+    low[n + e] = fabsf(xs[(int64_t)t * C] - lw);
+  }
+}
+
+// grid (chunk, b, i): partial[(b * n_res + i) * chunks + chunk] = sum over this chunk's items of the 4 feature L1 terms
+__global__ void __launch_bounds__(TS_ITEMS) td_score_partial_kernel(const float* __restrict__ filt, int T_, int C, int64_t n,
+                                                                      const int32_t* __restrict__ valid_units, int rows_per_unit,
+                                                                      int half, const __grid_constant__ TdResSet rs, int chunks,
+                                                                      float* __restrict__ partial) {
+  __shared__ float red[32];
+  const int chunk = blockIdx.x, b = blockIdx.y, i = blockIdx.z;
+  const TdRes& r = rs.r[i];
+  const int nb = ts_rows(valid_units, b, rows_per_unit, T_);
+  const int64_t items = (int64_t)ts_frames(nb, half, r) * C;
+  if ((int64_t)chunk * TS_ITEMS >= items) return;                   // uniform over the CTA
+  const float *low_r = filt, *hi_r = filt + n, *low_g = filt + 2 * n, *hi_g = filt + 3 * n;
+  const float iw = 1.f / (float)r.win;
+  const int64_t j = (int64_t)chunk * TS_ITEMS + threadIdx.x;
+  float acc = 0.f;
+  if (j < items) {
+    const int c = (int)(j % C), f = (int)(j / C);
+    const int64_t base = (int64_t)b * T_ * C + c;
+    const int start = f * r.shift + r.start0;
+    float ml_r = 0, pl_r = 0, ph_r = 0, mh_r = 0, ml_g = 0, pl_g = 0, ph_g = 0, mh_g = 0;
+    for (int q = 0; q < r.win; ++q) {
+      const int64_t o = base + (int64_t)reflect(start + q, nb) * C;
+      const float a = low_r[o], h = hi_r[o], a2 = low_g[o], h2 = hi_g[o];
+      ml_r += a; pl_r = fmaf(a, a, pl_r); ph_r = fmaf(h, h, ph_r); mh_r += h;
+      ml_g += a2; pl_g = fmaf(a2, a2, pl_g); ph_g = fmaf(h2, h2, ph_g); mh_g += h2;
+    }
+    acc = fabsf((ml_g - ml_r) * iw) + fabsf(pl_g - pl_r) + fabsf(ph_g - ph_r) + fabsf((mh_g - mh_r) * iw);
+  }
+  acc = block_sum(acc, red);
+  if (threadIdx.x == 0) partial[((int64_t)b * gridDim.z + i) * chunks + chunk] = acc;
+}
+
+// one thread per (b, i): the chunks in order, over F_b * C * 4 features; NaN where the sample has no frames
+__global__ void td_score_finish_kernel(const float* __restrict__ partial, const int32_t* __restrict__ valid_units,
+                                       int rows_per_unit, int T_, int C, int half, TdResSet rs, int B, int n_res, int chunks,
+                                       float* __restrict__ out) {
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= B * n_res) return;
+  const int64_t items = (int64_t)ts_frames(ts_rows(valid_units, k / n_res, rows_per_unit, T_), half, rs.r[k % n_res]) * C;
+  if (items == 0) { out[k] = __int_as_float(0x7fffffff); return; }
+  float s = 0.f;
+  for (int64_t q = 0; q * TS_ITEMS < items; ++q) s += partial[(int64_t)k * chunks + q];
+  out[k] = s / (float)(items * 4);
+}
+
 inline int grid_for(int64_t n, int per_thread = 1) {
   int64_t b = ceil_div64(n, 256 * (int64_t)per_thread);
   const int64_t cap = 148 * 8;
@@ -313,6 +407,38 @@ extern "C" int stg_td_loss(const float* x_real, const float* x_gen, int B, int T
                            const float* grad_scale, float* dx_gen, float* scratch, stg_stream_t stream) {
   const int wins[3] = {20, 51, 80}, shifts[3] = {8, 13, 16};  // time_domain_loss.py:88-93
   return stg_td_loss_ex(x_real, x_gen, B, T, C, 3, wins, shifts, 1, 9, losses, grad_scale, nullptr, dx_gen, scratch, stream);
+}
+
+extern "C" int stg_td_scores(const float* x_real, const float* x_gen, int B, int T, int C, const int32_t* valid_units,
+                             int32_t rows_per_unit, int n_res, const int* wins, const int* shifts, int pad_windows,
+                             int avg_window, float* out, float* scratch, stg_stream_t stream) {
+  if (!x_real || !x_gen || !valid_units || !wins || !shifts || !out || !scratch) return STG_EINVAL;
+  if (B < 1 || T < 1 || C < 1 || n_res < 1 || n_res > 8 || avg_window < 1 || (avg_window & 1) == 0) return STG_EINVAL;
+  if (rows_per_unit < 1 || T % rows_per_unit != 0) return STG_EINVAL;
+  if (B > 65535) return STG_EUNSUPPORTED;                           // grid y
+  TdResSet rs;
+  int64_t chunks = 1;                                               // of the longest sample (n_b = T) at any resolution
+  for (int i = 0; i < n_res; ++i) {
+    if (wins[i] < 1 || shifts[i] < 1) return STG_EINVAL;
+    const int p = pad_windows ? wins[i] / 2 : 0;
+    rs.r[i] = TdRes{wins[i], shifts[i], 0, -p};
+    const int64_t padded = (int64_t)T + 2 * p;
+    const int64_t frames = padded < wins[i] ? 0 : (padded - wins[i]) / shifts[i] + 1;
+    const int64_t ch = ceil_div64(frames * C, TS_ITEMS);
+    if (ch > chunks) chunks = ch;
+  }
+  const int half = avg_window / 2;
+  const int64_t n = (int64_t)B * T * C;
+  float* partial = scratch + 4 * n;       // [B][n_res][chunks]: chunks <= ceil((T + 1) * C / TS_ITEMS), since frames <= T + 1
+  td_filter_masked_kernel<<<grid_for(2 * n), 256, 0, S_>>>(x_real, x_gen, T, C, n, valid_units, rows_per_unit, half, scratch);
+  STG_LAUNCH_CHECK();
+  td_score_partial_kernel<<<dim3((unsigned)chunks, B, n_res), TS_ITEMS, 0, S_>>>(scratch, T, C, n, valid_units, rows_per_unit,
+                                                                                   half, rs, (int)chunks, partial);
+  STG_LAUNCH_CHECK();
+  td_score_finish_kernel<<<(B * n_res + 127) / 128, 128, 0, S_>>>(partial, valid_units, rows_per_unit, T, C, half, rs, B, n_res,
+                                                                   (int)chunks, out);
+  STG_LAUNCH_CHECK();
+  return STG_OK;
 }
 
 extern "C" int stg_td_features(const float* x, int B, int T, int C, int win, int shift, int pad_windows, int avg_window,

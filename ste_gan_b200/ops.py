@@ -454,6 +454,26 @@ def td_loss_ex(x_real: Tensor, x_gen: Tensor, resolutions, losses: Tensor, *, pa
                                      _ptr(losses), gs_host, _ptr(gs_dev), _ptr(dx_gen), _ptr(scratch), _stream()), "stg_td_loss_ex")
 
 
+def td_scores(x_real: Tensor, x_gen: Tensor, lengths: Tensor, rate: int, resolutions=None, pad_windows: bool = True,
+              avg_window: int = 9) -> Tensor:
+    """Per-utterance time-domain feature losses of a padded batch (stg_td_scores): x_real / x_gen fp32 [B, T, C], lengths
+    int32 [B] on the device (units of `rate` rows; sample b holds rate * lengths[b] rows, rows past them are never read) ->
+    fp32 [B, n_res], entry (b, i) = TimeDomainFeatureLoss(win_i, shift_i, pad_windows, avg_window).time_domain_loss on
+    sample b alone; NaN where the reference's reflect padding would raise.  resolutions: [(win, shift)], by default the
+    three of MultiTimeDomainFeatureLoss."""
+    if resolutions is None:
+        from .losses.time_domain_loss import _RES as resolutions
+    B, T, Cc = x_gen.shape
+    n, nr = B * T * Cc, len(resolutions)
+    _need(x_real, n, torch.float32, "x_real"); _need(x_gen, n, torch.float32, "x_gen"); _need(lengths, B, torch.int32, "lengths")
+    out = torch.empty((B, nr), device=x_gen.device, dtype=torch.float32)
+    scratch = torch.empty((4 * n + 8 * B * (((T + 1) * Cc + 255) // 256),), device=x_gen.device, dtype=torch.float32)
+    wins = (C.c_int * nr)(*[int(w) for w, _ in resolutions]); shifts = (C.c_int * nr)(*[int(s_) for _, s_ in resolutions])
+    check(_lib.load().stg_td_scores(_ptr(x_real), _ptr(x_gen), B, T, Cc, _ptr(lengths), int(rate), nr, wins, shifts,
+                                    int(pad_windows), int(avg_window), _ptr(out), _ptr(scratch), _stream()), "stg_td_scores")
+    return out
+
+
 def td_features(x: Tensor, win: int, shift: int, pad_windows: bool = True, avg_window: int = 9) -> Tensor:
     """[B,T,C] fp32 -> [B,F,C,4] time-domain features (time_domain_loss.py:57-68)."""
     x = x.contiguous().float()
